@@ -2,6 +2,7 @@
 """Benchmark of the decoder-block hot path (fused residual Add-RMSNorm -> SwiGLU feed-forward).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload 11b|90b] [--mode prefill|train]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic activations: norm2(attn_out, residual) ->
 ff(normed) (reference Model/model.py:271-272) at BASELINE.json configs[1] (Llama-3.2-11B text block, hidden 4096,
@@ -180,17 +181,16 @@ def cpu_reference(hidden, inter, tokens, steps, warmup, min_seconds=0.0, max_sec
 
 def run_reference(args):
     """Reference arm: the reference's own CPU implementation of the path, on this box's host cores, at OUR arm's config
-    (full 4 x 2048-token steps), bounded to a few minutes."""
+    (full 4 x 2048-token steps), exactly --steps timed steps."""
     hidden, inter, batch, seq, label = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if rank != 0:
         return
     tokens = batch * seq
-    tps, ms, cores, done = cpu_reference(hidden, inter, tokens, args.steps, min(args.warmup, 2), max_seconds=170.0)
+    tps, ms, cores, done = cpu_reference(hidden, inter, tokens, args.steps, min(args.warmup, 2), max_seconds=float("inf"))
     sample_txt = (f"{done} full steps of {tokens} tokens (one GPU's share of the workload), fp32, torch CPU (MKL) with {cores} "
-                  "threads; oracle port of reference Model/model.py:166-171,217 + Tools/swiglu/FusedSwiglu.py:18-20"
-                  + ("" if done >= args.steps else f"; stopped at the 170 s bound before the requested {args.steps} steps"))
+                  "threads; oracle port of reference Model/model.py:166-171,217 + Tools/swiglu/FusedSwiglu.py:18-20")
     line = {
         "impl": "reference", "metric": METRIC, "value": tps, "unit": UNIT, "n_gpus": args.gpus, "steps": done,
         "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
@@ -294,6 +294,29 @@ def _timed_steps(fn, steps, warm, dev, world):
         dist.barrier()
     torch.cuda.synchronize()
     return _max_over_ranks(e0.elapsed_time(e1), dev, world) / steps * 1e-3
+
+
+DUMP_BUDGET_BYTES = 60 << 20     # all arrays together, headers included, stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every tensor of `arrays` as out_dir/<name>.npy in float32, so that two builds run with the same arguments can be
+    compared output for output.  Smallest first, each array gets an equal share of what is left of DUMP_BUDGET_BYTES, so the
+    room small arrays do not use goes to the large ones.  An array larger than its share is stored as a 2-D sample of its rows
+    (last dimension kept whole), drawn from a fixed seed and sorted, so every run stores the same rows."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BUDGET_BYTES
+    for n, (name, t) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].numel())):
+        t = t.detach()
+        share = left // (len(arrays) - n)
+        if t.numel() * 4 > share:
+            rows = t.reshape(-1, t.shape[-1])
+            keep = share // (rows.shape[1] * 4)
+            idx = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = rows[idx.to(rows.device)]
+        left -= t.numel() * 4
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------ secondary numbers
@@ -858,12 +881,12 @@ def run_ours(args):
                 y.backward(dys_loc[i % nbuf])
                 for w in (fused.gamma, fused.w_gate, fused.w_up, fused.w_down):
                     w.grad = None
-                return y
+                return y, xx.grad
             x = x.detach().requires_grad_(True)
             normed = norm(x, residual=r)
             y = ffn(normed)
             y.backward(dys[i % nbuf])
-            return y
+            return y, x.grad
         with torch.no_grad():
             if fused is not None:
                 if instrument:
@@ -901,7 +924,7 @@ def run_ours(args):
 
     warm = max(3, args.warmup)
     for i in range(warm):
-        step(i)
+        last = step(i)      # held like the timed loop holds it, so the allocator reaches the same steady state
     barrier()
     sampler = ClockSampler(local)
     if rank == 0:
@@ -914,13 +937,24 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        step(i, instrument=((world == 1 or fused is not None) and not train))
+        if train and fused is None and i == args.steps - 1:   # the last step's gradients alone, not a sum over all steps
+            norm.zero_grad(set_to_none=True)
+            ffn.zero_grad(set_to_none=True)
+        last = step(i, instrument=((world == 1 or fused is not None) and not train))
     e1.record()
     barrier()
     t_wall1 = time.time()
     launches = _lib.lib().l32_kernel_launch_count() - launches0
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
+    if args.dump_outputs:
+        if train:
+            outs = {"y": last[0], "dx": last[1], "grad_gamma": norm.weight.grad, "grad_w_gate": ffn.swiglu.w_gate.grad,
+                    "grad_w_up": ffn.swiglu.w_up.grad, "grad_w_down": ffn.w_down.weight.grad}
+        else:
+            outs = {"y": last}
+        dump_outputs(args.dump_outputs, outs)
+    del last
     ms_total = _max_over_ranks(ms_total, dev, world)
     ms_step = ms_total / args.steps
     value = tokens / (ms_step * 1e-3)
@@ -1078,7 +1112,8 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=400)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 400; 20 for --impl reference, whose steps take seconds each on the CPU)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--workload", choices=sorted(WORKLOADS), default="11b")
@@ -1092,10 +1127,17 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true",
                     help="skip the secondary measurements (RMSNorm GB/s, decode, sustained, baselines, train, config 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="one GPU: after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32; "
+                         "at most 64 MB in all, larger outputs as the same seeded sample of rows in every run)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 20 if args.impl == "reference" else 400
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.gpus != 1):
+        ap.error("--dump-outputs is implemented for the GPU arm on one GPU")
     if args.impl == "reference":
-        if args.steps > 60:
-            args.steps = 20   # a CPU step is >= 1.3 s: the default K of the GPU arm would run for ten minutes
         run_reference(args)
     else:
         if not torch.cuda.is_available():
