@@ -55,7 +55,7 @@ extern "C" {
 /* ABI version of this header (bumped on any signature change).  2: tensor-parallel, LoRA and block-tail entry points.
  * 3: tensor-parallel backward; the all-gather entry points accept an A buffer distinct from the published one;
  *    l32_rmsnorm_backward_add, l32_block_tail_forward_ex, l32_linear_lora_forward / _backward, l32_lm_head_ce_*,
- *    l32_rope_kv_append, l32_gqa_attention_forward. */
+ *    l32_rope_kv_append, l32_gqa_attention_forward; later, additively: l32_gqa_attention_forward_train / _backward. */
 L32_API int l32_abi_version(void);
 /* Number of CUDA kernels this library has launched in the calling process so far (monotonic). */
 L32_API unsigned long long l32_kernel_launch_count(void);
@@ -285,6 +285,27 @@ L32_API int l32_gqa_attention_forward(const void* q, const void* cache_k, const 
                                       void* ctx, void* workspace, size_t workspace_bytes, int batch, int q_len, int heads,
                                       int kv_heads, int head_dim, int max_len, int kv_len, int past_len, int causal, int dtype,
                                       void* stream);
+
+/* Training calls (no KV cache): keys are [0, q_len) of cache_k / cache_v (rows [q_len, max_len), if any, must hold finite
+ * values: they are multiplied by zero probabilities), query i sits at position i.  Same masks as l32_gqa_attention_forward.  Deterministic: no floating-point atomics, the same inputs give the
+ * same bits.
+ * forward_train: ctx as l32_gqa_attention_forward, and lse [batch, heads, q_len] fp32: the log-sum-exp of each row's scaled
+ *   scores in the log2 domain, +inf for a row that sees no key.
+ * backward: from d_ctx (the gradient of ctx) and the forward's q_rot, K / V, ctx and lse: dq [batch, q_len, heads * head_dim],
+ *   dk / dv [batch, q_len, kv_heads * head_dim] -- the gradients of the projection outputs BEFORE RoPE (the inverse rotation at
+ *   position_ids [batch, q_len], rope_base as in l32_rope_kv_append, is applied).  A row that sees no key gets dq = 0 and
+ *   contributes nothing (the reference gives it a uniform softmax, whose loss a model ignores); a padded key gets dk = dv = 0.
+ *   workspace: l32_gqa_attention_backward_workspace_bytes(...) bytes, 16-byte aligned.  Enqueues three kernels; nothing
+ *   allocates or synchronises (graph-capturable). */
+L32_API int l32_gqa_attention_forward_train(const void* q_rot, const void* cache_k, const void* cache_v, const uint8_t* key_keep,
+                                            void* ctx, float* lse, int batch, int q_len, int heads, int kv_heads, int head_dim,
+                                            int max_len, int causal, int dtype, void* stream);
+L32_API size_t l32_gqa_attention_backward_workspace_bytes(int batch, int q_len, int heads);
+L32_API int l32_gqa_attention_backward(const void* d_ctx, const void* q_rot, const void* cache_k, const void* cache_v, const void* ctx,
+                                       const float* lse, const uint8_t* key_keep, const int64_t* position_ids, void* dq, void* dk,
+                                       void* dv, void* workspace, size_t workspace_bytes, int batch, int q_len, int heads,
+                                       int kv_heads, int head_dim, int max_len, int causal, float rope_base, int dtype,
+                                       void* stream);
 
 /* General tiled GEMM used by the entry points above (exposed for tests, tuning and the tensor-parallel
  * host code):  D[m,n] = A[m,k] B[n,k]^T  (+ A1 B1^T when a1 != NULL).

@@ -9,6 +9,7 @@ from .modules import (  # noqa: F401
     FusedFeedForward,
     FusedFeedforward,
     FusedSwiGLU,
+    GQAAttentionFunction,
     GroupQueryAttention,
     KVCache,
     LLAMARMSNorm,
@@ -31,4 +32,5 @@ __all__ = [
     "FFNFunction", "FFNLoRAFunction", "FusedFeedForward", "FusedFeedforward", "FusedSwiGLU", "LLAMARMSNorm", "Linear_LORA",
     "LinearFunction", "RMSNormFunction", "SwiGLUFunction", "block_tail", "convert_feedforward_to_fused", "convert_instances",
     "patch_reference", "BlockTailFunction", "LinearLoRAFunction", "chain_block_norms", "LMHeadCEFunction", "lm_head_loss", "shift_labels", "GroupQueryAttention", "KVCache",
+    "GQAAttentionFunction",
 ]

@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "_build")
 LIB = os.path.join(HERE, "libl32ffn.so")
-SOURCES = ["rmsnorm.cu", "gemm_sm100.cu", "ffn_decode.cu", "elementwise.cu", "tp.cu", "lmhead.cu", "attention.cu", "api.cu"]
+SOURCES = ["rmsnorm.cu", "gemm_sm100.cu", "ffn_decode.cu", "elementwise.cu", "tp.cu", "lmhead.cu", "attention.cu", "attention_bwd.cu", "api.cu"]
 HEADERS = ["l32_internal.cuh", "ptx_sm100.cuh", os.path.join("..", "..", "include", "l32_ffn.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",

@@ -765,6 +765,49 @@ int l32_gqa_attention_forward(const void* q, const void* cache_k, const void* ca
                          causal, workspace, workspace_bytes, dtype, as_stream(stream));
 }
 
+// Training forward of GroupQueryAttention's attention core (reference Model/model.py:238-253 under autograd): the flash
+// forward of l32_gqa_attention_forward over keys [0, q_len), which also stores the per-row log-sum-exp for the backward.
+int l32_gqa_attention_forward_train(const void* q_rot, const void* cache_k, const void* cache_v, const uint8_t* key_keep, void* ctx,
+                                    float* lse, int batch, int q_len, int heads, int kv_heads, int head_dim, int max_len, int causal,
+                                    int dtype, void* stream) {
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (batch < 0 || q_len < 0 || heads <= 0 || kv_heads <= 0 || (heads % kv_heads) != 0 || (head_dim != 64 && head_dim != 128) ||
+        max_len < q_len || max_len <= 0)
+        return L32_ERR_BAD_SHAPE;
+    if (batch == 0 || q_len == 0) return L32_OK;
+    if (q_rot == nullptr || cache_k == nullptr || cache_v == nullptr || ctx == nullptr || lse == nullptr) return L32_ERR_NULL;
+    if (!is_aligned16(q_rot) || !is_aligned16(cache_k) || !is_aligned16(cache_v) || !is_aligned16(ctx)) return L32_ERR_BAD_ALIGN;
+    return gqa_attention_train(q_rot, cache_k, cache_v, key_keep, ctx, lse, batch, q_len, heads, kv_heads, head_dim, max_len, causal,
+                               dtype, as_stream(stream));
+}
+
+size_t l32_gqa_attention_backward_workspace_bytes(int batch, int q_len, int heads) {
+    return gqa_attention_backward_workspace_bytes(batch, q_len, heads);
+}
+
+// Backward of the same (reference Model/model.py:238-253 under autograd: the saved softmax, repeat_kv and RoPE backward).
+int l32_gqa_attention_backward(const void* d_ctx, const void* q_rot, const void* cache_k, const void* cache_v, const void* ctx,
+                               const float* lse, const uint8_t* key_keep, const int64_t* position_ids, void* dq, void* dk, void* dv,
+                               void* workspace, size_t workspace_bytes, int batch, int q_len, int heads, int kv_heads, int head_dim,
+                               int max_len, int causal, float rope_base, int dtype, void* stream) {
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (batch < 0 || q_len < 0 || heads <= 0 || kv_heads <= 0 || (heads % kv_heads) != 0 || (head_dim != 64 && head_dim != 128) ||
+        max_len < q_len || max_len <= 0 || !(rope_base > 1.0f))
+        return L32_ERR_BAD_SHAPE;
+    if (batch == 0 || q_len == 0) return L32_OK;
+    if (d_ctx == nullptr || q_rot == nullptr || cache_k == nullptr || cache_v == nullptr || ctx == nullptr || lse == nullptr ||
+        position_ids == nullptr || dq == nullptr || dk == nullptr || dv == nullptr || workspace == nullptr)
+        return L32_ERR_NULL;
+    if (workspace_bytes < gqa_attention_backward_workspace_bytes(batch, q_len, heads) || !is_aligned16(workspace))
+        return L32_ERR_WORKSPACE;
+    if (!is_aligned16(d_ctx) || !is_aligned16(q_rot) || !is_aligned16(cache_k) || !is_aligned16(cache_v) || !is_aligned16(ctx) ||
+        !is_aligned16(dq) || !is_aligned16(dk) || !is_aligned16(dv))
+        return L32_ERR_BAD_ALIGN;
+    return gqa_attention_backward(d_ctx, q_rot, cache_k, cache_v, ctx, lse, key_keep, reinterpret_cast<const long long*>(position_ids),
+                                  dq, dk, dv, workspace, batch, q_len, heads, kv_heads, head_dim, max_len, causal, rope_base, dtype,
+                                  as_stream(stream));
+}
+
 int l32_gemm(const void* a, int64_t lda, int a_mn_major, const void* b, int64_t ldb, int b_mn_major, const void* a1,
              int64_t lda1, const void* b1, int64_t ldb1, void* d, int64_t ldd, int m, int n, int k, int k1, int dtype,
              int cta_group, int max_ctas, void* stream) {

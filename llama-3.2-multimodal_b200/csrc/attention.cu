@@ -44,6 +44,8 @@ struct AttnParams {
     int splits, tiles_per_split;
     float* part_o;       // [batch][heads][splits][q_len][head_dim] fp32
     float2* part_ml;     // [batch][heads][splits][q_len] (m_ref in the log2 domain, l)
+    float* lse;          // optional [batch, heads, q_len] (training): m_ref + log2(l) in the log2 domain, +inf for a row that
+                         // sees no key (the backward then forms exact zero probabilities for it).  Never with split-KV.
 };
 
 // L32_ATT_NOEXP / L32_ATT_NOPV / L32_ATT_NOLD: experiment builds only (wrong results) -- what the kernel costs without the
@@ -81,7 +83,8 @@ L32_DEVICE uint64_t add_f32x2(uint64_t a, uint64_t b) {
     return d;
 }
 
-template <int kD, typename T>
+// kLse: training forward, also stores the per-row log-sum-exp (a separate instantiation: the inference kernel is unchanged)
+template <int kD, typename T, bool kLse>
 __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ AttnParams p) {
     constexpr int kDAtoms = kD / 64;                       // 64-element (128-byte) column blocks of a head
     constexpr int kQBytes = kQTile * kD * 2;
@@ -413,6 +416,8 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
             }
         } else {
         const float inv = (ntiles > 0 && l > 0.f) ? 1.f / l : 0.f;     // a row without any visible key gives zeros
+        if (kLse && row_ok)
+            p.lse[(static_cast<size_t>(b) * p.heads + head) * p.q_len + qi] = inv > 0.f ? m_ref + log2f(l) : INFINITY;
         T* dst = static_cast<T*>(p.out) + (static_cast<size_t>(b) * p.q_len + (row_ok ? qi : 0)) * (static_cast<size_t>(p.heads) * kD) +
                  head * kD;
 #pragma unroll
@@ -503,12 +508,7 @@ __global__ void __launch_bounds__(128) rope_kv_append_kernel(T* q, const T* __re
     const int b = static_cast<int>(tok / q_len);
     if (static_cast<int>(threadIdx.x) < half) {
         const int i = threadIdx.x;
-        const float pos = static_cast<float>(position_ids[tok]);
-        const float inv_freq = exp2f(-log2_base * (2.0f * static_cast<float>(i) / static_cast<float>(d)));
-        float sn, cs;
-        sincosf(pos * inv_freq, &sn, &cs);
-        cs_sh[i] = cs;
-        sn_sh[i] = sn;
+        rope_cos_sin(static_cast<float>(position_ids[tok]), i, d, log2_base, cs_sh[i], sn_sh[i]);
     }
     __syncthreads();
     const int vph = d >> 4;                              // 16-byte vectors per half row
@@ -562,9 +562,9 @@ __global__ void __launch_bounds__(128) rope_kv_append_kernel(T* q, const T* __re
     }
 }
 
-template <int kD, typename T>
+template <int kD, typename T, bool kLse>
 int launch_attention(const AttnParams& p, cudaStream_t s) {
-    auto* kernel = gqa_attention_kernel<kD, T>;
+    auto* kernel = gqa_attention_kernel<kD, T, kLse>;
     size_t smem = kQTile * kD * 2 + 4 * kKvTile * kD * 2 + 128;   // tiles + barriers
     if (const char* v = getenv("L32_ATT_ONE_CTA_PER_SM")) {   // experiments only: pad so that only one CTA fits per SM
         if (*v == '1') smem = 160 * 1024;
@@ -609,7 +609,7 @@ int gqa_attention_packed(const void* q, const void* cache_k, const void* cache_v
                          int max_len, int kv_len, int splits, void* workspace, int dtype, cudaStream_t s);
 int gqa_attention_launch(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, int batch, int q_len,
                          int heads, int kv_heads, int head_dim, int max_len, int kv_len, int past_len, int causal, int splits,
-                         void* workspace, int dtype, cudaStream_t s);
+                         void* workspace, int dtype, cudaStream_t s, float* lse = nullptr);
 
 int rope_kv_append(void* q, const void* k_new, const void* v_new, const long long* position_ids, void* cache_k, void* cache_v,
                    int batch, int q_len, int heads, int kv_heads, int head_dim, int max_len, int past_len, float rope_base,
@@ -678,6 +678,15 @@ int gqa_attention(const void* q, const void* cache_k, const void* cache_v, const
                                 causal, 1, nullptr, dtype, s);
 }
 
+// Training forward: keys [0, q_len) of the K / V buffers, no past, no split-KV; also writes the per-row log-sum-exp.
+int gqa_attention_train(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, float* lse, int batch,
+                        int q_len, int heads, int kv_heads, int head_dim, int max_len, int causal, int dtype, cudaStream_t s) {
+    if (head_dim != 64 && head_dim != 128) return L32_ERR_BAD_SHAPE;
+    if (batch <= 0 || q_len <= 0) return L32_OK;
+    return gqa_attention_launch(q, cache_k, cache_v, keep, out, batch, q_len, heads, kv_heads, head_dim, max_len, q_len, 0, causal, 1,
+                                nullptr, dtype, s, lse);
+}
+
 // Decode layout: batch' = batch * kv_heads sequences of `group` query rows, one head.
 int gqa_attention_packed(const void* q, const void* cache_k, const void* cache_v, void* out, int batch2, int group, int head_dim,
                          int max_len, int kv_len, int splits, void* workspace, int dtype, cudaStream_t s) {
@@ -687,10 +696,11 @@ int gqa_attention_packed(const void* q, const void* cache_k, const void* cache_v
 
 int gqa_attention_launch(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, int batch, int q_len,
                          int heads, int kv_heads, int head_dim, int max_len, int kv_len, int past_len, int causal, int splits,
-                         void* workspace, int dtype, cudaStream_t s) {
+                         void* workspace, int dtype, cudaStream_t s, float* lse) {
     AttnParams p;
     memset(&p, 0, sizeof(p));
     p.out = out;
+    p.lse = lse;
     p.keep = keep;
     p.batch = batch; p.q_len = q_len; p.heads = heads; p.kv_heads = kv_heads; p.max_len = max_len; p.kv_len = kv_len;
     p.past_len = past_len; p.causal = causal;
@@ -713,10 +723,15 @@ int gqa_attention_launch(const void* q, const void* cache_k, const void* cache_v
         p.part_o = static_cast<float*>(workspace);
         p.part_ml = reinterpret_cast<float2*>(static_cast<uint8_t*>(workspace) + ((rows * head_dim * sizeof(float) + 255) & ~static_cast<size_t>(255)));
     }
+    if (lse != nullptr) {
+        if (dtype == L32_BF16)
+            return head_dim == 128 ? launch_attention<128, __nv_bfloat16, true>(p, s) : launch_attention<64, __nv_bfloat16, true>(p, s);
+        return head_dim == 128 ? launch_attention<128, __half, true>(p, s) : launch_attention<64, __half, true>(p, s);
+    }
     if (dtype == L32_BF16) {
-        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16>(p, s) : launch_attention<64, __nv_bfloat16>(p, s);
+        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16, false>(p, s) : launch_attention<64, __nv_bfloat16, false>(p, s);
     } else {
-        rc = head_dim == 128 ? launch_attention<128, __half>(p, s) : launch_attention<64, __half>(p, s);
+        rc = head_dim == 128 ? launch_attention<128, __half, false>(p, s) : launch_attention<64, __half, false>(p, s);
     }
     if (rc != L32_OK || p.splits == 1) return rc;
     // merge the split-KV partials

@@ -157,6 +157,21 @@ size_t gqa_attention_workspace_bytes(int batch, int q_len, int heads, int kv_hea
 int gqa_attention(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, int batch, int q_len,
                   int heads, int kv_heads, int head_dim, int max_len, int kv_len, int past_len, int causal, void* workspace,
                   size_t workspace_bytes, int dtype, cudaStream_t s);
+int gqa_attention_train(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, float* lse, int batch,
+                        int q_len, int heads, int kv_heads, int head_dim, int max_len, int causal, int dtype, cudaStream_t s);
+// RoPE angle of rotation pair i (of d / 2) at position `pos`: pos * base^(-2 i / d), cos / sin in fp32.  The forward rotation
+// (rope_kv_append_kernel) and the inverse rotation of the backward epilogues share it, so both use bit-identical angles.
+L32_DEVICE void rope_cos_sin(float pos, int i, int d, float log2_base, float& cs, float& sn) {
+    const float inv_freq = exp2f(-log2_base * (2.0f * static_cast<float>(i) / static_cast<float>(d)));
+    sincosf(pos * inv_freq, &sn, &cs);
+}
+
+// ---- attention_bwd.cu : attention backward for training calls (no cache, past_len = 0, keys = queries)
+size_t gqa_attention_backward_workspace_bytes(int batch, int q_len, int heads);
+int gqa_attention_backward(const void* d_ctx, const void* q, const void* cache_k, const void* cache_v, const void* ctx, const float* lse,
+                           const uint8_t* keep, const long long* position_ids, void* dq, void* dk, void* dv, void* workspace, int batch,
+                           int q_len, int heads, int kv_heads, int head_dim, int max_len, int causal, float rope_base, int dtype,
+                           cudaStream_t s);
 
 // ---- tp.cu : tensor-parallel glue (cross-GPU flags, reduction of the partial slots)
 cudaError_t tp_signal(void* const* peer_flags, int world, int index, uint32_t value, uint32_t* zero8, cudaStream_t s);

@@ -25,6 +25,7 @@ __all__ = [
     "RMSNormFunction", "LLAMARMSNorm", "SwiGLUFunction", "FusedSwiGLU", "LinearFunction", "Linear_LORA", "FFNFunction", "FFNLoRAFunction",
     "FusedFeedforward", "FusedFeedForward", "convert_feedforward_to_fused", "patch_reference", "convert_instances", "block_tail",
     "BlockTailFunction", "LinearLoRAFunction", "chain_block_norms", "LMHeadCEFunction", "lm_head_loss", "shift_labels", "GroupQueryAttention", "KVCache",
+    "GQAAttentionFunction",
 ]
 
 
@@ -553,14 +554,60 @@ def _rotate_half(x):
     return torch.cat((-x2, x1), dim=-1)
 
 
+class GQAAttentionFunction(torch.autograd.Function):
+    """ctx [b, t, heads*d] = attention over the PRE-RoPE projection outputs q [b, t, heads*d], k, v [b, t, kv_heads*d] of a
+    training call (no KV cache, query i at position_ids[:, i], keys = queries), on the tcgen05 kernels in both directions.
+    Saves O(t) tensors (the rotated q / k, v, ctx and the per-row log-sum-exp): no [B, heads, S, S] tensor exists.  The
+    backward is one C-ABI call (deterministic) that returns the gradients of q, k, v with the inverse RoPE applied."""
+
+    @staticmethod
+    def forward(ctx, q, k, v, position_ids, causal, key_keep, rope_base, kv_heads):
+        b, t, _ = q.shape
+        d = k.shape[-1] // kv_heads
+        q_rot = q.contiguous().clone()                  # rotated in place below: the caller's q stays as it was
+        ck = torch.empty(b, kv_heads, t, d, dtype=q.dtype, device=q.device)
+        cv = torch.empty_like(ck)
+        if key_keep is not None:
+            key_keep = key_keep.to(torch.uint8).contiguous()
+        ops.rope_kv_append(q_rot, k.contiguous(), v.contiguous(), position_ids, ck, cv, 0, rope_base)
+        out, lse = ops.gqa_attention_forward_train(q_rot, ck, cv, causal, key_keep)
+        ctx.save_for_backward(q_rot, ck, cv, out, lse, key_keep, position_ids)
+        ctx.causal, ctx.rope_base = causal, rope_base
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        q_rot, ck, cv, out, lse, keep, position_ids = ctx.saved_tensors
+        dq, dk, dv = ops.gqa_attention_backward(grad_out, q_rot, ck, cv, out, lse, position_ids, ctx.causal, keep, ctx.rope_base)
+        return dq, dk, dv, None, None, None, None, None
+
+
+def _mask_causal_keep(attention_mask, b, t, kv_len):
+    """The reference's Llama3Model mask (Model/model.py:304-319: causal + key padding) as (causal, key_keep [b, kv_len] | None).
+    None means no masking at all; the key-padding row is read from the last query row, which sees every key the causal part
+    allows."""
+    if attention_mask is None:
+        return False, None
+    keep = None
+    if attention_mask.dim() == 4 and attention_mask.shape[-1] == kv_len and attention_mask.shape[-2] == t and t > 1:
+        keep = attention_mask[:, 0, -1, :] > (torch.finfo(attention_mask.dtype).min / 2)
+        if keep.shape[0] != b:
+            keep = keep.expand(b, -1)
+    return True, keep
+
+
 class GroupQueryAttention(nn.Module):
     """Drop-in for reference Model/model.py:220-254 (same ctor, submodule names and state_dict keys: W_query, W_key, W_value,
     out_proj).  16-bit CUDA inference with head_dim 64 / 128: the three projections and out_proj run on the tcgen05 GEMM
     (fused with their adapter when they are Linear_LORA), RoPE + cache append is one kernel writing straight into the
     preallocated KVCache, and the attention itself is the flash-style tcgen05 kernel -- no [B, heads, S, S] scores, no
     repeat_kv copies, no torch.cat.  `attention_mask` is interpreted as the mask the reference's Llama3Model builds
-    (Model/model.py:304-319: causal + key padding); None means no masking at all, as in the reference.  Anything else
-    (fp32, CPU, autograd, other head sizes, a foreign cache object) evaluates the reference's own expressions."""
+    (Model/model.py:304-319: causal + key padding); None means no masking at all, as in the reference.
+    Under autograd without a cache (training) the same holds in both directions: the projections run as LinearFunction /
+    LinearLoRAFunction and the attention as GQAAttentionFunction (tcgen05 forward + backward, O(t) saved memory).  A query row
+    that sees no key gets zeros and no gradient (the reference gives it a uniform softmax; a model ignores its loss).
+    Anything else (fp32, CPU, other head sizes, a cache under autograd, a foreign cache object) evaluates the reference's own
+    expressions."""
 
     def __init__(self, config, layer_idx=None, dtype=None):
         super().__init__()
@@ -608,25 +655,44 @@ class GroupQueryAttention(nn.Module):
         ctx = (w @ v).transpose(1, 2).contiguous().reshape(b, t, -1)
         return self.out_proj(ctx)
 
-    def _fast_ok(self, x, kv_cache):
+    def _kernel_ok(self, x):
         ws = [m.linear.weight if _is_lora(m) else m.weight for m in (self.W_query, self.W_key, self.W_value, self.out_proj)]
         return (ops.supported(x) and self.head_dim in (64, 128) and x.dim() == 3 and x.numel() > 0 and
-                all(w.is_cuda and w.dtype == x.dtype for w in ws) and (kv_cache is None or isinstance(kv_cache, KVCache)) and
-                not _wants_grad(x, *ws, *[p for m in (self.W_query, self.W_key, self.W_value, self.out_proj) for p in m.parameters()]))
+                all(w.is_cuda and w.dtype == x.dtype for w in ws))
+
+    def _records_grad(self, x):
+        mods = (self.W_query, self.W_key, self.W_value, self.out_proj)
+        return _wants_grad(x, *[p for m in mods for p in m.parameters()])
+
+    def _fast_ok(self, x, kv_cache):
+        return (self._kernel_ok(x) and (kv_cache is None or isinstance(kv_cache, KVCache)) and not self._records_grad(x))
+
+    def _train_ok(self, x, kv_cache):
+        return kv_cache is None and self._kernel_ok(x) and self._records_grad(x)
 
     @staticmethod
     def _project(mod, x):
         return mod(x) if _is_lora(mod) else _linear(x, mod.weight, mod.bias)
 
     def forward(self, hidden_states, attention_mask=None, position_ids=None, kv_cache=None):
-        if (position_ids is None or not self._fast_ok(hidden_states, kv_cache) or
-                (attention_mask is not None and not attention_mask.is_floating_point())):
+        if (position_ids is None or (attention_mask is not None and not attention_mask.is_floating_point())):
+            return self._reference_forward(hidden_states, attention_mask, position_ids, kv_cache)
+        train = self._train_ok(hidden_states, kv_cache)
+        if not train and not self._fast_ok(hidden_states, kv_cache):
             return self._reference_forward(hidden_states, attention_mask, position_ids, kv_cache)
         b, t, _ = hidden_states.shape
         if position_ids.dim() == 1:
             position_ids = position_ids[None]
         if position_ids.shape[0] != b:
             position_ids = position_ids.expand(b, -1)
+        if train:
+            q = self._project(self.W_query, hidden_states)
+            k = self._project(self.W_key, hidden_states)
+            v = self._project(self.W_value, hidden_states)
+            causal, keep = _mask_causal_keep(attention_mask, b, t, t)
+            pos = position_ids.to(device=q.device, dtype=torch.int64).contiguous()
+            ctx = GQAAttentionFunction.apply(q, k, v, pos, causal, keep, self.rope_base, self.num_kv_groups)
+            return self._project(self.out_proj, ctx)
         projs = (self.W_query, self.W_key, self.W_value)
         if (not torch.is_grad_enabled() or not _wants_grad(hidden_states, *[m.weight for m in projs])) and all(
                 not _is_lora(m) and m.bias is None and m.weight.dtype == hidden_states.dtype and _dims8(*m.weight.shape) for m in projs):
@@ -643,14 +709,7 @@ class GroupQueryAttention(nn.Module):
         ops.rope_kv_append(q, k, v, position_ids.to(device=q.device, dtype=torch.int64), ck, cv, past, self.rope_base)
         cache.advance(layer, t)
         kv_len = past + t
-        causal, keep = False, None
-        if attention_mask is not None:
-            causal = True
-            if attention_mask.dim() == 4 and attention_mask.shape[-1] == kv_len and attention_mask.shape[-2] == t and t > 1:
-                # the last query row sees every key the causal part allows: what is still masked there is key padding
-                keep = attention_mask[:, 0, -1, :] > (torch.finfo(attention_mask.dtype).min / 2)
-                if keep.shape[0] != b:
-                    keep = keep.expand(b, -1)
+        causal, keep = _mask_causal_keep(attention_mask, b, t, kv_len)
         ctx = ops.gqa_attention_forward(q, ck, cv, kv_len, past, causal=causal, key_keep=keep)
         return self._project(self.out_proj, ctx)
 

@@ -480,6 +480,65 @@ def gqa_attention_forward(q, cache_k, cache_v, kv_len, past_len, *, causal=True,
     return ctx
 
 
+def _attention_train_args(q_rot, cache_k, cache_v, key_keep):
+    """Shapes of a training call (keys = queries, no past) and the key_keep bytes, checked as gqa_attention_forward does."""
+    b, t = q_rot.shape[0], q_rot.shape[1]
+    _, kvh, max_len, d = cache_k.shape
+    heads = q_rot.shape[-1] // d
+    for ten in (cache_k, cache_v):
+        if not ten.is_contiguous():
+            raise L32Error("attention: cache_k / cache_v must be contiguous")
+    keep = None
+    if key_keep is not None:
+        keep = key_keep.to(torch.uint8).contiguous()
+        if tuple(keep.shape) != (b, t):
+            raise L32Error(f"key_keep must be [batch, kv_len] = {(b, t)}, got {tuple(keep.shape)}")
+    return b, t, heads, kvh, d, max_len, keep
+
+
+def gqa_attention_forward_train(q_rot, cache_k, cache_v, causal=True, key_keep=None):
+    """Training forward over keys [0, t) of the K / V buffers: (ctx [b, t, heads*d], lse [b, heads, t] fp32, log2 domain, +inf
+    for a row that sees no key).  q_rot [b, t, heads*d] with RoPE applied."""
+    _check_cuda(q_rot, cache_k, cache_v, key_keep)
+    b, t, heads, kvh, d, max_len, keep = _attention_train_args(q_rot, cache_k, cache_v, key_keep)
+    qc = q_rot.contiguous()
+    ctx = torch.empty_like(qc)
+    lse = torch.empty(b, heads, t, dtype=torch.float32, device=q_rot.device)
+    with torch.cuda.device(q_rot.device):
+        check(lib().l32_gqa_attention_forward_train(_ptr(qc), _ptr(cache_k), _ptr(cache_v), _ptr(keep), _ptr(ctx), _ptr(lse), b, t,
+                                                    heads, kvh, d, max_len, int(bool(causal)), _dtype_code(qc), _stream(qc)),
+              "l32_gqa_attention_forward_train")
+    return ctx, lse
+
+
+def gqa_attention_backward(d_ctx, q_rot, cache_k, cache_v, ctx, lse, position_ids, causal=True, key_keep=None, rope_base=500000.0):
+    """Gradients of gqa_attention_forward_train with respect to the PRE-RoPE q [b, t, heads*d], k and v [b, t, kv_heads*d]:
+    (dq, dk, dv).  position_ids [b, t] int64: the positions RoPE was applied at."""
+    _check_cuda(d_ctx, q_rot, cache_k, cache_v, ctx, lse, position_ids, key_keep)
+    b, t, heads, kvh, d, max_len, keep = _attention_train_args(q_rot, cache_k, cache_v, key_keep)
+    qc, gc, oc = q_rot.contiguous(), d_ctx.contiguous(), ctx.contiguous()
+    if gc.dtype != qc.dtype:
+        gc = gc.to(qc.dtype)
+    pos = position_ids.contiguous()
+    if pos.dtype != torch.int64 or pos.numel() != b * t:
+        raise L32Error("gqa_attention_backward: position_ids must be int64 [batch, q_len]")
+    if lse.dtype != torch.float32 or lse.numel() != b * heads * t:
+        raise L32Error("gqa_attention_backward: lse must be the fp32 [batch, heads, q_len] of gqa_attention_forward_train")
+    lse = lse.contiguous()
+    dq = torch.empty_like(qc)
+    dk = torch.empty(b, t, kvh * d, dtype=qc.dtype, device=qc.device)
+    dv = torch.empty_like(dk)
+    L = lib()
+    ws_bytes = L.l32_gqa_attention_backward_workspace_bytes(b, t, heads)
+    ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=qc.device)
+    with torch.cuda.device(qc.device):
+        check(L.l32_gqa_attention_backward(_ptr(gc), _ptr(qc), _ptr(cache_k), _ptr(cache_v), _ptr(oc), _ptr(lse), _ptr(keep), _ptr(pos),
+                                           _ptr(dq), _ptr(dk), _ptr(dv), _ptr(ws), ws_bytes, b, t, heads, kvh, d, max_len,
+                                           int(bool(causal)), float(rope_base), _dtype_code(qc), _stream(qc)),
+              "l32_gqa_attention_backward")
+    return dq, dk, dv
+
+
 # --------------------------------------------------------------------------------------------- lm_head + cross entropy
 def lm_head_ce_forward(hidden_states, weight, labels_shifted, ignore_index=-100):
     """logits = hidden_states weight^T and the mean cross entropy against `labels_shifted` (int64, one per token row, already
