@@ -55,7 +55,9 @@ extern "C" {
 /* ABI version of this header (bumped on any signature change).  2: tensor-parallel, LoRA and block-tail entry points.
  * 3: tensor-parallel backward; the all-gather entry points accept an A buffer distinct from the published one;
  *    l32_rmsnorm_backward_add, l32_block_tail_forward_ex, l32_linear_lora_forward / _backward, l32_lm_head_ce_*,
- *    l32_rope_kv_append, l32_gqa_attention_forward; later, additively: l32_gqa_attention_forward_train / _backward. */
+ *    l32_rope_kv_append, l32_gqa_attention_forward; later, additively: l32_gqa_attention_forward_train / _backward, and
+ *    the tensor-parallel attention GEMMs l32_tp_linear_group_forward_allgather, l32_tp_linear_forward_allgather and
+ *    l32_tp_linear_group_backward_dx_reduce_scatter. */
 L32_API int l32_abi_version(void);
 /* Number of CUDA kernels this library has launched in the calling process so far (monotonic). */
 L32_API unsigned long long l32_kernel_launch_count(void);
@@ -384,6 +386,34 @@ L32_API int l32_tp_ffn_backward_dact_allgather(void* dy_full, const void* const*
 L32_API int l32_tp_ffn_backward_dx_reduce_scatter(const void* d_gate, const void* d_up, const void* w_gate, const void* w_up,
                                                   void* const* peer_slots, int rank, int world, int64_t rows_per_rank,
                                                   int64_t tokens, int hidden, int inter_local, int dtype, void* stream);
+
+/* Tensor-parallel attention (heads sharded by KV group: rank r owns query heads [r H/p, (r+1) H/p) and KV heads
+ * [r kv/p, (r+1) kv/p)).  No reference counterpart (the reference has no distributed code); the oracle is
+ * Model/model.py:238-253 with the shards summed.
+ *
+ * Up to three projections of the SAME gathered activations in one persistent launch: y[i] = x_full w[i]^T, w[i]
+ * [out_features[i], in_features] K-major (the shard's rows of W_query / W_key / W_value), y[i] [tokens, out_features[i]].
+ * The all-gather of x_full is pulled inside the kernel exactly as in l32_tp_swiglu_forward_allgather (same meaning of
+ * x_full, peer_x, ready, done, epoch, rows_per_rank); every problem's tiles start at the own rows.  At world == 1 this is
+ * the tiled path of l32_linear_group_forward. */
+L32_API int l32_tp_linear_group_forward_allgather(void* x_full, const void* const* peer_x, const uint32_t* ready,
+                                                  uint32_t* done, uint32_t epoch, int rank, int world, int64_t rows_per_rank,
+                                                  const void* const* w, void* const* y, const int* out_features, int count,
+                                                  int64_t tokens, int in_features, int dtype, void* stream);
+/* y [tokens, out_features] = a_full w^T with the all-gather of a_full pulled in (arguments as above).  w_mn_major = 0:
+ * w is [out_features, in_features]; w_mn_major = 1: w is [in_features, out_features] (e.g. d_ctx = dY_full out_proj_shard
+ * with the out_proj shard [hidden, heads_local * head_dim] as it is). */
+L32_API int l32_tp_linear_forward_allgather(void* a_full, const void* const* peer_a, const uint32_t* ready, uint32_t* done,
+                                            uint32_t epoch, int rank, int world, int64_t rows_per_rank, const void* w,
+                                            int w_mn_major, void* y, int64_t tokens, int in_features, int out_features,
+                                            int dtype, void* stream);
+/* partial dx [tokens, hidden] = sum_{i < num_phases} dy[i] w[i] (ONE GEMM, up to three accumulation phases): dy[i]
+ * [tokens, k[i]], w[i] [k[i], hidden] (row slices of W_query / W_key / W_value, consumed MN-major); every row is stored
+ * into the slot of the rank that owns it (peer_slots as in l32_tp_linear_forward_reduce_scatter). */
+L32_API int l32_tp_linear_group_backward_dx_reduce_scatter(const void* const* dy, const void* const* w, const int* k,
+                                                           int num_phases, void* const* peer_slots, int rank, int world,
+                                                           int64_t rows_per_rank, int64_t tokens, int hidden, int dtype,
+                                                           void* stream);
 
 /* The two forward calls above as ONE persistent kernel: gate/up tiles (all-gather pulled in) and down tiles (reduce-scatter pushed
  * out) share the tile loop -- the down tiles of one group of rows are interleaved with the gate/up tiles of the next

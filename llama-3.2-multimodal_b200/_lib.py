@@ -72,6 +72,12 @@ SIGNATURES = {
                                            [c_int64, c_int, c_int, c_int, c_void_p]),
     "l32_tp_ffn_backward_dx_reduce_scatter": (c_int, [c_void_p] * 5 + [c_int, c_int, c_int64, c_int64, c_int, c_int, c_int,
                                                                        c_void_p]),
+    "l32_tp_linear_group_forward_allgather": (c_int, [c_void_p] * 4 + [ctypes.c_uint32, c_int, c_int, c_int64] + [c_void_p] * 3 +
+                                              [c_int, c_int64, c_int, c_int, c_void_p]),
+    "l32_tp_linear_forward_allgather": (c_int, [c_void_p] * 4 + [ctypes.c_uint32, c_int, c_int, c_int64, c_void_p, c_int, c_void_p,
+                                                                 c_int64, c_int, c_int, c_int, c_void_p]),
+    "l32_tp_linear_group_backward_dx_reduce_scatter": (c_int, [c_void_p] * 3 + [c_int, c_void_p, c_int, c_int, c_int64, c_int64,
+                                                                                c_int, c_int, c_void_p]),
     "l32_tp_ffn_forward_fused": (c_int, [c_void_p] * 4 + [ctypes.c_uint32, c_int, c_int, c_int64] + [c_void_p] * 6 +
                                  [c_int64, c_int, c_int, c_int, c_void_p]),
     "l32_tp_reduce_partials": (c_int, [c_void_p, c_void_p, ctypes.c_uint32, c_int, c_int, c_void_p, c_void_p, c_int64,

@@ -1010,6 +1010,94 @@ int l32_tp_ffn_backward_dx_reduce_scatter(const void* d_gate, const void* d_up, 
     return gemm_sm100(g, as_stream(stream));
 }
 
+/* ---- tensor-parallel attention: q/k/v of the shard with the all-gather pulled in, the backward's three-phase dX pushed out */
+int l32_tp_linear_group_forward_allgather(void* x_full, const void* const* peer_x, const uint32_t* ready, uint32_t* done,
+                                          uint32_t epoch, int rank, int world, int64_t rows_per_rank, const void* const* w,
+                                          void* const* y, const int* out_features, int count, int64_t tokens, int in_features,
+                                          int dtype, void* stream) {
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (count < 1 || count > 3 || !tp_args_ok(rank, world, rows_per_rank, tokens)) return L32_ERR_BAD_SHAPE;
+    if (w == nullptr || y == nullptr || out_features == nullptr) return L32_ERR_NULL;
+    for (int i = 0; i < count; ++i) {
+        if (!shapes_ok(tokens, in_features, out_features[i])) return L32_ERR_BAD_SHAPE;
+        if (w[i] == nullptr || y[i] == nullptr) return L32_ERR_NULL;
+    }
+    if (tokens == 0) return L32_OK;
+    if (x_full == nullptr) return L32_ERR_NULL;
+    cudaStream_t s = as_stream(stream);
+    GemmProblem g = blank(static_cast<int>(tokens), out_features[0], dtype);
+    g.k[0] = in_features;
+    g.a[0] = op(x_full, in_features, 0);
+    g.b[0] = op(w[0], in_features, 0);
+    g.epilogue = EPI_STORE;
+    g.d[0] = y[0];
+    g.ldd = out_features[0];
+    g.cta_group = 2;
+    if (count > 1) {
+        g.group_count = count;
+        for (int i = 0; i < count; ++i) {
+            GroupMember& q = g.group[i];
+            q.a = x_full; q.lda = in_features; q.m = static_cast<int>(tokens);
+            q.b = w[i]; q.ldb = in_features; q.n = out_features[i];
+            q.d = y[i]; q.ldd = out_features[i];
+        }
+    }
+    const int rc = setup_allgather(g, x_full, peer_x, ready, done, epoch, rank, world, rows_per_rank, s);
+    if (rc != L32_OK) return rc;
+    return gemm_sm100(g, s);
+}
+
+int l32_tp_linear_forward_allgather(void* a_full, const void* const* peer_a, const uint32_t* ready, uint32_t* done,
+                                    uint32_t epoch, int rank, int world, int64_t rows_per_rank, const void* w, int w_mn_major,
+                                    void* y, int64_t tokens, int in_features, int out_features, int dtype, void* stream) {
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (!shapes_ok(tokens, in_features, out_features) || !tp_args_ok(rank, world, rows_per_rank, tokens) ||
+        (w_mn_major != 0 && w_mn_major != 1))
+        return L32_ERR_BAD_SHAPE;
+    if (tokens == 0) return L32_OK;
+    if (a_full == nullptr || w == nullptr || y == nullptr) return L32_ERR_NULL;
+    cudaStream_t s = as_stream(stream);
+    GemmProblem g = blank(static_cast<int>(tokens), out_features, dtype);
+    g.k[0] = in_features;
+    g.a[0] = op(a_full, in_features, 0);
+    g.b[0] = op(w, w_mn_major ? out_features : in_features, w_mn_major);
+    g.epilogue = EPI_STORE;
+    g.d[0] = y;
+    g.ldd = out_features;
+    g.cta_group = 2;
+    const int rc = setup_allgather(g, a_full, peer_a, ready, done, epoch, rank, world, rows_per_rank, s);
+    if (rc != L32_OK) return rc;
+    return gemm_sm100(g, s);
+}
+
+int l32_tp_linear_group_backward_dx_reduce_scatter(const void* const* dy, const void* const* w, const int* k, int num_phases,
+                                                   void* const* peer_slots, int rank, int world, int64_t rows_per_rank,
+                                                   int64_t tokens, int hidden, int dtype, void* stream) {
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (num_phases < 1 || num_phases > 3 || !tp_args_ok(rank, world, rows_per_rank, tokens)) return L32_ERR_BAD_SHAPE;
+    if (k == nullptr) return L32_ERR_NULL;
+    for (int i = 0; i < num_phases; ++i)
+        if (!shapes_ok(tokens, hidden, k[i])) return L32_ERR_BAD_SHAPE;
+    if (tokens == 0) return L32_OK;
+    if (dy == nullptr || w == nullptr) return L32_ERR_NULL;
+    for (int i = 0; i < num_phases; ++i)
+        if (dy[i] == nullptr || w[i] == nullptr) return L32_ERR_NULL;
+    // partial dx = sum_i dy_i w_i (w_i [k_i, hidden] consumed MN-major): one GEMM, rows pushed to their owners' slots
+    GemmProblem g = blank(static_cast<int>(tokens), hidden, dtype);
+    g.num_phases = num_phases;
+    for (int i = 0; i < num_phases; ++i) {
+        g.k[i] = k[i];
+        g.a[i] = op(dy[i], k[i], 0);
+        g.b[i] = op(w[i], hidden, 1);
+    }
+    g.epilogue = EPI_STORE;
+    g.ldd = hidden;
+    g.cta_group = 2;
+    const int rc = setup_reduce_scatter(g, peer_slots, rank, world, rows_per_rank, tokens);
+    if (rc != L32_OK) return rc;
+    return gemm_sm100(g, as_stream(stream));
+}
+
 int l32_tp_ffn_forward_fused(void* x_full, const void* const* peer_x, const uint32_t* ready, uint32_t* done, uint32_t epoch,
                              int rank, int world, int64_t rows_per_rank, const void* w_gate, const void* w_up,
                              const void* w_down, void* act_ws, uint32_t* act_done, void* const* peer_slots, int64_t tokens,

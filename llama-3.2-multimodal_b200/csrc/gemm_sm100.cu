@@ -63,7 +63,7 @@ struct GemmKernelParams {
     CUtensorMap map_a[kMaxGroup];   // per accumulation phase -- or, for a grouped launch (nprob > 1), per problem
     CUtensorMap map_b[kMaxGroup];
     int m, n;
-    int k[2];
+    int k[kMaxGroup];
     int num_phases;
     int a_mn_major, b_mn_major;
     int tiles_m, tiles_n, raster_group;
@@ -308,7 +308,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_kernel(const __grid_constant
             if (grouped) {
                 int pr = 0;
                 while (pr + 1 < p.nprob && t >= p.gstart[pr + 1]) ++pr;
-                const TileOrder go = {p.gtm[pr], p.gtn[pr], p.raster_group, 0, 0, 0, 0};
+                // m_rotate is nonzero only with the all-gather, where every problem has the same rows
+                const TileOrder go = {p.gtm[pr], p.gtn[pr], p.raster_group, p.m_rotate, 0, 0, 0};
                 TileCoord c = tile_coord(t - p.gstart[pr], go);
                 c.prob = pr;                                   // here: index of the problem of the group
                 return c;
@@ -320,12 +321,12 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_kernel(const __grid_constant
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&p.map_a[0]);
         tma_prefetch_desc(&p.map_b[0]);
-        if (p.num_phases == 2 || p.nprob > 1) tma_prefetch_desc(&p.map_a[1]);
-        if (p.nprob > 2) {
+        if (p.num_phases > 1 || p.nprob > 1) tma_prefetch_desc(&p.map_a[1]);
+        if (p.nprob > 2 || p.num_phases > 2) {
             tma_prefetch_desc(&p.map_a[2]);
             tma_prefetch_desc(&p.map_b[2]);
         }
-        if (p.num_phases == 2 || p.nprob > 1 || kEpi == EPI_SWIGLU || kTp) tma_prefetch_desc(&p.map_b[1]);
+        if (p.num_phases > 1 || p.nprob > 1 || kEpi == EPI_SWIGLU || kTp) tma_prefetch_desc(&p.map_b[1]);
         if constexpr (kEpi == EPI_SWIGLU_BWD) {
             tma_prefetch_desc(&p.map_out[0]);
             tma_prefetch_desc(&p.map_out[1]);
@@ -916,7 +917,7 @@ int gemm_sm100(const GemmProblem& g, cudaStream_t s) {
     const bool ffn_tp = g.epilogue == EPI_FFN_TP;
     const bool swiglu_like = g.epilogue == EPI_SWIGLU || ffn_tp;
     if (g.dtype != L32_BF16 && g.dtype != L32_FP16) return L32_ERR_BAD_DTYPE;
-    if (g.m < 0 || g.n <= 0 || g.num_phases < 1 || g.num_phases > 2) return L32_ERR_BAD_SHAPE;
+    if (g.m < 0 || g.n <= 0 || g.num_phases < 1 || g.num_phases > kMaxGroup) return L32_ERR_BAD_SHAPE;
     if (g.m == 0) return L32_OK;
     if ((g.n % 8) != 0 || (g.ldd % 8) != 0) return L32_ERR_BAD_ALIGN;
     if (swiglu_like && (g.num_phases != 1 || g.b[0].mn_major || g.b[1].mn_major)) return L32_ERR_BAD_SHAPE;
@@ -1030,10 +1031,16 @@ int gemm_sm100(const GemmProblem& g, cudaStream_t s) {
         }
     }
     if (g.group_count > 1) {
-        // a grouped launch: every problem shares K, the operand majors and the dtype; no bias / addend / collectives
+        // a grouped launch: every problem shares K, the operand majors and the dtype; no bias / addend / reduce-scatter.
+        // The all-gather is allowed when every problem reads the same gathered A (e.g. the q / k / v projections of one
+        // tensor-parallel attention shard): the pullers fetch it once and every tile waits for the chunk it reads.
         if (g.group_count > kMaxGroup || g.epilogue != EPI_STORE || g.num_phases != 1 || g.e[0] != nullptr || g.bias[0] != nullptr ||
-            g.rs.world > 0 || g.ag.world > 0 || cta_group != 2 || g.k[0] <= 0)
+            g.rs.world > 0 || cta_group != 2 || g.k[0] <= 0)
             return L32_ERR_BAD_SHAPE;
+        if (g.ag.world > 1) {
+            for (int i = 0; i < g.group_count; ++i)
+                if (g.group[i].a != g.a[0].ptr || g.group[i].lda != g.k[0] || g.group[i].m != g.m) return L32_ERR_BAD_SHAPE;
+        }
         kp.nprob = g.group_count;
         int start = 0;
         for (int i = 0; i < g.group_count; ++i) {
@@ -1056,7 +1063,7 @@ int gemm_sm100(const GemmProblem& g, cudaStream_t s) {
         kp.gstart[g.group_count] = start;
         kp.k[0] = g.k[0];
         kp.m_il_world = 0;
-        kp.m_rotate = 0;
+        if (g.ag.world <= 1) kp.m_rotate = 0;   // all-gather: own rows first (setup_allgather's rotation), in every problem
         if (g.dtype == L32_BF16) return launch_epi<2, __nv_bfloat16>(kp, EPI_STORE, start, g.max_ctas, s);
         return launch_epi<2, __half>(kp, EPI_STORE, start, g.max_ctas, s);
     }

@@ -102,10 +102,10 @@ struct GroupMember {
 
 struct GemmProblem {
     int m, n;               // D is [m, n]; for EPI_SWIGLU n = intermediate size (act columns)
-    int num_phases;         // 1, or 2 for D = A0*B0^T + A1*B1^T (EPI_SWIGLU: must be 1)
-    int k[2];               // reduction length of each phase
-    GemmOperand a[2];       // a[1] used when num_phases == 2
-    GemmOperand b[2];       // EPI_SWIGLU: b[0] = gate weights, b[1] = up weights (both K-major)
+    int num_phases;         // 1 to 3: D = sum_p A_p*B_p^T (EPI_SWIGLU: must be 1)
+    int k[3];               // reduction length of each phase
+    GemmOperand a[3];       // a[p] used when p < num_phases
+    GemmOperand b[3];       // EPI_SWIGLU: b[0] = gate weights, b[1] = up weights (both K-major)
     int epilogue;           // EPI_*
     void* d[3];             // outputs, see EPI_*; optional ones may be null
     const void* e[2];       // EPI_SWIGLU_BWD: gate / up caches [m, n];  EPI_STORE: e[0] = optional addend [m, n] (D += addend)
@@ -121,7 +121,8 @@ struct GemmProblem {
     TpFfnDown dn;           // EPI_FFN_TP only
     CeOutputs ce;           // EPI_CE only
     int group_count;        // > 1: grouped launch (EPI_STORE, cta_group 2): `group` replaces m / n / a[].ptr / b[].ptr / d
-    GroupMember group[3];   //      (k[0], a[0].mn_major, b[0].mn_major and dtype are shared)
+    GroupMember group[3];   //      (k[0], a[0].mn_major, b[0].mn_major and dtype are shared; with `ag` every member
+                            //      reads the same K-major A = a[0], [m, k[0]] with a dense pitch)
 };
 int gemm_sm100(const GemmProblem& p, cudaStream_t s);   // returns L32_* / cudaError_t
 void debug_tile_order(int t, int tiles_m, int tiles_n, int group, int m_rotate, int il_world, int il_tpc, int il_rank, int* out3);

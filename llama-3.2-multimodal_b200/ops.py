@@ -734,3 +734,66 @@ def tp_reduce_partials(slots, flags, epoch, rank, rows, addend=None, out=None):
                                            int(rows), slot_rows, hidden, _dtype_code(slots), _stream(slots)),
               "l32_tp_reduce_partials")
     return y
+
+
+def tp_linear_group_forward_allgather(x_full, peer_x_ptrs, ready, done, epoch, rank, rows_per_rank, weights):
+    """[x_full w^T for w in weights] (1..3 K-major [out_i, hidden] weights, e.g. the q / k / v rows of a rank's heads) in one
+    persistent launch with the all-gather of x_full pulled in, as in tp_swiglu_forward_allgather."""
+    _check_cuda(x_full, ready, done, *weights)
+    if not 1 <= len(weights) <= 3:
+        raise L32Error("tp_linear_group_forward_allgather takes one to three weights")
+    tokens, hidden = x_full.shape
+    for w in weights:
+        if w.dim() != 2 or w.shape[1] != hidden or not w.is_contiguous() or w.dtype != x_full.dtype:
+            raise L32Error(f"tp linear group: x_full[..., {hidden}] {x_full.dtype} vs weight{tuple(w.shape)} {w.dtype}")
+    ys = [torch.empty(tokens, w.shape[0], dtype=x_full.dtype, device=x_full.device) for w in weights]
+    n = len(weights)
+    w_arr = (ctypes.c_void_p * n)(*[_ptr(w) for w in weights])
+    y_arr = (ctypes.c_void_p * n)(*[_ptr(y) for y in ys])
+    o_arr = (ctypes.c_int * n)(*[w.shape[0] for w in weights])
+    with torch.cuda.device(x_full.device):
+        check(lib().l32_tp_linear_group_forward_allgather(_ptr(x_full), _ptr_array(peer_x_ptrs), _ptr(ready), _ptr(done), int(epoch),
+                                                          int(rank), len(peer_x_ptrs), int(rows_per_rank), w_arr, y_arr, o_arr, n,
+                                                          tokens, hidden, _dtype_code(x_full), _stream(x_full)),
+              "l32_tp_linear_group_forward_allgather")
+    return ys
+
+
+def tp_linear_forward_allgather(a_full, peer_a_ptrs, ready, done, epoch, rank, rows_per_rank, weight, w_mn_major=False):
+    """y = a_full W with the all-gather of a_full pulled in.  weight [out, in] (w_mn_major=False, y = a w^T) or [in, out]
+    (w_mn_major=True, y = a w: e.g. the out_proj shard [hidden, heads_local*d] in the backward)."""
+    _check_cuda(a_full, ready, done, weight)
+    tokens, in_f = a_full.shape
+    out_f = weight.shape[1] if w_mn_major else weight.shape[0]
+    if (weight.shape[0] if w_mn_major else weight.shape[1]) != in_f or not weight.is_contiguous() or weight.dtype != a_full.dtype:
+        raise L32Error(f"tp linear: a_full[..., {in_f}] {a_full.dtype} vs weight{tuple(weight.shape)} {weight.dtype}")
+    y = torch.empty(tokens, out_f, dtype=a_full.dtype, device=a_full.device)
+    with torch.cuda.device(a_full.device):
+        check(lib().l32_tp_linear_forward_allgather(_ptr(a_full), _ptr_array(peer_a_ptrs), _ptr(ready), _ptr(done), int(epoch),
+                                                    int(rank), len(peer_a_ptrs), int(rows_per_rank), _ptr(weight), int(bool(w_mn_major)),
+                                                    _ptr(y), tokens, in_f, out_f, _dtype_code(a_full), _stream(a_full)),
+              "l32_tp_linear_forward_allgather")
+    return y
+
+
+def tp_linear_group_backward_dx_reduce_scatter(dys, weights, peer_slot_ptrs, rank, rows_per_rank):
+    """Partial dX = sum_i dys[i] weights[i] (dys[i] [tokens, k_i], weights[i] [k_i, hidden]; one GEMM of up to three
+    accumulation phases) with every row pushed into its owner's slot, as in tp_ffn_backward_dx_reduce_scatter."""
+    _check_cuda(*dys, *weights)
+    n = len(dys)
+    if not 1 <= n <= 3 or len(weights) != n:
+        raise L32Error("tp_linear_group_backward_dx_reduce_scatter takes one to three (dy, weight) pairs")
+    tokens = dys[0].shape[0]
+    hidden = weights[0].shape[1]
+    for dy, w in zip(dys, weights):
+        if (dy.dim() != 2 or dy.shape[0] != tokens or w.shape != (dy.shape[1], hidden) or not dy.is_contiguous() or
+                not w.is_contiguous() or dy.dtype != w.dtype or dy.dtype != dys[0].dtype):
+            raise L32Error(f"tp dx: dy{tuple(dy.shape)} {dy.dtype} vs weight{tuple(w.shape)} {w.dtype}")
+    dy_arr = (ctypes.c_void_p * n)(*[_ptr(t) for t in dys])
+    w_arr = (ctypes.c_void_p * n)(*[_ptr(w) for w in weights])
+    k_arr = (ctypes.c_int * n)(*[dy.shape[1] for dy in dys])
+    with torch.cuda.device(dys[0].device):
+        check(lib().l32_tp_linear_group_backward_dx_reduce_scatter(dy_arr, w_arr, k_arr, n, _ptr_array(peer_slot_ptrs), int(rank),
+                                                                   len(peer_slot_ptrs), int(rows_per_rank), tokens, hidden,
+                                                                   _dtype_code(dys[0]), _stream(dys[0])),
+              "l32_tp_linear_group_backward_dx_reduce_scatter")
