@@ -281,7 +281,8 @@ L32_API int l32_rope_kv_append(void* q, const void* k_new, const void* v_new, co
  * workspace (optional): l32_gqa_attention_workspace_bytes(...) bytes.  With it a decode step (q_len == 1) splits the cached
  * keys over several CTAs per KV head (fp32 partials + a merge kernel, fixed order: deterministic), which is what keeps small
  * batches with long contexts from running on a handful of SMs; without it (or when the function returns 0) one CTA per KV head
- * walks the whole cache. */
+ * walks the whole cache.  The function returns non-zero exactly when the call will split: q_len == 1, no key_keep, a group
+ * heads / kv_heads of 2 to 128, and enough keys.  Cache rows at or beyond kv_len are never read (whatever they hold). */
 L32_API size_t l32_gqa_attention_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int kv_len);
 L32_API int l32_gqa_attention_forward(const void* q, const void* cache_k, const void* cache_v, const uint8_t* key_keep,
                                       void* ctx, void* workspace, size_t workspace_bytes, int batch, int q_len, int heads,

@@ -32,8 +32,9 @@ constexpr int kUmmaKAtt = 16;
 
 struct AttnParams {
     CUtensorMap map_q;   // [batch * q_len, heads * head_dim], box {64, 128}
-    CUtensorMap map_k;   // [batch * kv_heads * max_len, head_dim], box {64, 64}
-    CUtensorMap map_v;   // same tensor shape as K, box {64, 64}
+    CUtensorMap map_k;   // [batch * kv_heads][kv_len][head_dim] with planes max_len * head_dim apart, box {64, 64, 1}: the
+                         // rows [kv_len, tile end) of the last tile arrive as zeros, whatever the cache holds there
+    CUtensorMap map_v;   // same tensor shape as K, box {64, 64, 1}
     void* out;           // [batch * q_len, heads * head_dim]
     const uint8_t* keep; // optional [batch, kv_len]: 0 = padded key (never attended)
     int batch, q_len, heads, kv_heads, max_len, kv_len, past_len, causal;
@@ -155,7 +156,8 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
     const int total_tiles = (hi + kKvTile - 1) / kKvTile;
     const int tile0 = split * p.tiles_per_split;                          // first key tile of this CTA (0 without split-KV)
     const int ntiles = p.splits > 1 ? max(0, min(p.tiles_per_split, total_tiles - tile0)) : total_tiles;
-    const int kv_row0 = (b * p.kv_heads + kvh) * p.max_len + tile0 * kKvTile;
+    const int kv_plane = b * p.kv_heads + kvh;
+    const int key0 = tile0 * kKvTile;
 
     if (warp == 4) {
         // ------------------------------------------------------------------ TMA producer + MMA issuer (one thread)
@@ -170,14 +172,16 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
                 mbar_arrive_expect_tx(&bar_k[s], kKBytes);
 #pragma unroll
                 for (int a = 0; a < kDAtoms; ++a)
-                    tma_load_2d(sk + s * kKBytes + a * (kKvTile * 128), &p.map_k, &bar_k[s], a * 64, kv_row0 + t * kKvTile, kEvictNormal);
+                    tma_load_3d(sk + s * kKBytes + a * (kKvTile * 128), &p.map_k, &bar_k[s], a * 64, key0 + t * kKvTile, kv_plane,
+                                kEvictNormal);
             };
             auto load_v = [&](int t) {
                 const int s = t & 1;
                 mbar_arrive_expect_tx(&bar_v[s], kKBytes);
 #pragma unroll
                 for (int a = 0; a < kDAtoms; ++a)
-                    tma_load_2d(sv + s * kKBytes + a * (kKvTile * 128), &p.map_v, &bar_v[s], a * 64, kv_row0 + t * kKvTile, kEvictNormal);
+                    tma_load_3d(sv + s * kKBytes + a * (kKvTile * 128), &p.map_v, &bar_v[s], a * 64, key0 + t * kKvTile, kv_plane,
+                                kEvictNormal);
             };
             // S[128, 64] = Q[128, kD] K[64, kD]^T of tile t into accumulator t & 1
             const uint32_t q_addr = smem_u32(sq);
@@ -644,12 +648,21 @@ int rope_kv_append(void* q, const void* k_new, const void* v_new, const long lon
     return static_cast<int>(e);
 }
 
-size_t gqa_attention_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int kv_len) {
-    if (q_len != 1 || batch <= 0) return 0;               // split-KV serves decode (one query per sequence) only
+// Split-KV plan of a decode call without key padding: the number of key splits (1 = none).  Only the packed decode path
+// splits: one query per sequence, the `group` query heads of a KV group as the rows of ONE query tile (a split CTA covers
+// rows [0, kQTile) only, so a larger group is not split).
+static int decode_splits(int batch, int q_len, int heads, int kv_heads, int kv_len) {
+    const int group = heads / kv_heads;
+    if (q_len != 1 || batch <= 0 || group < 2 || group > kQTile) return 1;
     const int tiles = (kv_len + kKvTile - 1) / kKvTile;
     const int ctas = batch * kv_heads;                    // decode packs the heads of a KV group into one CTA
     int splits = (2 * num_sms() + ctas - 1) / ctas;       // aim at two CTAs per SM
     if (splits > tiles / 2) splits = tiles / 2;           // at least two key tiles (128 keys) per split
+    return splits < 2 ? 1 : splits;
+}
+
+size_t gqa_attention_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int kv_len) {
+    const int splits = decode_splits(batch, q_len, heads, kv_heads, kv_len);
     if (splits < 2) return 0;
     return static_cast<size_t>(batch) * heads * splits * (static_cast<size_t>(head_dim) + 2) * sizeof(float) + 256;
 }
@@ -664,13 +677,9 @@ int gqa_attention(const void* q, const void* cache_k, const void* cache_v, const
         // memory), so every K / V tile is read once per group instead of once per query head.  One query per sequence sees
         // the whole cache: no causal predicate needed.
         const int group = heads / kv_heads;
-        int splits = 1;
-        if (workspace != nullptr && workspace_bytes >= gqa_attention_workspace_bytes(batch, 1, heads, kv_heads, head_dim, kv_len) &&
-            gqa_attention_workspace_bytes(batch, 1, heads, kv_heads, head_dim, kv_len) > 0) {
-            const int tiles = (kv_len + kKvTile - 1) / kKvTile;
-            splits = (2 * num_sms() + batch * kv_heads - 1) / (batch * kv_heads);
-            if (splits > tiles / 2) splits = tiles / 2;
-        }
+        const size_t need = gqa_attention_workspace_bytes(batch, 1, heads, kv_heads, head_dim, kv_len);
+        const int splits = (need > 0 && workspace != nullptr && workspace_bytes >= need) ? decode_splits(batch, 1, heads, kv_heads, kv_len)
+                                                                                         : 1;   // too short: one pass
         return gqa_attention_packed(q, cache_k, cache_v, out, batch * kv_heads, group, head_dim, max_len, kv_len, splits, workspace,
                                     dtype, s);
     }
@@ -710,10 +719,14 @@ int gqa_attention_launch(const void* q, const void* cache_k, const void* cache_v
     int rc = make_tensor_map_2d(&p.map_q, q, static_cast<uint64_t>(batch) * q_len, static_cast<uint64_t>(heads) * head_dim,
                                 static_cast<uint64_t>(heads) * head_dim, kQTile, 64, dtype);
     if (rc != L32_OK) return rc;
-    const uint64_t kv_rows = static_cast<uint64_t>(batch) * kv_heads * max_len;
-    rc = make_tensor_map_2d(&p.map_k, cache_k, kv_rows, head_dim, head_dim, kKvTile, 64, dtype);
+    // K / V: one plane per (batch, kv head), cut at kv_len.  Masked keys get P = 0, but 0 * NaN and 0 * Inf are NaN in the
+    // P V product: the rows of the last tile beyond kv_len (stale cache capacity, or the next head's keys) must not reach
+    // shared memory with whatever they hold, so TMA fills them with zeros.
+    const uint64_t planes = static_cast<uint64_t>(batch) * kv_heads, plane_elems = static_cast<uint64_t>(max_len) * head_dim;
+    const uint64_t kv_rows = static_cast<uint64_t>(kv_len > 0 ? kv_len : 1);   // kv_len 0: no tile is loaded
+    rc = make_tensor_map_3d(&p.map_k, cache_k, planes, kv_rows, head_dim, head_dim, plane_elems, kKvTile, dtype);
     if (rc != L32_OK) return rc;
-    rc = make_tensor_map_2d(&p.map_v, cache_v, kv_rows, head_dim, head_dim, kKvTile, 64, dtype);
+    rc = make_tensor_map_3d(&p.map_v, cache_v, planes, kv_rows, head_dim, head_dim, plane_elems, kKvTile, dtype);
     if (rc != L32_OK) return rc;
     p.splits = splits > 1 ? splits : 1;
     if (p.splits > 1) {

@@ -900,6 +900,31 @@ int make_tensor_map_2d_sw(CUtensorMap* map, const void* ptr, uint64_t rows, uint
     return r == CUDA_SUCCESS ? L32_OK : L32_ERR_DRIVER;
 }
 
+int make_tensor_map_3d(CUtensorMap* map, const void* ptr, uint64_t planes, uint64_t rows, uint64_t cols, uint64_t ld_elems,
+                       uint64_t plane_elems, uint32_t box_rows, int dtype) {
+    EncodeTiledFn fn = encode_tiled_fn();
+    if (fn == nullptr) return L32_ERR_DRIVER;
+    if (!is_aligned16(ptr) || (ld_elems % 8) != 0 || (plane_elems % 8) != 0) return L32_ERR_BAD_ALIGN;
+    if (box_rows == 0 || box_rows > 256 || planes == 0 || rows == 0) return L32_ERR_BAD_SHAPE;
+    const cuuint64_t gdim[3] = {cols, rows, planes};
+    const cuuint64_t gstride[2] = {ld_elems * 2, plane_elems * 2};
+    const cuuint32_t box[3] = {64, box_rows, 1};
+    const cuuint32_t estride[3] = {1, 1, 1};
+    const CUtensorMapDataType dt = (dtype == L32_BF16) ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+    auto encode = [&] {
+        return fn(map, dt, 3, const_cast<void*>(ptr), gdim, gstride, box, estride, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    };
+    CUresult r = encode();
+    if ((r == CUDA_ERROR_INVALID_CONTEXT || r == CUDA_ERROR_NOT_INITIALIZED) && cudaFree(nullptr) == cudaSuccess)
+        r = encode();   // no current driver context on this thread yet: see make_tensor_map_2d_sw
+    if (r != CUDA_SUCCESS && getenv("L32_DEBUG") != nullptr)
+        fprintf(stderr, "[l32] cuTensorMapEncodeTiled (3-D) failed (%d): ptr %p planes %llu rows %llu cols %llu\n", static_cast<int>(r),
+                ptr, static_cast<unsigned long long>(planes), static_cast<unsigned long long>(rows),
+                static_cast<unsigned long long>(cols));
+    return r == CUDA_SUCCESS ? L32_OK : L32_ERR_DRIVER;
+}
+
 // Host-side view of the persistent kernels' tile sequences (tests/test_tile_order.py checks on the CPU that every tile is
 // visited exactly once and that every down tile of EPI_FFN_TP comes well after the act tiles it consumes).
 void debug_tile_order(int t, int tiles_m, int tiles_n, int group, int m_rotate, int il_world, int il_tpc, int il_rank, int* out3) {

@@ -187,5 +187,9 @@ int make_tensor_map_2d(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_
                        uint32_t box_rows, uint32_t box_cols, int dtype);
 int make_tensor_map_2d_sw(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint64_t ld_elems,
                           uint32_t box_rows, uint32_t box_cols, int dtype, int swizzle_bytes);
+// 3-D [planes, rows, cols] 16-bit tensor with rows `ld_elems` and planes `plane_elems` apart, box {64 cols, box_rows, 1 plane},
+// 128-byte swizzled.  A box row at or beyond `rows` of its plane is zero-filled, never read from the next plane.
+int make_tensor_map_3d(CUtensorMap* map, const void* ptr, uint64_t planes, uint64_t rows, uint64_t cols, uint64_t ld_elems,
+                       uint64_t plane_elems, uint32_t box_rows, int dtype);
 
 }  // namespace l32

@@ -176,6 +176,15 @@ L32_DEVICE void tma_load_2d(void* smem_dst, const CUtensorMap* map, uint64_t* ba
         "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "l"(hint)
         : "memory");
 }
+// 3-D tile load, completion on this CTA's mbarrier (elements outside the map's extent arrive as zeros).
+L32_DEVICE void tma_load_3d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int32_t c0, int32_t c1, int32_t c2,
+                            uint64_t hint) {
+    asm volatile(
+        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
+        " [%0], [%1, {%3, %4, %5}], [%2], %6;" ::"r"(smem_u32(smem_dst)),
+        "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "l"(hint)
+        : "memory");
+}
 // 2-D tile load issued by either CTA of a cta_group::2 pair; the transaction bytes are
 // credited to the LEADER (even) CTA's mbarrier at the same smem offset.
 L32_DEVICE void tma_load_2d_pair(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int32_t c0, int32_t c1,

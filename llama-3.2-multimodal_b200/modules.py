@@ -585,11 +585,11 @@ class GQAAttentionFunction(torch.autograd.Function):
 def _mask_causal_keep(attention_mask, b, t, kv_len):
     """The reference's Llama3Model mask (Model/model.py:304-319: causal + key padding) as (causal, key_keep [b, kv_len] | None).
     None means no masking at all; the key-padding row is read from the last query row, which sees every key the causal part
-    allows."""
+    allows.  A decode step (t = 1) reads it too: a [b, 1, 1, kv_len] mask pads keys of the cache like a prefill mask does."""
     if attention_mask is None:
         return False, None
     keep = None
-    if attention_mask.dim() == 4 and attention_mask.shape[-1] == kv_len and attention_mask.shape[-2] == t and t > 1:
+    if attention_mask.dim() == 4 and attention_mask.shape[-1] == kv_len and attention_mask.shape[-2] == t:
         keep = attention_mask[:, 0, -1, :] > (torch.finfo(attention_mask.dtype).min / 2)
         if keep.shape[0] != b:
             keep = keep.expand(b, -1)
