@@ -441,6 +441,15 @@ L32_API int l32_tp_reduce_partials(const void* slots, const uint32_t* flags, uin
  *   out3 = {problem (0 gate/up or plain, 1 down), m_tile, n_tile} of the t-th tile. */
 L32_API int l32_debug_tile_order(int kind, int t, const int* cfg, int* out3);
 
+/* Launch plan of the tiled GEMM for one (not grouped) problem D[m, n], as the library would launch it (no GPU needed).
+ *   epilogue : 0 plain store (256-column tiles), 1 fused gate/up + SwiGLU (n = intermediate size), 2 SwiGLU backward,
+ *              4 lm_head + cross entropy
+ *   cta_group: 0 = auto (2 above 128 rows), 1 or 2;  max_ctas: 0 = every SM;  num_sms: 0 = the current device's
+ *   out[7]   = {cta_group, tiles_m, tiles_n, n_act (act columns per tile of epilogue 1, else 128), raster_group (m-tiles
+ *              per raster group), num_tiles, ctas launched}.
+ * Reads the L32_SWIGLU_TILE_N and L32_RASTER_GROUP overrides like the launch does. */
+L32_API int l32_debug_gemm_plan(int epilogue, int m, int n, int cta_group, int max_ctas, int num_sms, int* out);
+
 /* Elementwise helpers (unfused reference points for tests / benchmarks of the fusion saving). */
 L32_API int l32_swiglu_act(const void* gate, const void* up, void* act, int64_t n, int dtype, void* stream);
 

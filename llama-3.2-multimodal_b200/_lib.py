@@ -61,6 +61,7 @@ SIGNATURES = {
     "l32_gemm": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_int64, c_int, c_void_p, c_int64, c_void_p, c_int64,
                          c_void_p, c_int64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "l32_debug_tile_order": (c_int, [c_int, c_int, c_void_p, c_void_p]),
+    "l32_debug_gemm_plan": (c_int, [c_int] * 6 + [c_void_p]),
     "l32_swiglu_act": (c_int, [c_void_p] * 3 + [c_int64, c_int, c_void_p]),
     "l32_tp_peer_copy": (c_int, [c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_int, c_void_p]),
     "l32_tp_signal": (c_int, [c_void_p, c_int, c_int, ctypes.c_uint32, c_void_p, c_void_p]),

@@ -1165,6 +1165,12 @@ int l32_debug_tile_order(int kind, int t, const int* cfg, int* out3) {
     return L32_OK;
 }
 
+int l32_debug_gemm_plan(int epilogue, int m, int n, int cta_group, int max_ctas, int num_sms, int* out) {
+    if (out == nullptr) return L32_ERR_NULL;
+    if (epilogue != EPI_STORE && epilogue != EPI_SWIGLU && epilogue != EPI_SWIGLU_BWD && epilogue != EPI_CE) return L32_ERR_BAD_SHAPE;
+    return debug_gemm_plan(epilogue, m, n, cta_group, max_ctas, num_sms, out);
+}
+
 int l32_swiglu_act(const void* gate, const void* up, void* act, int64_t n, int dtype, void* stream) {
     if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
     if (n < 0 || (n % 8) != 0) return L32_ERR_BAD_SHAPE;

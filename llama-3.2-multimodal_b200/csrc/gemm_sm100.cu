@@ -780,8 +780,9 @@ EncodeTiledFn encode_tiled_fn() {
     return fn;
 }
 
+// ctas: grid size from plan_ctas (a multiple of kCtaGroup)
 template <int kCtaGroup, int kEpi, typename T>
-int launch(const GemmKernelParams& kp, int num_tiles, int max_ctas, cudaStream_t s) {
+int launch(const GemmKernelParams& kp, int ctas, cudaStream_t s) {
     using Cfg = TileCfg<kCtaGroup>;
     auto* kernel = gemm_kernel<kCtaGroup, kEpi, T>;
     static bool configured_dev[kMaxDevices] = {};   // per instantiation and device
@@ -791,11 +792,7 @@ int launch(const GemmKernelParams& kp, int num_tiles, int max_ctas, cudaStream_t
         if (e != cudaSuccess) return static_cast<int>(e);
         configured = true;
     }
-    int ctas = num_sms();
-    if (max_ctas > 0 && max_ctas < ctas) ctas = max_ctas;
     int clusters = ctas / kCtaGroup;
-    if (clusters > num_tiles) clusters = num_tiles;
-    if (clusters < 1) clusters = 1;
 
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(static_cast<unsigned>(clusters * kCtaGroup));
@@ -835,17 +832,76 @@ int launch(const GemmKernelParams& kp, int num_tiles, int max_ctas, cudaStream_t
 }
 
 template <int kCtaGroup, typename T>
-int launch_epi(const GemmKernelParams& kp, int epi, int num_tiles, int max_ctas, cudaStream_t s) {
+int launch_epi(const GemmKernelParams& kp, int epi, int ctas, cudaStream_t s) {
     switch (epi) {
-        case EPI_STORE: return launch<kCtaGroup, EPI_STORE, T>(kp, num_tiles, max_ctas, s);
-        case EPI_CE: return launch<kCtaGroup, EPI_CE, T>(kp, num_tiles, max_ctas, s);
-        case EPI_SWIGLU: return launch<kCtaGroup, EPI_SWIGLU, T>(kp, num_tiles, max_ctas, s);
-        case EPI_SWIGLU_BWD: return launch<kCtaGroup, EPI_SWIGLU_BWD, T>(kp, num_tiles, max_ctas, s);
+        case EPI_STORE: return launch<kCtaGroup, EPI_STORE, T>(kp, ctas, s);
+        case EPI_CE: return launch<kCtaGroup, EPI_CE, T>(kp, ctas, s);
+        case EPI_SWIGLU: return launch<kCtaGroup, EPI_SWIGLU, T>(kp, ctas, s);
+        case EPI_SWIGLU_BWD: return launch<kCtaGroup, EPI_SWIGLU_BWD, T>(kp, ctas, s);
         case EPI_FFN_TP:
-            if constexpr (kCtaGroup == 2) return launch<2, EPI_FFN_TP, T>(kp, num_tiles, max_ctas, s);
+            if constexpr (kCtaGroup == 2) return launch<2, EPI_FFN_TP, T>(kp, ctas, s);
             else return L32_ERR_BAD_SHAPE;
         default: return L32_ERR_BAD_SHAPE;
     }
+}
+
+// CTAs of the persistent grid: one cluster of cta_group CTAs per SM pair (or SM), never more clusters than tiles.
+int plan_ctas(int num_tiles, int cta_group, int max_ctas, int sms) {
+    int ctas = sms;
+    if (max_ctas > 0 && max_ctas < ctas) ctas = max_ctas;
+    int clusters = ctas / cta_group;
+    if (clusters > num_tiles) clusters = num_tiles;
+    if (clusters < 1) clusters = 1;
+    return clusters * cta_group;
+}
+
+// The host decisions of one (not grouped) launch of gemm_sm100.  EPI_FFN_TP adds its down tiles, and a grouped launch its
+// problems' tiles, to num_tiles afterwards (and re-plans ctas).
+struct GemmPlan {
+    int cta_group, tiles_m, tiles_n, n_act, raster_group, num_tiles, ctas;
+};
+
+int plan_gemm(int epilogue, int m, int n, int cta_group_req, int raster_group_req, int max_ctas, int sms, GemmPlan& pl) {
+    const bool swiglu_like = epilogue == EPI_SWIGLU || epilogue == EPI_FFN_TP;
+    int cta_group = cta_group_req;
+    if (cta_group == 0) cta_group = (m > kBlockM) ? 2 : 1;
+    if (cta_group != 1 && cta_group != 2) return L32_ERR_BAD_SHAPE;
+    pl.cta_group = cta_group;
+    const int tile_m = kBlockM * cta_group;
+    pl.tiles_m = (m + tile_m - 1) / tile_m;
+    // EPI_SWIGLU: pick the act-column tile width (multiple of 16) that minimises waves x tile cost -- e.g. a
+    // tensor-parallel shard of 1792 act columns is 7 waves of 112 columns instead of 7 waves of 128 (the last one
+    // nearly empty).  Ties go to the wider tile.
+    int n_act = 128;
+    if (swiglu_like) {
+        int ctas = sms;
+        if (max_ctas > 0 && max_ctas < ctas) ctas = max_ctas;
+        const long long clusters = ctas / cta_group > 0 ? ctas / cta_group : 1;
+        long long best = -1;
+        for (int cand = 128; cand >= 64; cand -= 16) {
+            const long long tiles = static_cast<long long>(pl.tiles_m) * ((n + cand - 1) / cand);
+            const long long cost = ((tiles + clusters - 1) / clusters) * (cand + 12);   // + fixed per-tile overhead
+            if (best < 0 || cost < best) { best = cost; n_act = cand; }
+        }
+        if (const char* env = getenv("L32_SWIGLU_TILE_N")) {   // tuning knob for experiments only
+            const int v = atoi(env);
+            if (v >= 16 && v <= 128 && (v % 16) == 0) n_act = v;
+        }
+    }
+    pl.n_act = n_act;
+    const int tile_n_out = swiglu_like ? n_act : 256;
+    pl.tiles_n = (n + tile_n_out - 1) / tile_n_out;
+    // m-tiles per raster group: 2048 rows for the plain / backward epilogues, 4096 rows for the fused gate/up GEMM (its B
+    // operand -- two weight matrices -- is the big one: larger groups re-read it from HBM half as often; measured
+    // +1.8 % at the 11B shape, scripts/raster_ab.py)
+    pl.raster_group = raster_group_req > 0 ? raster_group_req : (swiglu_like ? 32 : 16) / cta_group;
+    if (const char* env = getenv("L32_RASTER_GROUP")) {   // tuning knob for experiments only
+        const int v = atoi(env);
+        if (v > 0) pl.raster_group = v;
+    }
+    pl.num_tiles = pl.tiles_m * pl.tiles_n;
+    pl.ctas = plan_ctas(pl.num_tiles, cta_group, max_ctas, sms);
+    return L32_OK;
 }
 
 }  // namespace
@@ -937,6 +993,16 @@ void debug_ffn_tile_order(int t, int tiles_m, int n_gu, int n_dn, int group, int
     const TileCoord c = ffn_tile_coord(t, o);
     out3[0] = c.prob; out3[1] = c.m_blk; out3[2] = c.n_blk;
 }
+// The launch plan gemm_sm100 would use (tests/test_gemm_plan.py restates it; the GPU tests pick their shapes with it).
+int debug_gemm_plan(int epilogue, int m, int n, int cta_group, int max_ctas, int sms, int* out7) {
+    if (m <= 0 || n <= 0 || sms < 0) return L32_ERR_BAD_SHAPE;
+    GemmPlan pl;
+    const int rc = plan_gemm(epilogue, m, n, cta_group, 0, max_ctas, sms > 0 ? sms : num_sms(), pl);
+    if (rc != L32_OK) return rc;
+    const int v[7] = {pl.cta_group, pl.tiles_m, pl.tiles_n, pl.n_act, pl.raster_group, pl.num_tiles, pl.ctas};
+    for (int i = 0; i < 7; ++i) out7[i] = v[i];
+    return L32_OK;
+}
 
 int gemm_sm100(const GemmProblem& g, cudaStream_t s) {
     const bool ffn_tp = g.epilogue == EPI_FFN_TP;
@@ -955,9 +1021,10 @@ int gemm_sm100(const GemmProblem& g, cudaStream_t s) {
         if (!is_aligned16(g.e[0]) || !is_aligned16(g.e[1])) return L32_ERR_BAD_ALIGN;
     }
 
-    int cta_group = g.cta_group;
-    if (cta_group == 0) cta_group = (g.m > kBlockM) ? 2 : 1;
-    if (cta_group != 1 && cta_group != 2) return L32_ERR_BAD_SHAPE;
+    const int sms = num_sms();
+    GemmPlan plan;
+    if (const int rc = plan_gemm(g.epilogue, g.m, g.n, g.cta_group, g.raster_group, g.max_ctas, sms, plan); rc != L32_OK) return rc;
+    const int cta_group = plan.cta_group;
     if (ffn_tp) {
         if (cta_group != 2 || g.dn.w == nullptr || g.dn.n <= 0 || (g.dn.n % 8) != 0 || g.dn.act_done == nullptr ||
             g.rs.world < 1 || g.d[0] == nullptr || g.d[1] != nullptr || g.a[0].mn_major || g.bias[0] != nullptr ||
@@ -973,37 +1040,11 @@ int gemm_sm100(const GemmProblem& g, cudaStream_t s) {
     kp.a_mn_major = g.a[0].mn_major;
     kp.b_mn_major = g.b[0].mn_major;
     const int tile_m = kBlockM * cta_group;
-    kp.tiles_m = (g.m + tile_m - 1) / tile_m;
-    // EPI_SWIGLU: pick the act-column tile width (multiple of 16) that minimises waves x tile cost -- e.g. a
-    // tensor-parallel shard of 1792 act columns is 7 waves of 112 columns instead of 7 waves of 128 (the last one
-    // nearly empty).  Ties go to the wider tile.
-    int n_act = 128;
-    if (swiglu_like) {
-        int ctas = num_sms();
-        if (g.max_ctas > 0 && g.max_ctas < ctas) ctas = g.max_ctas;
-        const long long clusters = ctas / cta_group > 0 ? ctas / cta_group : 1;
-        long long best = -1;
-        for (int cand = 128; cand >= 64; cand -= 16) {
-            const long long tiles = static_cast<long long>(kp.tiles_m) * ((g.n + cand - 1) / cand);
-            const long long cost = ((tiles + clusters - 1) / clusters) * (cand + 12);   // + fixed per-tile overhead
-            if (best < 0 || cost < best) { best = cost; n_act = cand; }
-        }
-        if (const char* env = getenv("L32_SWIGLU_TILE_N")) {   // tuning knob for experiments only
-            const int v = atoi(env);
-            if (v >= 16 && v <= 128 && (v % 16) == 0) n_act = v;
-        }
-    }
+    kp.tiles_m = plan.tiles_m;
+    const int n_act = plan.n_act;
     kp.n_act = n_act;
-    const int tile_n_out = swiglu_like ? n_act : 256;
-    kp.tiles_n = (g.n + tile_n_out - 1) / tile_n_out;
-    // m-tiles per raster group: 2048 rows for the plain / backward epilogues, 4096 rows for the fused gate/up GEMM (its B
-    // operand -- two weight matrices -- is the big one: larger groups re-read it from HBM half as often; measured
-    // +1.8 % at the 11B shape, scripts/raster_ab.py)
-    kp.raster_group = g.raster_group > 0 ? g.raster_group : (swiglu_like ? 32 : 16) / cta_group;
-    if (const char* env = getenv("L32_RASTER_GROUP")) {   // tuning knob for experiments only
-        const int v = atoi(env);
-        if (v > 0) kp.raster_group = v;
-    }
+    kp.tiles_n = plan.tiles_n;
+    kp.raster_group = plan.raster_group;
     kp.idesc = make_idesc_f16(g.dtype == L32_BF16, static_cast<uint32_t>(tile_m),
                               swiglu_like ? static_cast<uint32_t>(2 * n_act) : static_cast<uint32_t>(kAccCols),
                               g.a[0].mn_major != 0, g.b[0].mn_major != 0);
@@ -1089,8 +1130,9 @@ int gemm_sm100(const GemmProblem& g, cudaStream_t s) {
         kp.k[0] = g.k[0];
         kp.m_il_world = 0;
         if (g.ag.world <= 1) kp.m_rotate = 0;   // all-gather: own rows first (setup_allgather's rotation), in every problem
-        if (g.dtype == L32_BF16) return launch_epi<2, __nv_bfloat16>(kp, EPI_STORE, start, g.max_ctas, s);
-        return launch_epi<2, __half>(kp, EPI_STORE, start, g.max_ctas, s);
+        const int ctas = plan_ctas(start, 2, g.max_ctas, sms);
+        if (g.dtype == L32_BF16) return launch_epi<2, __nv_bfloat16>(kp, EPI_STORE, ctas, s);
+        return launch_epi<2, __half>(kp, EPI_STORE, ctas, s);
     }
     if (g.epilogue == EPI_CE) {
         if (g.ce.labels == nullptr || g.ce.partials == nullptr || g.ce.target == nullptr) return L32_ERR_NULL;
@@ -1122,7 +1164,7 @@ int gemm_sm100(const GemmProblem& g, cudaStream_t s) {
         if (grp > kp.tiles_m) grp = kp.tiles_m;
         while (kp.tiles_m % grp != 0) --grp;
         kp.raster_group = grp;
-        int ctas = num_sms();
+        int ctas = sms;
         if (g.max_ctas > 0 && g.max_ctas < ctas) ctas = g.max_ctas;
         const int a_tiles = grp * kp.tiles_n;
         kp.ffn_prefix = a_tiles < ctas / 2 ? a_tiles : ctas / 2;   // one wave of gate/up-only tiles at the head of a round
@@ -1131,15 +1173,16 @@ int gemm_sm100(const GemmProblem& g, cudaStream_t s) {
             if (v >= 0 && v <= a_tiles) kp.ffn_prefix = v;
         }
         kp.m_il_world = 0;
+        plan.num_tiles = kp.tiles_m * (kp.tiles_n + kp.tiles_n_dn);
+        plan.ctas = plan_ctas(plan.num_tiles, cta_group, g.max_ctas, sms);
     }
 
-    const int num_tiles = kp.tiles_m * (kp.tiles_n + kp.tiles_n_dn);
     if (g.dtype == L32_BF16) {
-        if (cta_group == 2) return launch_epi<2, __nv_bfloat16>(kp, g.epilogue, num_tiles, g.max_ctas, s);
-        return launch_epi<1, __nv_bfloat16>(kp, g.epilogue, num_tiles, g.max_ctas, s);
+        if (cta_group == 2) return launch_epi<2, __nv_bfloat16>(kp, g.epilogue, plan.ctas, s);
+        return launch_epi<1, __nv_bfloat16>(kp, g.epilogue, plan.ctas, s);
     }
-    if (cta_group == 2) return launch_epi<2, __half>(kp, g.epilogue, num_tiles, g.max_ctas, s);
-    return launch_epi<1, __half>(kp, g.epilogue, num_tiles, g.max_ctas, s);
+    if (cta_group == 2) return launch_epi<2, __half>(kp, g.epilogue, plan.ctas, s);
+    return launch_epi<1, __half>(kp, g.epilogue, plan.ctas, s);
 }
 
 }  // namespace l32

@@ -127,6 +127,7 @@ struct GemmProblem {
 int gemm_sm100(const GemmProblem& p, cudaStream_t s);   // returns L32_* / cudaError_t
 void debug_tile_order(int t, int tiles_m, int tiles_n, int group, int m_rotate, int il_world, int il_tpc, int il_rank, int* out3);
 void debug_ffn_tile_order(int t, int tiles_m, int n_gu, int n_dn, int group, int m_rotate, int prefix, int* out3);
+int debug_gemm_plan(int epilogue, int m, int n, int cta_group, int max_ctas, int sms, int* out7);
 
 // ---- elementwise.cu (n = element count, multiple of 8)
 cudaError_t swiglu_bwd_elementwise(const void* d_act, const void* gate, const void* up, void* d_gate, void* d_up,
