@@ -57,7 +57,8 @@ extern "C" {
  *    l32_rmsnorm_backward_add, l32_block_tail_forward_ex, l32_linear_lora_forward / _backward, l32_lm_head_ce_*,
  *    l32_rope_kv_append, l32_gqa_attention_forward; later, additively: l32_gqa_attention_forward_train / _backward, and
  *    the tensor-parallel attention GEMMs l32_tp_linear_group_forward_allgather, l32_tp_linear_forward_allgather and
- *    l32_tp_linear_group_backward_dx_reduce_scatter. */
+ *    l32_tp_linear_group_backward_dx_reduce_scatter, and the paged KV cache l32_rope_kv_append_paged and
+ *    l32_gqa_attention_forward_paged. */
 L32_API int l32_abi_version(void);
 /* Number of CUDA kernels this library has launched in the calling process so far (monotonic). */
 L32_API unsigned long long l32_kernel_launch_count(void);
@@ -309,6 +310,45 @@ L32_API int l32_gqa_attention_backward(const void* d_ctx, const void* q_rot, con
                                        void* dv, void* workspace, size_t workspace_bytes, int batch, int q_len, int heads,
                                        int kv_heads, int head_dim, int max_len, int causal, float rope_base, int dtype,
                                        void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Paged KV cache: per-sequence lengths in device memory, keys in fixed-size pages named by a block table (inference only).
+ * Layout:
+ *   page       : L32_KV_PAGE = 64 tokens, the attention kernel's key tile (one key tile is exactly one page).
+ *   pool_k / pool_v : [num_pages, kv_heads, L32_KV_PAGE, head_dim] per layer, one (page, kv head) slice = 64 x head_dim
+ *                contiguous elements.  Page index p names the same slot in every layer's pool (one allocator serves all layers).
+ *   block_table : int32 [batch, max_pages_per_seq]; logical page j of sequence b is block_table[b][j].
+ *   past_lens   : int32 [batch], tokens already cached for sequence b.
+ *   new_lens    : int32 [batch] or NULL: tokens this call appends for sequence b (NULL: every row has q_len).  The keys a call
+ *                sees for sequence b are [0, past_lens[b] + new_lens[b]); its query i sits at position past_lens[b] + i.
+ *   q, ctx      : [batch, q_len, heads * head_dim], right-padded: query rows i >= new_lens[b] are padding.
+ * CONTRACT on stale rows: every row of a page at or beyond its sequence's length must hold FINITE values (they are multiplied by
+ *   zero probabilities, and 0 * NaN is NaN in P V).  Pools that start zeroed and are written only by l32_rope_kv_append_paged
+ *   keep this without zeroing a page when it is handed to another sequence.
+ * The table and length values live in device memory and are TRUSTED: every page index must lie in [0, num_pages), every
+ *   past_lens[b] + new_lens[b] must be <= max_pages_per_seq * 64 (and <= max_kv_len for the attention) and every page a call
+ *   reads or writes must be in the table.  The caller (the Python PagedKVCache) checks them when it builds them.
+ * Same rules as the other entry points: nothing allocates or synchronises, everything is graph-capturable, and argument errors
+ * return L32_ERR_* before any launch.
+ */
+#define L32_KV_PAGE 64
+/* RoPE on q (in place, every row) and on k_new while it is stored at position past_lens[b] + t of sequence b, i.e. row
+ * (pos % 64) of page block_table[b][pos / 64]; v_new stored next to it.  Tokens t >= new_lens[b] write nothing to the pools.
+ * position_ids [batch, q_len] int64 as in l32_rope_kv_append.  head_dim 64 or 128. */
+L32_API int l32_rope_kv_append_paged(void* q, const void* k_new, const void* v_new, const int64_t* position_ids, void* pool_k,
+                                     void* pool_v, const int32_t* block_table, const int32_t* past_lens, const int32_t* new_lens,
+                                     int batch, int q_len, int heads, int kv_heads, int head_dim, int num_pages, int max_pages_per_seq,
+                                     float rope_base, int dtype, void* stream);
+/* ctx = causal attention of each sequence's queries over its own keys (for one query per sequence that is no mask at all).
+ * Padded query rows yield exact zeros.  max_kv_len: a host bound >= every past_lens[b] + new_lens[b]; it sizes the split-KV
+ * plan of a decode step (q_len == 1) exactly as kv_len does for l32_gqa_attention_forward, so the workspace is
+ * l32_gqa_attention_workspace_bytes(batch, q_len, heads, kv_heads, head_dim, max_kv_len) (optional, as there).  With uniform
+ * lengths, max_kv_len equal to them and the same keys laid out in pages, the result is bit-identical to
+ * l32_gqa_attention_forward's. */
+L32_API int l32_gqa_attention_forward_paged(const void* q, const void* pool_k, const void* pool_v, const int32_t* block_table,
+                                            const int32_t* past_lens, const int32_t* new_lens, void* ctx, void* workspace,
+                                            size_t workspace_bytes, int batch, int q_len, int heads, int kv_heads, int head_dim,
+                                            int num_pages, int max_pages_per_seq, int max_kv_len, int dtype, void* stream);
 
 /* General tiled GEMM used by the entry points above (exposed for tests, tuning and the tensor-parallel
  * host code):  D[m,n] = A[m,k] B[n,k]^T  (+ A1 B1^T when a1 != NULL).

@@ -12,6 +12,7 @@ from .modules import (  # noqa: F401
     GQAAttentionFunction,
     GroupQueryAttention,
     KVCache,
+    PagedKVCache,
     LLAMARMSNorm,
     LMHeadCEFunction,
     Linear_LORA,
@@ -32,5 +33,5 @@ __all__ = [
     "FFNFunction", "FFNLoRAFunction", "FusedFeedForward", "FusedFeedforward", "FusedSwiGLU", "LLAMARMSNorm", "Linear_LORA",
     "LinearFunction", "RMSNormFunction", "SwiGLUFunction", "block_tail", "convert_feedforward_to_fused", "convert_instances",
     "patch_reference", "BlockTailFunction", "LinearLoRAFunction", "chain_block_norms", "LMHeadCEFunction", "lm_head_loss", "shift_labels", "GroupQueryAttention", "KVCache",
-    "GQAAttentionFunction",
+    "GQAAttentionFunction", "PagedKVCache",
 ]

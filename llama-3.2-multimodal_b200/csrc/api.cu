@@ -808,6 +808,47 @@ int l32_gqa_attention_backward(const void* d_ctx, const void* q_rot, const void*
                                   as_stream(stream));
 }
 
+// Paged KV cache (no reference counterpart: the reference's cache is one torch.cat'ed tensor per layer).  Only the host-side
+// arguments can be checked here; the table and length values in device memory are trusted (include/l32_ffn.h).
+static bool paged_shape_ok(int batch, int q_len, int heads, int kv_heads, int head_dim, int num_pages, int max_pages_per_seq) {
+    return batch >= 0 && q_len >= 0 && heads > 0 && kv_heads > 0 && (heads % kv_heads) == 0 && (head_dim == 64 || head_dim == 128) &&
+           num_pages > 0 && max_pages_per_seq > 0 && static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE <= 0x7fffffffll &&
+           static_cast<long long>(num_pages) * kv_heads <= 0x7fffffffll;
+}
+
+int l32_rope_kv_append_paged(void* q, const void* k_new, const void* v_new, const int64_t* position_ids, void* pool_k, void* pool_v,
+                             const int32_t* block_table, const int32_t* past_lens, const int32_t* new_lens, int batch, int q_len,
+                             int heads, int kv_heads, int head_dim, int num_pages, int max_pages_per_seq, float rope_base, int dtype,
+                             void* stream) {
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (!paged_shape_ok(batch, q_len, heads, kv_heads, head_dim, num_pages, max_pages_per_seq) || !(rope_base > 1.0f))
+        return L32_ERR_BAD_SHAPE;
+    if (batch == 0 || q_len == 0) return L32_OK;
+    if (q == nullptr || k_new == nullptr || v_new == nullptr || position_ids == nullptr || pool_k == nullptr || pool_v == nullptr ||
+        block_table == nullptr || past_lens == nullptr)
+        return L32_ERR_NULL;
+    return rope_kv_append_paged(q, k_new, v_new, reinterpret_cast<const long long*>(position_ids), pool_k, pool_v, block_table,
+                                past_lens, new_lens, batch, q_len, heads, kv_heads, head_dim, max_pages_per_seq, rope_base, dtype,
+                                as_stream(stream));
+}
+
+int l32_gqa_attention_forward_paged(const void* q, const void* pool_k, const void* pool_v, const int32_t* block_table,
+                                    const int32_t* past_lens, const int32_t* new_lens, void* ctx, void* workspace, size_t workspace_bytes,
+                                    int batch, int q_len, int heads, int kv_heads, int head_dim, int num_pages, int max_pages_per_seq,
+                                    int max_kv_len, int dtype, void* stream) {
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (!paged_shape_ok(batch, q_len, heads, kv_heads, head_dim, num_pages, max_pages_per_seq) || max_kv_len < 0 ||
+        static_cast<long long>(max_kv_len) > static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE)
+        return L32_ERR_BAD_SHAPE;
+    if (batch == 0 || q_len == 0) return L32_OK;
+    if (q == nullptr || pool_k == nullptr || pool_v == nullptr || block_table == nullptr || past_lens == nullptr || ctx == nullptr)
+        return L32_ERR_NULL;
+    if (!is_aligned16(q) || !is_aligned16(pool_k) || !is_aligned16(pool_v) || !is_aligned16(ctx)) return L32_ERR_BAD_ALIGN;
+    if (workspace != nullptr && !is_aligned16(workspace)) return L32_ERR_WORKSPACE;
+    return gqa_attention_paged(q, pool_k, pool_v, block_table, past_lens, new_lens, ctx, workspace, workspace_bytes, batch, q_len, heads,
+                               kv_heads, head_dim, num_pages, max_pages_per_seq, max_kv_len, dtype, as_stream(stream));
+}
+
 int l32_gemm(const void* a, int64_t lda, int a_mn_major, const void* b, int64_t ldb, int b_mn_major, const void* a1,
              int64_t lda1, const void* b1, int64_t ldb1, void* d, int64_t ldd, int m, int n, int k, int k1, int dtype,
              int cta_group, int max_ctas, void* stream) {

@@ -47,7 +47,17 @@ struct AttnParams {
     float2* part_ml;     // [batch][heads][splits][q_len] (m_ref in the log2 domain, l)
     float* lse;          // optional [batch, heads, q_len] (training): m_ref + log2(l) in the log2 domain, +inf for a row that
                          // sees no key (the backward then forms exact zero probabilities for it).  Never with split-KV.
+    // Paged cache (kPaged instances only).  map_k / map_v are then {d, kKvTile, num_pages * page_kv_heads}: key tile t of a
+    // sequence is page block_table[seq][t], plane page * page_kv_heads + kv head.  kv_len / past_len / tiles_per_split above
+    // are unused: each CTA reads its sequence's lengths from device memory and divides its own tiles over the splits.
+    const int* block_table;   // [sequences, pages_per_seq]
+    const int* past_lens;     // [sequences]
+    const int* new_lens;      // [sequences], or null: every sequence has q_len new tokens (the packed decode: one)
+    int pages_per_seq, page_kv_heads;
+    int packed;               // packed decode: CTA batch index = sequence * page_kv_heads + kv head, its q_len rows are the
+                              // query heads of ONE query
 };
+static_assert(L32_KV_PAGE == kKvTile, "a KV-cache page is one key tile");
 
 // L32_ATT_NOEXP / L32_ATT_NOPV / L32_ATT_NOLD: experiment builds only (wrong results) -- what the kernel costs without the
 // exponentials, without the P V MMAs, without the S reads from TMEM.
@@ -85,7 +95,8 @@ L32_DEVICE uint64_t add_f32x2(uint64_t a, uint64_t b) {
 }
 
 // kLse: training forward, also stores the per-row log-sum-exp (a separate instantiation: the inference kernel is unchanged)
-template <int kD, typename T, bool kLse>
+// kPaged: K / V from a paged cache, lengths per sequence from device memory (AttnParams, "paged cache")
+template <int kD, typename T, bool kLse, bool kPaged>
 __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ AttnParams p) {
     constexpr int kDAtoms = kD / 64;                       // 64-element (128-byte) column blocks of a head
     constexpr int kQBytes = kQTile * kD * 2;
@@ -149,13 +160,31 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
     pdl_launch_dependents();
     pdl_wait_prior_grid();
 
+    // paged: the CTA's sequence, its kv head in the pool and its lengths (written by earlier work of the stream).  Query rows
+    // [q_rows, q_len) are right padding of a ragged call: they see no key and store zeros.
+    int kv_len = p.kv_len, past_len = p.past_len, q_rows = p.q_len, tiles_per_split = p.tiles_per_split;
+    int seq = b, kvh_pool = kvh;
+    if constexpr (kPaged) {
+        if (p.packed) {
+            seq = b / p.page_kv_heads;
+            kvh_pool = b % p.page_kv_heads;
+        }
+        past_len = p.past_lens[seq];
+        const int n_new = p.new_lens != nullptr ? p.new_lens[seq] : (p.packed ? 1 : p.q_len);
+        kv_len = past_len + n_new;
+        q_rows = p.packed ? (n_new > 0 ? p.q_len : 0) : min(n_new, p.q_len);
+    }
     // keys this query tile can see: [0, hi)
-    const int q_last = min(q0 + kQTile, p.q_len) - 1;
-    int hi = p.kv_len;
-    if (p.causal) hi = min(hi, p.past_len + q_last + 1);
+    const int q_last = min(q0 + kQTile, q_rows) - 1;
+    int hi = kv_len;
+    if (p.causal) hi = min(hi, past_len + q_last + 1);
+    if constexpr (kPaged) {
+        if (q_last < q0) hi = 0;                                          // the whole query tile is padding
+    }
     const int total_tiles = (hi + kKvTile - 1) / kKvTile;
-    const int tile0 = split * p.tiles_per_split;                          // first key tile of this CTA (0 without split-KV)
-    const int ntiles = p.splits > 1 ? max(0, min(p.tiles_per_split, total_tiles - tile0)) : total_tiles;
+    if constexpr (kPaged) tiles_per_split = (total_tiles + p.splits - 1) / p.splits;   // the host plan, per sequence
+    const int tile0 = split * tiles_per_split;                            // first key tile of this CTA (0 without split-KV)
+    const int ntiles = p.splits > 1 ? max(0, min(tiles_per_split, total_tiles - tile0)) : total_tiles;
     const int kv_plane = b * p.kv_heads + kvh;
     const int key0 = tile0 * kKvTile;
 
@@ -166,23 +195,43 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
         // CTA barrier waiting for it).
         if (ntiles > 0 && elect_one()) {   // elect.sync: ptxas knows the branch is single-lane (a lane == 0 test makes it wrap every
                                               // tcgen05.mma / TMA instruction in an ELECT ... BRA.U.ANY loop: ~140 clocks per MMA)
-            // K tile, K-major: [64 keys][64 dims] per column block;  V tile: the same boxes, consumed as an MN-major B operand
-            auto load_k = [&](int t) {
+            // K tile, K-major: [64 keys][64 dims] per column block;  V tile: the same boxes, consumed as an MN-major B operand.
+            // pg: paged, the pool page of tile t
+            auto load_k = [&](int t, int pg) {
                 const int s = t & 1;
                 mbar_arrive_expect_tx(&bar_k[s], kKBytes);
 #pragma unroll
-                for (int a = 0; a < kDAtoms; ++a)
-                    tma_load_3d(sk + s * kKBytes + a * (kKvTile * 128), &p.map_k, &bar_k[s], a * 64, key0 + t * kKvTile, kv_plane,
-                                kEvictNormal);
+                for (int a = 0; a < kDAtoms; ++a) {
+                    if constexpr (kPaged)
+                        tma_load_3d(sk + s * kKBytes + a * (kKvTile * 128), &p.map_k, &bar_k[s], a * 64, 0,
+                                    pg * p.page_kv_heads + kvh_pool, kEvictNormal);
+                    else
+                        tma_load_3d(sk + s * kKBytes + a * (kKvTile * 128), &p.map_k, &bar_k[s], a * 64, key0 + t * kKvTile, kv_plane,
+                                    kEvictNormal);
+                }
             };
-            auto load_v = [&](int t) {
+            auto load_v = [&](int t, int pg) {
                 const int s = t & 1;
                 mbar_arrive_expect_tx(&bar_v[s], kKBytes);
 #pragma unroll
-                for (int a = 0; a < kDAtoms; ++a)
-                    tma_load_3d(sv + s * kKBytes + a * (kKvTile * 128), &p.map_v, &bar_v[s], a * 64, key0 + t * kKvTile, kv_plane,
-                                kEvictNormal);
+                for (int a = 0; a < kDAtoms; ++a) {
+                    if constexpr (kPaged)
+                        tma_load_3d(sv + s * kKBytes + a * (kKvTile * 128), &p.map_v, &bar_v[s], a * 64, 0,
+                                    pg * p.page_kv_heads + kvh_pool, kEvictNormal);
+                    else
+                        tma_load_3d(sv + s * kKBytes + a * (kKvTile * 128), &p.map_v, &bar_v[s], a * 64, key0 + t * kKvTile, kv_plane,
+                                    kEvictNormal);
+                }
             };
+            // Paged: the block-table entries are read a tile before the load that needs them (pg2 / pg3 = pages of tiles
+            // t + 2 / t + 3 at step t), so no global-load latency sits in the TMA issue chain.
+            const int* pages = nullptr;
+            int pg0 = 0, pg1 = 0, pg2 = 0, pg3 = 0;
+            auto page = [&](int t) { return t < ntiles ? __ldg(pages + t) : 0; };
+            if constexpr (kPaged) {
+                pages = p.block_table + static_cast<size_t>(seq) * p.pages_per_seq + tile0;
+                pg0 = page(0); pg1 = page(1); pg2 = page(2); pg3 = page(3);
+            }
             // S[128, 64] = Q[128, kD] K[64, kD]^T of tile t into accumulator t & 1
             const uint32_t q_addr = smem_u32(sq);
             auto issue_s = [&](int t) {
@@ -203,10 +252,10 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
 #pragma unroll
             for (int a = 0; a < kDAtoms; ++a)
                 tma_load_2d(sq + a * (kQTile * 128), &p.map_q, bar_q, head * kD + a * 64, b * p.q_len + q0, kEvictNormal);
-            load_k(0);
-            if (ntiles > 1) load_k(1);
-            load_v(0);
-            if (ntiles > 1) load_v(1);
+            load_k(0, pg0);
+            if (ntiles > 1) load_k(1, pg1);
+            load_v(0, pg0);
+            if (ntiles > 1) load_v(1, pg1);
             // P (16-bit) is written by the softmax warps over the first 32 columns of the S accumulator it was computed from,
             // and P V takes it from there (A operand in tensor memory): no shared-memory P tile, no generic -> async proxy
             // fence.  The tensor pipe executes in issue order, so S of tile t + 2 -- issued right behind P V of tile t --
@@ -216,10 +265,12 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
             if (ntiles > 1) issue_s(1);
             if (ntiles > 2) {                             // K stage 0 is free once S of tile 0 is complete
                 mbar_wait(&bar_s[0], 0);
-                load_k(2);
+                load_k(2, pg2);
             }
             for (int t = 0; t < ntiles; ++t) {
                 const int s = t & 1;
+                int pg_next = 0;
+                if constexpr (kPaged) pg_next = page(t + 4);   // used at step t + 1: its latency hides behind this step's waits
                 // O[128, kD] (+)= P[128, 64] V[64, kD]   (V consumed MN-major: [64 keys][kD]); tile 0 overwrites
                 mbar_wait(&bar_p[s], (t >> 1) & 1u);
                 mbar_wait(&bar_v[s], (t >> 1) & 1u);
@@ -237,18 +288,20 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
                 if (t + 2 < ntiles) issue_s(t + 2);       // (K of tile t + 2 was requested a tile ago)
                 if (t + 3 < ntiles) {                     // K stage (t + 1) & 1 is free once S of tile t + 1 is complete
                     mbar_wait(&bar_s[s ^ 1], ((t + 1) >> 1) & 1u);
-                    load_k(t + 3);
+                    load_k(t + 3, pg3);
                 }
                 if (t + 2 < ntiles) {                     // V stage t & 1 is free once P V of tile t is complete
                     mbar_wait(bar_o, t & 1u);
-                    load_v(t + 2);
+                    load_v(t + 2, pg2);
                 }
+                pg2 = pg3;
+                pg3 = pg_next;
             }
         }
     } else {
         // ------------------------------------------------------------------ softmax warps: one query row per thread = one TMEM lane
         const int qi = q0 + tid;                       // query index inside the sequence
-        const int qpos = p.past_len + qi;              // its absolute position
+        const int qpos = past_len + qi;                // its absolute position
         const bool row_ok = qi < p.q_len;
         // Online softmax with a LAZY reference: the output accumulator stays in TMEM across the key tiles (P V accumulates
         // there) and is rescaled -- a TMEM read-modify-write of this thread's row -- only when the row maximum outgrows the
@@ -274,10 +327,12 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
                 keep_hi = __ballot_sync(0xffffffffu, kb < p.kv_len && keep_row[kb] != 0);
             }
             // A tile every key of which is visible needs no per-element predicates (all but the diagonal / last / padded tiles).
-            const bool full = (j0 + kKvTile <= p.kv_len) && (!p.causal || j0 + kKvTile - 1 <= qpos) && (keep_lo & keep_hi) == 0xffffffffu;
+            int kvl = p.kv_len;
+            if constexpr (kPaged) kvl = kv_len;
+            const bool full = (j0 + kKvTile <= kvl) && (!p.causal || j0 + kKvTile - 1 <= qpos) && (keep_lo & keep_hi) == 0xffffffffu;
             if (!full) {
                 // keys [0, lim) of the tile pass the length / causal tests
-                const int lim = min(p.kv_len, p.causal ? qpos + 1 : p.kv_len) - j0;
+                const int lim = min(kvl, p.causal ? qpos + 1 : kvl) - j0;
                 const uint32_t vis_lo = (lim >= 32 ? 0xffffffffu : (lim > 0 ? (1u << lim) - 1u : 0u)) & keep_lo;
                 const uint32_t vis_hi = (lim >= 64 ? 0xffffffffu : (lim > 32 ? (1u << (lim - 32)) - 1u : 0u)) & keep_hi;
 #pragma unroll
@@ -434,6 +489,12 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
 #pragma unroll
                 for (int j = 0; j < 32; ++j) v[j] = 0u;
             }
+            if constexpr (kPaged) {
+                if (qi >= q_rows) {                    // right padding: exact zeros
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) v[j] = 0u;
+                }
+            }
             if (row_ok) {
 #pragma unroll
                 for (int j4 = 0; j4 < 4; ++j4) {
@@ -499,11 +560,16 @@ __global__ void __launch_bounds__(128) attention_combine_kernel(const float* __r
 // its heads + 2 kv_heads head rows through shared memory; every thread then moves 16-byte vectors: thread (slot, j) takes
 // elements [8 j, 8 j + 8) of both halves of the head rows slot, slot + 16, ... (q heads rotated in place, k heads rotated
 // into the cache, v heads copied into the cache).
-template <typename T>
+// kPaged: the cache is a page pool [num_pages, kv_heads, kKvTile, d]; token t of sequence b goes to position pos = past_lens[b]
+// + t, i.e. row pos % kKvTile of page block_table[b][pos / kKvTile].  A token t >= new_lens[b] (right padding) writes no
+// cache row (its q is still rotated).
+template <typename T, bool kPaged>
 __global__ void __launch_bounds__(128) rope_kv_append_kernel(T* q, const T* __restrict__ k_new, const T* __restrict__ v_new,
                                                             const long long* __restrict__ position_ids, T* cache_k, T* cache_v,
                                                             int q_len, int heads, int kv_heads, int d, int max_len,
-                                                            int past_len, float log2_base) {
+                                                            int past_len, float log2_base, const int* __restrict__ block_table,
+                                                            const int* __restrict__ past_lens, const int* __restrict__ new_lens,
+                                                            int pages_per_seq) {
     __shared__ float cs_sh[64], sn_sh[64];             // d / 2 <= 64
     pdl_wait_prior_grid();
     const int half = d >> 1;
@@ -524,7 +590,17 @@ __global__ void __launch_bounds__(128) rope_kv_append_kernel(T* q, const T* __re
         cs[e] = cs_sh[8 * j + e];
         sn[e] = sn_sh[8 * j + e];
     }
-    const int units = heads + 2 * kv_heads;
+    int units = heads + 2 * kv_heads;
+    long long page = 0;
+    int row = 0;
+    if constexpr (kPaged) {
+        const int pos = past_lens[b] + t;
+        if (new_lens != nullptr && t >= new_lens[b])
+            units = heads;
+        else
+            page = block_table[static_cast<long long>(b) * pages_per_seq + pos / kKvTile];
+        row = pos % kKvTile;
+    }
     for (int u = slot; u < units; u += 16) {
         const T* src;
         T* dst;
@@ -536,11 +612,17 @@ __global__ void __launch_bounds__(128) rope_kv_append_kernel(T* q, const T* __re
         } else if (u < heads + kv_heads) {
             const int h = u - heads;
             src = k_new + (tok * kv_heads + h) * d;
-            dst = cache_k + ((static_cast<long long>(b) * kv_heads + h) * max_len + past_len + t) * d;
+            if constexpr (kPaged)
+                dst = cache_k + ((page * kv_heads + h) * kKvTile + row) * d;
+            else
+                dst = cache_k + ((static_cast<long long>(b) * kv_heads + h) * max_len + past_len + t) * d;
         } else {
             const int h = u - heads - kv_heads;
             src = v_new + (tok * kv_heads + h) * d;
-            dst = cache_v + ((static_cast<long long>(b) * kv_heads + h) * max_len + past_len + t) * d;
+            if constexpr (kPaged)
+                dst = cache_v + ((page * kv_heads + h) * kKvTile + row) * d;
+            else
+                dst = cache_v + ((static_cast<long long>(b) * kv_heads + h) * max_len + past_len + t) * d;
             rotate = false;
         }
         const uint4 lo = *reinterpret_cast<const uint4*>(src + 8 * j);
@@ -566,9 +648,9 @@ __global__ void __launch_bounds__(128) rope_kv_append_kernel(T* q, const T* __re
     }
 }
 
-template <int kD, typename T, bool kLse>
+template <int kD, typename T, bool kLse, bool kPaged>
 int launch_attention(const AttnParams& p, cudaStream_t s) {
-    auto* kernel = gqa_attention_kernel<kD, T, kLse>;
+    auto* kernel = gqa_attention_kernel<kD, T, kLse, kPaged>;
     size_t smem = kQTile * kD * 2 + 4 * kKvTile * kD * 2 + 128;   // tiles + barriers
     if (const char* v = getenv("L32_ATT_ONE_CTA_PER_SM")) {   // experiments only: pad so that only one CTA fits per SM
         if (*v == '1') smem = 160 * 1024;
@@ -607,17 +689,86 @@ int launch_attention(const AttnParams& p, cudaStream_t s) {
     return static_cast<int>(e);
 }
 
-}  // namespace
+// Fields every attention launch shares: shapes, scale, instruction descriptors and the Q map.
+int attention_setup(AttnParams& p, const void* q, void* out, int batch, int q_len, int heads, int kv_heads, int head_dim,
+                    int causal, int dtype) {
+    memset(&p, 0, sizeof(p));
+    p.out = out;
+    p.batch = batch; p.q_len = q_len; p.heads = heads; p.kv_heads = kv_heads; p.causal = causal;
+    p.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(head_dim));
+    p.idesc_s = make_idesc_f16(dtype == L32_BF16, kQTile, kKvTile, false, false);
+    p.idesc_o = make_idesc_f16(dtype == L32_BF16, kQTile, static_cast<uint32_t>(head_dim), false, true);
+    return make_tensor_map_2d(&p.map_q, q, static_cast<uint64_t>(batch) * q_len, static_cast<uint64_t>(heads) * head_dim,
+                              static_cast<uint64_t>(heads) * head_dim, kQTile, 64, dtype);
+}
 
-int gqa_attention_packed(const void* q, const void* cache_k, const void* cache_v, void* out, int batch2, int group, int head_dim,
-                         int max_len, int kv_len, int splits, void* workspace, int dtype, cudaStream_t s);
-int gqa_attention_launch(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, int batch, int q_len,
-                         int heads, int kv_heads, int head_dim, int max_len, int kv_len, int past_len, int causal, int splits,
-                         void* workspace, int dtype, cudaStream_t s, float* lse = nullptr);
+// Split-KV: `splits` CTAs per (batch, head) over the key tiles of kv_len keys; the partials go to the workspace.
+void attention_split(AttnParams& p, int splits, int kv_len, int head_dim, void* workspace) {
+    p.splits = splits > 1 ? splits : 1;
+    if (p.splits > 1) {
+        const int tiles = (kv_len + kKvTile - 1) / kKvTile;
+        p.tiles_per_split = (tiles + p.splits - 1) / p.splits;
+        const size_t rows = static_cast<size_t>(p.batch) * p.heads * p.splits * p.q_len;
+        p.part_o = static_cast<float*>(workspace);
+        p.part_ml = reinterpret_cast<float2*>(static_cast<uint8_t*>(workspace) + ((rows * head_dim * sizeof(float) + 255) & ~static_cast<size_t>(255)));
+    }
+}
 
-int rope_kv_append(void* q, const void* k_new, const void* v_new, const long long* position_ids, void* cache_k, void* cache_v,
-                   int batch, int q_len, int heads, int kv_heads, int head_dim, int max_len, int past_len, float rope_base,
-                   int dtype, cudaStream_t s) {
+// The inference kernel, then (split-KV) the merge of its partials.
+template <bool kPaged>
+int attention_run(const AttnParams& p, int head_dim, int dtype, cudaStream_t s) {
+    int rc;
+    if (dtype == L32_BF16) {
+        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16, false, kPaged>(p, s) : launch_attention<64, __nv_bfloat16, false, kPaged>(p, s);
+    } else {
+        rc = head_dim == 128 ? launch_attention<128, __half, false, kPaged>(p, s) : launch_attention<64, __half, false, kPaged>(p, s);
+    }
+    if (rc != L32_OK || p.splits == 1) return rc;
+    // merge the split-KV partials
+    const long long rows = static_cast<long long>(p.batch) * p.heads * p.q_len;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(static_cast<unsigned>((rows + 3) / 4));
+    cfg.blockDim = dim3(128);
+    cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    const float* po = p.part_o;
+    const float2* pml = p.part_ml;
+    cudaError_t e;
+    if (dtype == L32_BF16)
+        e = cudaLaunchKernelEx(&cfg, attention_combine_kernel<__nv_bfloat16>, po, pml, static_cast<__nv_bfloat16*>(p.out), p.batch,
+                               p.heads, p.q_len, p.splits, head_dim);
+    else
+        e = cudaLaunchKernelEx(&cfg, attention_combine_kernel<__half>, po, pml, static_cast<__half*>(p.out), p.batch, p.heads, p.q_len,
+                               p.splits, head_dim);
+    if (e == cudaSuccess) count_launch();
+    return static_cast<int>(e);
+}
+
+// Paged-cache arguments of rope_kv_append_kernel (null: the contiguous cache).
+struct RopePages {
+    const int* block_table;
+    const int* past_lens;
+    const int* new_lens;
+    int pages_per_seq;
+};
+
+template <typename T, bool kPaged>
+cudaError_t launch_rope(const cudaLaunchConfig_t& cfg, void* q, const void* k_new, const void* v_new, const long long* position_ids,
+                        void* cache_k, void* cache_v, int q_len, int heads, int kv_heads, int head_dim, int max_len, int past_len,
+                        float log2_base, const RopePages& pg) {
+    return cudaLaunchKernelEx(&cfg, rope_kv_append_kernel<T, kPaged>, static_cast<T*>(q), static_cast<const T*>(k_new),
+                              static_cast<const T*>(v_new), position_ids, static_cast<T*>(cache_k), static_cast<T*>(cache_v), q_len,
+                              heads, kv_heads, head_dim, max_len, past_len, log2_base, pg.block_table, pg.past_lens, pg.new_lens,
+                              pg.pages_per_seq);
+}
+
+int rope_append(void* q, const void* k_new, const void* v_new, const long long* position_ids, void* cache_k, void* cache_v,
+                int batch, int q_len, int heads, int kv_heads, int head_dim, int max_len, int past_len, float rope_base, int dtype,
+                cudaStream_t s, const RopePages* pages) {
     const long long tokens = static_cast<long long>(batch) * q_len;
     if (tokens == 0) return L32_OK;
     if (head_dim != 64 && head_dim != 128) return L32_ERR_BAD_SHAPE;
@@ -634,18 +785,44 @@ int rope_kv_append(void* q, const void* k_new, const void* v_new, const long lon
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     const float log2_base = log2f(rope_base);
+    const RopePages none = {nullptr, nullptr, nullptr, 0};
+    const RopePages& pg = pages != nullptr ? *pages : none;
     cudaError_t e;
     if (dtype == L32_BF16)
-        e = cudaLaunchKernelEx(&cfg, rope_kv_append_kernel<__nv_bfloat16>, static_cast<__nv_bfloat16*>(q),
-                               static_cast<const __nv_bfloat16*>(k_new), static_cast<const __nv_bfloat16*>(v_new), position_ids,
-                               static_cast<__nv_bfloat16*>(cache_k), static_cast<__nv_bfloat16*>(cache_v), q_len, heads,
-                               kv_heads, head_dim, max_len, past_len, log2_base);
+        e = pages != nullptr ? launch_rope<__nv_bfloat16, true>(cfg, q, k_new, v_new, position_ids, cache_k, cache_v, q_len, heads,
+                                                                kv_heads, head_dim, max_len, past_len, log2_base, pg)
+                             : launch_rope<__nv_bfloat16, false>(cfg, q, k_new, v_new, position_ids, cache_k, cache_v, q_len, heads,
+                                                                 kv_heads, head_dim, max_len, past_len, log2_base, pg);
     else
-        e = cudaLaunchKernelEx(&cfg, rope_kv_append_kernel<__half>, static_cast<__half*>(q), static_cast<const __half*>(k_new),
-                               static_cast<const __half*>(v_new), position_ids, static_cast<__half*>(cache_k),
-                               static_cast<__half*>(cache_v), q_len, heads, kv_heads, head_dim, max_len, past_len, log2_base);
+        e = pages != nullptr ? launch_rope<__half, true>(cfg, q, k_new, v_new, position_ids, cache_k, cache_v, q_len, heads, kv_heads,
+                                                         head_dim, max_len, past_len, log2_base, pg)
+                             : launch_rope<__half, false>(cfg, q, k_new, v_new, position_ids, cache_k, cache_v, q_len, heads, kv_heads,
+                                                          head_dim, max_len, past_len, log2_base, pg);
     if (e == cudaSuccess) count_launch();
     return static_cast<int>(e);
+}
+
+}  // namespace
+
+int gqa_attention_packed(const void* q, const void* cache_k, const void* cache_v, void* out, int batch2, int group, int head_dim,
+                         int max_len, int kv_len, int splits, void* workspace, int dtype, cudaStream_t s);
+int gqa_attention_launch(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, int batch, int q_len,
+                         int heads, int kv_heads, int head_dim, int max_len, int kv_len, int past_len, int causal, int splits,
+                         void* workspace, int dtype, cudaStream_t s, float* lse = nullptr);
+
+int rope_kv_append(void* q, const void* k_new, const void* v_new, const long long* position_ids, void* cache_k, void* cache_v,
+                   int batch, int q_len, int heads, int kv_heads, int head_dim, int max_len, int past_len, float rope_base,
+                   int dtype, cudaStream_t s) {
+    return rope_append(q, k_new, v_new, position_ids, cache_k, cache_v, batch, q_len, heads, kv_heads, head_dim, max_len, past_len,
+                       rope_base, dtype, s, nullptr);
+}
+
+int rope_kv_append_paged(void* q, const void* k_new, const void* v_new, const long long* position_ids, void* pool_k, void* pool_v,
+                         const int* block_table, const int* past_lens, const int* new_lens, int batch, int q_len, int heads,
+                         int kv_heads, int head_dim, int max_pages_per_seq, float rope_base, int dtype, cudaStream_t s) {
+    const RopePages pages = {block_table, past_lens, new_lens, max_pages_per_seq};
+    return rope_append(q, k_new, v_new, position_ids, pool_k, pool_v, batch, q_len, heads, kv_heads, head_dim, kKvTile, 0, rope_base,
+                       dtype, s, &pages);
 }
 
 // Split-KV plan of a decode call without key padding: the number of key splits (1 = none).  Only the packed decode path
@@ -687,6 +864,42 @@ int gqa_attention(const void* q, const void* cache_k, const void* cache_v, const
                                 causal, 1, nullptr, dtype, s);
 }
 
+// Paged cache: the same three launch shapes (packed decode, its split-KV form, the general causal kernel) with K / V tiles
+// read through the block table and each sequence's lengths read from device memory.  The split plan is the contiguous
+// path's for kv_len = max_kv_len (a host bound on every sequence's length); each sequence then divides its own key tiles over
+// those splits.
+int gqa_attention_paged(const void* q, const void* pool_k, const void* pool_v, const int* block_table, const int* past_lens,
+                        const int* new_lens, void* out, void* workspace, size_t workspace_bytes, int batch, int q_len, int heads,
+                        int kv_heads, int head_dim, int num_pages, int max_pages_per_seq, int max_kv_len, int dtype, cudaStream_t s) {
+    if (head_dim != 64 && head_dim != 128) return L32_ERR_BAD_SHAPE;
+    if (batch <= 0 || q_len <= 0) return L32_OK;
+    const bool packed = q_len == 1 && heads > kv_heads;
+    AttnParams p;
+    int rc = packed ? attention_setup(p, q, out, batch * kv_heads, heads / kv_heads, 1, 1, head_dim, 0, dtype)
+                    : attention_setup(p, q, out, batch, q_len, heads, kv_heads, head_dim, 1, dtype);
+    if (rc != L32_OK) return rc;
+    p.block_table = block_table;
+    p.past_lens = past_lens;
+    p.new_lens = new_lens;
+    p.pages_per_seq = max_pages_per_seq;
+    p.page_kv_heads = kv_heads;
+    p.packed = packed ? 1 : 0;
+    // K / V: one plane per (page, kv head) of kKvTile rows.  Rows of a page past its sequence's length are read as they are
+    // and get P = 0: the pool's contract keeps them finite (include/l32_ffn.h).
+    const uint64_t planes = static_cast<uint64_t>(num_pages) * kv_heads, plane_elems = static_cast<uint64_t>(kKvTile) * head_dim;
+    rc = make_tensor_map_3d(&p.map_k, pool_k, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
+    if (rc != L32_OK) return rc;
+    rc = make_tensor_map_3d(&p.map_v, pool_v, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
+    if (rc != L32_OK) return rc;
+    int splits = 1;
+    if (packed) {
+        const size_t need = gqa_attention_workspace_bytes(batch, 1, heads, kv_heads, head_dim, max_kv_len);
+        if (need > 0 && workspace != nullptr && workspace_bytes >= need) splits = decode_splits(batch, 1, heads, kv_heads, max_kv_len);
+    }
+    attention_split(p, splits, max_kv_len, head_dim, workspace);
+    return attention_run<true>(p, head_dim, dtype, s);
+}
+
 // Training forward: keys [0, q_len) of the K / V buffers, no past, no split-KV; also writes the per-row log-sum-exp.
 int gqa_attention_train(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, float* lse, int batch,
                         int q_len, int heads, int kv_heads, int head_dim, int max_len, int causal, int dtype, cudaStream_t s) {
@@ -707,18 +920,11 @@ int gqa_attention_launch(const void* q, const void* cache_k, const void* cache_v
                          int heads, int kv_heads, int head_dim, int max_len, int kv_len, int past_len, int causal, int splits,
                          void* workspace, int dtype, cudaStream_t s, float* lse) {
     AttnParams p;
-    memset(&p, 0, sizeof(p));
-    p.out = out;
+    int rc = attention_setup(p, q, out, batch, q_len, heads, kv_heads, head_dim, causal, dtype);
+    if (rc != L32_OK) return rc;
     p.lse = lse;
     p.keep = keep;
-    p.batch = batch; p.q_len = q_len; p.heads = heads; p.kv_heads = kv_heads; p.max_len = max_len; p.kv_len = kv_len;
-    p.past_len = past_len; p.causal = causal;
-    p.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(head_dim));
-    p.idesc_s = make_idesc_f16(dtype == L32_BF16, kQTile, kKvTile, false, false);
-    p.idesc_o = make_idesc_f16(dtype == L32_BF16, kQTile, static_cast<uint32_t>(head_dim), false, true);
-    int rc = make_tensor_map_2d(&p.map_q, q, static_cast<uint64_t>(batch) * q_len, static_cast<uint64_t>(heads) * head_dim,
-                                static_cast<uint64_t>(heads) * head_dim, kQTile, 64, dtype);
-    if (rc != L32_OK) return rc;
+    p.max_len = max_len; p.kv_len = kv_len; p.past_len = past_len;
     // K / V: one plane per (batch, kv head), cut at kv_len.  Masked keys get P = 0, but 0 * NaN and 0 * Inf are NaN in the
     // P V product: the rows of the last tile beyond kv_len (stale cache capacity, or the next head's keys) must not reach
     // shared memory with whatever they hold, so TMA fills them with zeros.
@@ -728,47 +934,13 @@ int gqa_attention_launch(const void* q, const void* cache_k, const void* cache_v
     if (rc != L32_OK) return rc;
     rc = make_tensor_map_3d(&p.map_v, cache_v, planes, kv_rows, head_dim, head_dim, plane_elems, kKvTile, dtype);
     if (rc != L32_OK) return rc;
-    p.splits = splits > 1 ? splits : 1;
-    if (p.splits > 1) {
-        const int tiles = (kv_len + kKvTile - 1) / kKvTile;
-        p.tiles_per_split = (tiles + p.splits - 1) / p.splits;
-        const size_t rows = static_cast<size_t>(batch) * heads * p.splits * q_len;
-        p.part_o = static_cast<float*>(workspace);
-        p.part_ml = reinterpret_cast<float2*>(static_cast<uint8_t*>(workspace) + ((rows * head_dim * sizeof(float) + 255) & ~static_cast<size_t>(255)));
-    }
+    attention_split(p, splits, kv_len, head_dim, workspace);
     if (lse != nullptr) {
         if (dtype == L32_BF16)
-            return head_dim == 128 ? launch_attention<128, __nv_bfloat16, true>(p, s) : launch_attention<64, __nv_bfloat16, true>(p, s);
-        return head_dim == 128 ? launch_attention<128, __half, true>(p, s) : launch_attention<64, __half, true>(p, s);
+            return head_dim == 128 ? launch_attention<128, __nv_bfloat16, true, false>(p, s) : launch_attention<64, __nv_bfloat16, true, false>(p, s);
+        return head_dim == 128 ? launch_attention<128, __half, true, false>(p, s) : launch_attention<64, __half, true, false>(p, s);
     }
-    if (dtype == L32_BF16) {
-        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16, false>(p, s) : launch_attention<64, __nv_bfloat16, false>(p, s);
-    } else {
-        rc = head_dim == 128 ? launch_attention<128, __half, false>(p, s) : launch_attention<64, __half, false>(p, s);
-    }
-    if (rc != L32_OK || p.splits == 1) return rc;
-    // merge the split-KV partials
-    const long long rows = static_cast<long long>(batch) * heads * q_len;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(static_cast<unsigned>((rows + 3) / 4));
-    cfg.blockDim = dim3(128);
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    const float* po = p.part_o;
-    const float2* pml = p.part_ml;
-    cudaError_t e;
-    if (dtype == L32_BF16)
-        e = cudaLaunchKernelEx(&cfg, attention_combine_kernel<__nv_bfloat16>, po, pml, static_cast<__nv_bfloat16*>(out), batch, heads,
-                               q_len, p.splits, head_dim);
-    else
-        e = cudaLaunchKernelEx(&cfg, attention_combine_kernel<__half>, po, pml, static_cast<__half*>(out), batch, heads, q_len,
-                               p.splits, head_dim);
-    if (e == cudaSuccess) count_launch();
-    return static_cast<int>(e);
+    return attention_run<false>(p, head_dim, dtype, s);
 }
 
 }  // namespace l32

@@ -161,6 +161,13 @@ int gqa_attention(const void* q, const void* cache_k, const void* cache_v, const
                   size_t workspace_bytes, int dtype, cudaStream_t s);
 int gqa_attention_train(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, float* lse, int batch,
                         int q_len, int heads, int kv_heads, int head_dim, int max_len, int causal, int dtype, cudaStream_t s);
+// paged KV cache (pools [num_pages, kv_heads, L32_KV_PAGE, head_dim], block table, per-sequence lengths in device memory)
+int rope_kv_append_paged(void* q, const void* k_new, const void* v_new, const long long* position_ids, void* pool_k, void* pool_v,
+                         const int* block_table, const int* past_lens, const int* new_lens, int batch, int q_len, int heads,
+                         int kv_heads, int head_dim, int max_pages_per_seq, float rope_base, int dtype, cudaStream_t s);
+int gqa_attention_paged(const void* q, const void* pool_k, const void* pool_v, const int* block_table, const int* past_lens,
+                        const int* new_lens, void* out, void* workspace, size_t workspace_bytes, int batch, int q_len, int heads,
+                        int kv_heads, int head_dim, int num_pages, int max_pages_per_seq, int max_kv_len, int dtype, cudaStream_t s);
 // RoPE angle of rotation pair i (of d / 2) at position `pos`: pos * base^(-2 i / d), cos / sin in fp32.  The forward rotation
 // (rope_kv_append_kernel) and the inverse rotation of the backward epilogues share it, so both use bit-identical angles.
 L32_DEVICE void rope_cos_sin(float pos, int i, int d, float log2_base, float& cs, float& sn) {

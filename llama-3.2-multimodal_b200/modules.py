@@ -25,7 +25,7 @@ __all__ = [
     "RMSNormFunction", "LLAMARMSNorm", "SwiGLUFunction", "FusedSwiGLU", "LinearFunction", "Linear_LORA", "FFNFunction", "FFNLoRAFunction",
     "FusedFeedforward", "FusedFeedForward", "convert_feedforward_to_fused", "patch_reference", "convert_instances", "block_tail",
     "BlockTailFunction", "LinearLoRAFunction", "chain_block_norms", "LMHeadCEFunction", "lm_head_loss", "shift_labels", "GroupQueryAttention", "KVCache",
-    "GQAAttentionFunction",
+    "GQAAttentionFunction", "PagedKVCache",
 ]
 
 
@@ -549,6 +549,145 @@ class KVCache:
         return self.key_cache[layer_idx], self.value_cache[layer_idx]
 
 
+class PagedKVCache:
+    """KV cache for serving several sequences at once (inference only): keys / values live in pages of 64 tokens
+    (ops.KV_PAGE, one key tile of the attention kernel) named by a block table, and every sequence has its own length.
+    A finished sequence hands its pages back (`free_sequence`) and a new one can join in the same step (`add_sequence`).
+
+    Per layer one pool for K and one for V, [num_pages, kv_heads, 64, head_dim], zero-initialised on the layer's first
+    forward; page index p names the same slot in every layer, so one allocator serves all layers.  The host keeps the
+    bookkeeping (free list, each sequence's pages and length) and is the source of truth: nothing is ever read back from
+    the device.  The block table and the lengths of the current batch live in static device buffers sized for `max_batch`,
+    so a CUDA graph captured over a forward stays valid while `set_batch` changes their contents between replays.
+
+    One step:  set_batch(ids, new_lens) -> every layer's forward -> advance().
+    Rows of the device buffers past len(ids) hold zero lengths: a forward over more rows than the batch (a graph captured
+    at a larger batch) leaves those rows' output zero and writes no page.
+    Pages handed out again keep what the previous sequence wrote: finite values, which is all the kernels require of rows
+    past a sequence's length (include/l32_ffn.h)."""
+
+    def __init__(self, num_pages: int, max_batch: int, max_pages_per_seq: int, device=None):
+        if num_pages <= 0 or max_batch <= 0 or max_pages_per_seq <= 0:
+            raise ValueError("PagedKVCache: num_pages, max_batch and max_pages_per_seq must be positive")
+        self.num_pages, self.max_batch, self.max_pages_per_seq = int(num_pages), int(max_batch), int(max_pages_per_seq)
+        self.page_size = ops.KV_PAGE
+        self._free = list(range(self.num_pages - 1, -1, -1))   # pop() hands out the lowest free page first
+        self._pages: dict = {}                                   # sequence id -> its pages, in logical order
+        self._len: dict = {}                                     # sequence id -> tokens cached
+        self._next_id = 0
+        self.batch_ids: list = []
+        self.batch_new_lens: list = []
+        self._pool_k: list = []                                  # per layer
+        self._pool_v: list = []
+        if device is None and torch.cuda.is_available():
+            device = torch.device("cuda", torch.cuda.current_device())
+        self.device = None if device is None else torch.device(device)
+        # one device buffer: the block table [max_batch, max_pages_per_seq], then past_lens [max_batch], new_lens [max_batch]
+        n = self.max_batch * (self.max_pages_per_seq + 2)
+        self._dev = torch.zeros(n, dtype=torch.int32, device=self.device) if self.device is not None else None
+        self.block_table = self.past_lens = self.new_lens = None
+        if self._dev is not None:
+            t = self.max_batch * self.max_pages_per_seq
+            self.block_table = self._dev[:t].view(self.max_batch, self.max_pages_per_seq)
+            self.past_lens = self._dev[t:t + self.max_batch]
+            self.new_lens = self._dev[t + self.max_batch:]
+
+    # -- allocator
+    @property
+    def free_pages(self) -> int:
+        return len(self._free)
+
+    @property
+    def max_kv_len(self) -> int:
+        """The bound on every sequence's length the attention's split plan is sized for."""
+        return self.max_pages_per_seq * self.page_size
+
+    def add_sequence(self) -> int:
+        sid = self._next_id
+        self._next_id += 1
+        self._pages[sid] = []
+        self._len[sid] = 0
+        return sid
+
+    def free_sequence(self, sid: int) -> None:
+        """Hand the sequence's pages back.  If it is part of the current batch, that batch is dropped: call set_batch again
+        before the next forward."""
+        pages = self._pages.pop(sid)
+        del self._len[sid]
+        self._free.extend(reversed(pages))
+        if sid in self.batch_ids:
+            self.batch_ids, self.batch_new_lens = [], []
+
+    def length(self, sid: int) -> int:
+        return self._len[sid]
+
+    def pages(self, sid: int) -> list:
+        return list(self._pages[sid])
+
+    def set_batch(self, ids, new_lens) -> None:
+        """Choose the sequences (rows, in this order) of the next forward calls and the number of tokens each appends, reserve
+        the pages those tokens need and upload the block table and lengths (stream-ordered copies from pinned host memory on
+        the current stream).  Raises before anything is reserved or enqueued when the pages run out or a sequence would
+        outgrow max_pages_per_seq."""
+        ids, new_lens = [int(i) for i in ids], [int(n) for n in new_lens]
+        if len(ids) != len(new_lens) or not 0 < len(ids) <= self.max_batch:
+            raise ValueError(f"set_batch: {len(ids)} ids / {len(new_lens)} lengths for a cache of max_batch {self.max_batch}")
+        if len(set(ids)) != len(ids) or any(i not in self._pages for i in ids):
+            raise ValueError(f"set_batch: ids must be distinct live sequences, got {ids}")
+        if any(n < 0 for n in new_lens):
+            raise ValueError(f"set_batch: negative new length in {new_lens}")
+        want = []
+        for sid, n in zip(ids, new_lens):
+            need = -(-(self._len[sid] + n) // self.page_size)
+            if need > self.max_pages_per_seq:
+                raise ValueError(f"set_batch: sequence {sid} would hold {self._len[sid] + n} tokens, more than max_pages_per_seq "
+                                 f"* {self.page_size} = {self.max_kv_len}")
+            want.append(max(0, need - len(self._pages[sid])))
+        if sum(want) > len(self._free):
+            raise RuntimeError(f"PagedKVCache out of pages: this step needs {sum(want)} more, {len(self._free)} free of "
+                               f"{self.num_pages}")
+        for sid, w in zip(ids, want):
+            self._pages[sid].extend(self._free.pop() for _ in range(w))
+        self.batch_ids, self.batch_new_lens = ids, new_lens
+        host = torch.zeros(self.max_batch * (self.max_pages_per_seq + 2), dtype=torch.int32,
+                           pin_memory=self._dev is not None)
+        t = self.max_batch * self.max_pages_per_seq
+        table = host[:t].view(self.max_batch, self.max_pages_per_seq)
+        for r, sid in enumerate(ids):
+            pages = self._pages[sid]
+            if any(not 0 <= p < self.num_pages for p in pages):
+                raise RuntimeError(f"PagedKVCache: page index out of range in sequence {sid}: {pages}")
+            if pages:
+                table[r, :len(pages)] = torch.tensor(pages, dtype=torch.int32)
+            host[t + r] = self._len[sid]
+            host[t + self.max_batch + r] = new_lens[r]
+        self._host = host                                   # (the last upload's contents, for inspection)
+        if self._dev is not None:
+            # torch's pinned-memory allocator keeps `host` from being reused until this copy has run, so no host-side wait
+            self._dev.copy_(host, non_blocking=True)
+
+    def advance(self) -> None:
+        """After the step's last layer: every sequence of the batch now holds its new tokens."""
+        for sid, n in zip(self.batch_ids, self.batch_new_lens):
+            self._len[sid] += n
+
+    # -- per-layer pools
+    def pools(self, layer_idx, kv_heads, head_dim, dtype, device):
+        """(pool_k, pool_v) of layer `layer_idx`, created zeroed on first use with this geometry."""
+        while len(self._pool_k) <= layer_idx:
+            self._pool_k.append(None)
+            self._pool_v.append(None)
+        k = self._pool_k[layer_idx]
+        shape = (self.num_pages, kv_heads, self.page_size, head_dim)
+        if k is None:
+            k = torch.zeros(shape, dtype=dtype, device=device)
+            self._pool_k[layer_idx], self._pool_v[layer_idx] = k, torch.zeros_like(k)
+        elif tuple(k.shape) != shape or k.dtype != dtype or k.device != torch.device(device):
+            raise ValueError(f"PagedKVCache layer {layer_idx}: pool is {tuple(k.shape)} {k.dtype} on {k.device}, this call "
+                             f"needs {shape} {dtype} on {device}")
+        return self._pool_k[layer_idx], self._pool_v[layer_idx]
+
+
 def _rotate_half(x):
     x1, x2 = x[..., : x.shape[-1] // 2], x[..., x.shape[-1] // 2:]
     return torch.cat((-x2, x1), dim=-1)
@@ -674,7 +813,49 @@ class GroupQueryAttention(nn.Module):
     def _project(mod, x):
         return mod(x) if _is_lora(mod) else _linear(x, mod.weight, mod.bias)
 
+    def _qkv(self, hidden_states):
+        projs = (self.W_query, self.W_key, self.W_value)
+        if (not torch.is_grad_enabled() or not _wants_grad(hidden_states, *[m.weight for m in projs])) and all(
+                not _is_lora(m) and m.bias is None and m.weight.dtype == hidden_states.dtype and _dims8(*m.weight.shape) for m in projs):
+            # inference: the three projections of the same activations in ONE launch (reference Model/model.py:231-233)
+            return ops.linear_group_forward(hidden_states, [m.weight for m in projs])
+        q = self._project(self.W_query, hidden_states)           # [b, t, heads * d]: the kernels read this layout as it is
+        k = self._project(self.W_key, hidden_states)
+        v = self._project(self.W_value, hidden_states)
+        return q, k, v
+
+    def _paged_forward(self, hidden_states, attention_mask, position_ids, cache):
+        """Inference over a PagedKVCache: row r of hidden_states [len(batch), t, hidden] (right-padded, t >= every new length)
+        is sequence cache.batch_ids[r]; attention is causal over that sequence's own keys.  There are no reference expressions
+        for a paged cache, so inputs the kernels do not take are an error."""
+        if attention_mask is not None:
+            raise ValueError("GroupQueryAttention with a PagedKVCache takes no attention_mask: the cache's lengths are the mask")
+        if position_ids is None:
+            raise ValueError("GroupQueryAttention with a PagedKVCache needs position_ids")
+        if self._records_grad(hidden_states):
+            raise ValueError("a PagedKVCache is inference-only: run the forward under torch.no_grad()")
+        if not self._kernel_ok(hidden_states):
+            raise ValueError("GroupQueryAttention with a PagedKVCache runs on the sm_100a kernels only: CUDA bf16 / fp16 "
+                             "[batch, t, hidden] inputs and weights, head_dim 64 or 128")
+        b, t, _ = hidden_states.shape
+        if not cache.batch_ids or b != len(cache.batch_ids) or t < max(cache.batch_new_lens):
+            raise ValueError(f"hidden_states [{b}, {t}, ...] does not fit the cache's batch: {len(cache.batch_ids)} sequences "
+                             f"appending {cache.batch_new_lens} tokens (call set_batch first)")
+        if cache.device is None or hidden_states.device != cache.device:
+            raise ValueError(f"PagedKVCache on {cache.device}, hidden_states on {hidden_states.device}")
+        if position_ids.dim() == 1:
+            position_ids = position_ids[None]
+        pos = position_ids.to(device=hidden_states.device, dtype=torch.int64).expand(b, t).contiguous()
+        q, k, v = self._qkv(hidden_states)
+        pk, pv = cache.pools(self.layer_idx or 0, self.num_kv_groups, self.head_dim, q.dtype, q.device)
+        ops.rope_kv_append_paged(q, k, v, pos, pk, pv, cache.block_table, cache.past_lens, cache.new_lens, self.rope_base)
+        ctx = ops.gqa_attention_forward_paged(q, pk, pv, cache.block_table, cache.past_lens, cache.new_lens,
+                                              max_kv_len=cache.max_kv_len)
+        return self._project(self.out_proj, ctx)
+
     def forward(self, hidden_states, attention_mask=None, position_ids=None, kv_cache=None):
+        if isinstance(kv_cache, PagedKVCache):
+            return self._paged_forward(hidden_states, attention_mask, position_ids, kv_cache)
         if (position_ids is None or (attention_mask is not None and not attention_mask.is_floating_point())):
             return self._reference_forward(hidden_states, attention_mask, position_ids, kv_cache)
         train = self._train_ok(hidden_states, kv_cache)
@@ -693,15 +874,7 @@ class GroupQueryAttention(nn.Module):
             pos = position_ids.to(device=q.device, dtype=torch.int64).contiguous()
             ctx = GQAAttentionFunction.apply(q, k, v, pos, causal, keep, self.rope_base, self.num_kv_groups)
             return self._project(self.out_proj, ctx)
-        projs = (self.W_query, self.W_key, self.W_value)
-        if (not torch.is_grad_enabled() or not _wants_grad(hidden_states, *[m.weight for m in projs])) and all(
-                not _is_lora(m) and m.bias is None and m.weight.dtype == hidden_states.dtype and _dims8(*m.weight.shape) for m in projs):
-            # inference: the three projections of the same activations in ONE launch (reference Model/model.py:231-233)
-            q, k, v = ops.linear_group_forward(hidden_states, [m.weight for m in projs])
-        else:
-            q = self._project(self.W_query, hidden_states)       # [b, t, heads * d]: the kernels read this layout as it is
-            k = self._project(self.W_key, hidden_states)
-            v = self._project(self.W_value, hidden_states)
+        q, k, v = self._qkv(hidden_states)
         cache = kv_cache if kv_cache is not None else KVCache()
         layer = self.layer_idx if kv_cache is not None else 0
         past = cache.length(layer)

@@ -13,6 +13,7 @@ import torch
 from ._lib import L32Error, check, lib
 
 _DT = {torch.bfloat16: 0, torch.float16: 1}
+KV_PAGE = 64   # tokens per page of a paged KV cache (L32_KV_PAGE, include/l32_ffn.h): one key tile of the attention kernel
 
 
 def _dtype_code(t: torch.Tensor) -> int:
@@ -477,6 +478,67 @@ def gqa_attention_forward(q, cache_k, cache_v, kv_len, past_len, *, causal=True,
         check(L.l32_gqa_attention_forward(_ptr(qc), _ptr(cache_k), _ptr(cache_v), _ptr(keep), _ptr(ctx), _ptr(ws), ws_bytes, b, t,
                                           heads, kvh, d, max_len, int(kv_len), int(past_len), int(bool(causal)), _dtype_code(qc),
                                           _stream(qc)), "l32_gqa_attention_forward")
+    return ctx
+
+
+def _paged_args(q, pool_k, pool_v, block_table, past_lens, new_lens, what):
+    """Shapes of a paged-cache call, checked: (b, t, heads, kv_heads, d, num_pages, max_pages_per_seq)."""
+    b, t = q.shape[0], q.shape[1]
+    num_pages, kvh, page, d = pool_k.shape
+    if page != KV_PAGE or tuple(pool_v.shape) != tuple(pool_k.shape) or pool_v.dtype != pool_k.dtype:
+        raise L32Error(f"{what}: pools must both be [num_pages, kv_heads, {KV_PAGE}, head_dim], got {tuple(pool_k.shape)} / "
+                       f"{tuple(pool_v.shape)}")
+    if q.dim() != 3 or q.shape[-1] % d != 0 or q.dtype != pool_k.dtype:
+        raise L32Error(f"{what}: q must be [batch, q_len, heads * {d}] {pool_k.dtype}, got {tuple(q.shape)} {q.dtype}")
+    for ten in (q, pool_k, pool_v, block_table, past_lens, new_lens):
+        if ten is not None and not ten.is_contiguous():
+            raise L32Error(f"{what}: tensors must be contiguous")
+    for name, ten in (("block_table", block_table), ("past_lens", past_lens), ("new_lens", new_lens)):
+        if ten is not None and ten.dtype != torch.int32:
+            raise L32Error(f"{what}: {name} must be int32")
+    if block_table.dim() != 2 or block_table.shape[0] < b or past_lens.numel() < b or (new_lens is not None and new_lens.numel() < b):
+        raise L32Error(f"{what}: block_table [>= {b}, max_pages], past_lens / new_lens [>= {b}] expected")
+    return b, t, q.shape[-1] // d, kvh, d, num_pages, block_table.shape[1]
+
+
+def rope_kv_append_paged(q, k_new, v_new, position_ids, pool_k, pool_v, block_table, past_lens, new_lens=None, rope_base=500000.0):
+    """RoPE on q [b, t, heads*d] IN PLACE and on k_new while it is stored into the paged pool_k [num_pages, kv_heads, 64, d]:
+    token i of sequence b goes to position past_lens[b] + i, row pos % 64 of page block_table[b][pos // 64]; v_new is stored
+    next to it.  Tokens i >= new_lens[b] write nothing.  block_table int32 [>= b, max_pages], past_lens / new_lens int32
+    [>= b] in device memory: their values are trusted (PagedKVCache checks them when it builds them)."""
+    _check_cuda(q, k_new, v_new, position_ids, pool_k, pool_v, block_table, past_lens, new_lens)
+    b, t, heads, kvh, d, num_pages, max_pages = _paged_args(q, pool_k, pool_v, block_table, past_lens, new_lens,
+                                                            "rope_kv_append_paged")
+    for ten in (k_new, v_new):
+        if not ten.is_contiguous() or ten.shape[:2] != q.shape[:2] or ten.shape[-1] != kvh * d:
+            raise L32Error(f"rope_kv_append_paged: k_new / v_new must be contiguous [{b}, {t}, {kvh * d}]")
+    pos = position_ids.contiguous()
+    if pos.dtype != torch.int64 or pos.numel() != b * t:
+        raise L32Error("rope_kv_append_paged: position_ids must be int64 [batch, q_len]")
+    with torch.cuda.device(q.device):
+        check(lib().l32_rope_kv_append_paged(_ptr(q), _ptr(k_new), _ptr(v_new), _ptr(pos), _ptr(pool_k), _ptr(pool_v),
+                                             _ptr(block_table), _ptr(past_lens), _ptr(new_lens), b, t, heads, kvh, d, num_pages,
+                                             max_pages, float(rope_base), _dtype_code(q), _stream(q)),
+              "l32_rope_kv_append_paged")
+
+
+def gqa_attention_forward_paged(q, pool_k, pool_v, block_table, past_lens, new_lens=None, *, max_kv_len=None):
+    """ctx [b, t, heads*d]: causal attention of each sequence's queries (positions past_lens[b] + i, RoPE applied) over its own
+    keys [0, past_lens[b] + new_lens[b]) in the paged pools; padded query rows (i >= new_lens[b]) give zeros.  max_kv_len: a
+    bound on every sequence's length that sizes the split-KV plan (default: the table's capacity, max_pages * 64)."""
+    _check_cuda(q, pool_k, pool_v, block_table, past_lens, new_lens)
+    b, t, heads, kvh, d, num_pages, max_pages = _paged_args(q, pool_k, pool_v, block_table, past_lens, new_lens,
+                                                            "gqa_attention_forward_paged")
+    max_kv_len = max_pages * KV_PAGE if max_kv_len is None else int(max_kv_len)
+    ctx = torch.empty_like(q)
+    L = lib()
+    ws_bytes = L.l32_gqa_attention_workspace_bytes(b, t, heads, kvh, d, max_kv_len)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=q.device) if ws_bytes else None
+    with torch.cuda.device(q.device):
+        check(L.l32_gqa_attention_forward_paged(_ptr(q), _ptr(pool_k), _ptr(pool_v), _ptr(block_table), _ptr(past_lens),
+                                                _ptr(new_lens), _ptr(ctx), _ptr(ws), ws_bytes, b, t, heads, kvh, d, num_pages,
+                                                max_pages, max_kv_len, _dtype_code(q), _stream(q)),
+              "l32_gqa_attention_forward_paged")
     return ctx
 
 
