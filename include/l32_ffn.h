@@ -57,8 +57,8 @@ extern "C" {
  *    l32_rmsnorm_backward_add, l32_block_tail_forward_ex, l32_linear_lora_forward / _backward, l32_lm_head_ce_*,
  *    l32_rope_kv_append, l32_gqa_attention_forward; later, additively: l32_gqa_attention_forward_train / _backward, and
  *    the tensor-parallel attention GEMMs l32_tp_linear_group_forward_allgather, l32_tp_linear_forward_allgather and
- *    l32_tp_linear_group_backward_dx_reduce_scatter, and the paged KV cache l32_rope_kv_append_paged and
- *    l32_gqa_attention_forward_paged. */
+ *    l32_tp_linear_group_backward_dx_reduce_scatter, the paged KV cache l32_rope_kv_append_paged and
+ *    l32_gqa_attention_forward_paged, and its cascade decode l32_gqa_attention_forward_paged_cascade. */
 L32_API int l32_abi_version(void);
 /* Number of CUDA kernels this library has launched in the calling process so far (monotonic). */
 L32_API unsigned long long l32_kernel_launch_count(void);
@@ -349,6 +349,39 @@ L32_API int l32_gqa_attention_forward_paged(const void* q, const void* pool_k, c
                                             const int32_t* past_lens, const int32_t* new_lens, void* ctx, void* workspace,
                                             size_t workspace_bytes, int batch, int q_len, int heads, int kv_heads, int head_dim,
                                             int num_pages, int max_pages_per_seq, int max_kv_len, int dtype, void* stream);
+
+/* Cascade decode over a paged cache whose sequences share prefix pages (forked sequences: PagedKVCache.fork).  One decode step
+ * (one query per sequence, group = heads / kv_heads in [2, L32_CASCADE_TILE_ROWS]) computed as
+ *   prefix pass : per (kv head, prefix work item) one query tile of L32_CASCADE_TILE_ROWS rows holding the `group` query
+ *                 heads of up to floor(128 / group) member sequences, over the item's shared key tiles (read once for all
+ *                 its members);
+ *   own-key pass: per (sequence, kv head, split) the packed paged decode over the sequence's keys from its shared tiles on;
+ *   combine     : the row's prefix partials, then its split partials, merged in that fixed order.
+ * Same layout and stale-row contract as l32_gqa_attention_forward_paged (q_len = 1; new_lens NULL means one new token per
+ * sequence, 0 marks a row that yields zeros).  The plan, int32 in device memory, TRUSTED like the table:
+ *   plan_items  : [1 + 5 * max_items]: the item count n <= max_items, then per item (first_seq, tile0, tiles, member0,
+ *                 members): keys [tile0 * 64, (tile0 + tiles) * 64) read through block_table row first_seq, for the query
+ *                 rows of sequences plan_members[member0 .. member0 + members), members * group <= 128.
+ *   plan_members: [batch] sequence indices.
+ *   plan_seq    : [batch][4] per sequence (shared_tiles, first_item, items, row0): its keys [0, shared_tiles * 64) are covered
+ *                 by items first_item .. first_item + items - 1, where it is member row0 / group (query tile rows row0 ..
+ *                 row0 + group - 1); items = 0 for a sequence outside the prefix pass (shared_tiles = 0).
+ *   The prefix tiles of a sequence must be full pages of ITS table (the same pages as first_seq's) and lie below
+ *   past_lens[b]: they are read with no mask.  Items past n are ignored, as is every workspace slot the plan does not name.
+ * max_items: the plan's capacity; it fixes the launch shape, so a CUDA graph captured once stays valid while the plan's
+ * contents change between replays.  max_kv_len: as for l32_gqa_attention_forward_paged (sizes the own-key split plan).
+ * workspace: l32_gqa_attention_cascade_workspace_bytes(...) bytes, 16-byte aligned (required).  Enqueues two kernels.
+ * Deterministic: the same inputs give the same bits. */
+#define L32_CASCADE_TILE_ROWS 128
+#define L32_CASCADE_MAX_ITEMS 65535
+L32_API size_t l32_gqa_attention_cascade_workspace_bytes(int batch, int heads, int kv_heads, int head_dim, int max_kv_len,
+                                                         int max_items);
+L32_API int l32_gqa_attention_forward_paged_cascade(const void* q, const void* pool_k, const void* pool_v, const int32_t* block_table,
+                                                    const int32_t* past_lens, const int32_t* new_lens, const int32_t* plan_items,
+                                                    const int32_t* plan_members, const int32_t* plan_seq, void* ctx, void* workspace,
+                                                    size_t workspace_bytes, int batch, int heads, int kv_heads, int head_dim,
+                                                    int num_pages, int max_pages_per_seq, int max_kv_len, int max_items, int dtype,
+                                                    void* stream);
 
 /* General tiled GEMM used by the entry points above (exposed for tests, tuning and the tensor-parallel
  * host code):  D[m,n] = A[m,k] B[n,k]^T  (+ A1 B1^T when a1 != NULL).

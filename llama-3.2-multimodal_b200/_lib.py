@@ -55,6 +55,8 @@ SIGNATURES = {
     "l32_gqa_attention_backward": (c_int, [c_void_p] * 12 + [c_size_t] + [c_int] * 7 + [c_float, c_int, c_void_p]),
     "l32_rope_kv_append_paged": (c_int, [c_void_p] * 9 + [c_int] * 7 + [c_float, c_int, c_void_p]),
     "l32_gqa_attention_forward_paged": (c_int, [c_void_p] * 8 + [c_size_t] + [c_int] * 9 + [c_void_p]),
+    "l32_gqa_attention_cascade_workspace_bytes": (c_size_t, [c_int] * 6),
+    "l32_gqa_attention_forward_paged_cascade": (c_int, [c_void_p] * 11 + [c_size_t] + [c_int] * 9 + [c_void_p]),
     "l32_ffn_backward_workspace_bytes": (c_size_t, [c_int64, c_int]),
     "l32_ffn_backward": (c_int, [c_void_p] * 12 + [c_size_t, c_int64, c_int, c_int, c_int, c_void_p]),
     "l32_ffn_lora_forward": (c_int, [c_void_p] * 11 + [c_int64, c_int, c_int, c_int, c_int, c_void_p]),

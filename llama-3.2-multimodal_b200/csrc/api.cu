@@ -849,6 +849,40 @@ int l32_gqa_attention_forward_paged(const void* q, const void* pool_k, const voi
                                kv_heads, head_dim, num_pages, max_pages_per_seq, max_kv_len, dtype, as_stream(stream));
 }
 
+static bool cascade_shape_ok(int batch, int heads, int kv_heads, int head_dim, int max_kv_len, int max_items) {
+    return batch >= 0 && heads > 0 && kv_heads > 0 && (heads % kv_heads) == 0 && heads / kv_heads >= 2 &&
+           heads / kv_heads <= L32_CASCADE_TILE_ROWS && (head_dim == 64 || head_dim == 128) && max_kv_len >= 0 && max_items > 0 &&
+           max_items <= L32_CASCADE_MAX_ITEMS;
+}
+
+size_t l32_gqa_attention_cascade_workspace_bytes(int batch, int heads, int kv_heads, int head_dim, int max_kv_len, int max_items) {
+    if (!cascade_shape_ok(batch, heads, kv_heads, head_dim, max_kv_len, max_items) || batch == 0) return 0;
+    return gqa_attention_cascade_workspace_bytes(batch, heads, kv_heads, head_dim, max_kv_len, max_items);
+}
+
+int l32_gqa_attention_forward_paged_cascade(const void* q, const void* pool_k, const void* pool_v, const int32_t* block_table,
+                                            const int32_t* past_lens, const int32_t* new_lens, const int32_t* plan_items,
+                                            const int32_t* plan_members, const int32_t* plan_seq, void* ctx, void* workspace,
+                                            size_t workspace_bytes, int batch, int heads, int kv_heads, int head_dim, int num_pages,
+                                            int max_pages_per_seq, int max_kv_len, int max_items, int dtype, void* stream) {
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (!paged_shape_ok(batch, 1, heads, kv_heads, head_dim, num_pages, max_pages_per_seq) ||
+        !cascade_shape_ok(batch, heads, kv_heads, head_dim, max_kv_len, max_items) ||
+        static_cast<long long>(max_kv_len) > static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE)
+        return L32_ERR_BAD_SHAPE;
+    if (batch == 0) return L32_OK;
+    if (q == nullptr || pool_k == nullptr || pool_v == nullptr || block_table == nullptr || past_lens == nullptr || ctx == nullptr ||
+        plan_items == nullptr || plan_members == nullptr || plan_seq == nullptr || workspace == nullptr)
+        return L32_ERR_NULL;
+    if (!is_aligned16(q) || !is_aligned16(pool_k) || !is_aligned16(pool_v) || !is_aligned16(ctx)) return L32_ERR_BAD_ALIGN;
+    if (!is_aligned16(workspace) ||
+        workspace_bytes < gqa_attention_cascade_workspace_bytes(batch, heads, kv_heads, head_dim, max_kv_len, max_items))
+        return L32_ERR_WORKSPACE;
+    return gqa_attention_paged_cascade(q, pool_k, pool_v, block_table, past_lens, new_lens, plan_items, plan_members, plan_seq,
+                                       max_items, ctx, workspace, batch, heads, kv_heads, head_dim, num_pages, max_pages_per_seq,
+                                       max_kv_len, dtype, as_stream(stream));
+}
+
 int l32_gemm(const void* a, int64_t lda, int a_mn_major, const void* b, int64_t ldb, int b_mn_major, const void* a1,
              int64_t lda1, const void* b1, int64_t ldb1, void* d, int64_t ldd, int m, int n, int k, int k1, int dtype,
              int cta_group, int max_ctas, void* stream) {

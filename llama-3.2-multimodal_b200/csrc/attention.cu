@@ -56,6 +56,18 @@ struct AttnParams {
     int pages_per_seq, page_kv_heads;
     int packed;               // packed decode: CTA batch index = sequence * page_kv_heads + kv head, its q_len rows are the
                               // query heads of ONE query
+    // Cascade decode (kCascade instances; plan layout in include/l32_ffn.h).  Packed decode shapes (q_len = group, batch =
+    // sequences * page_kv_heads); grid (casc_max_items + sequences * splits, page_kv_heads).  blockIdx.x < casc_max_items:
+    // prefix work item blockIdx.x (past the plan's count: nothing to do); the rest: own-key split (x - casc_max_items) %
+    // splits of sequence (x - casc_max_items) / splits, over its key tiles from its shared tiles on.  Every CTA writes
+    // partials; attention_combine_kernel<T, true> merges them.
+    const void* q;                 // [sequences, page_kv_heads * group, head_dim]: the Q tile is gathered by the softmax warps
+    const int* casc_items;         // [1 + 5 * casc_max_items]
+    const int* casc_members;       // [sequences]
+    const int* casc_seq;           // [sequences][4]
+    int casc_max_items;
+    float* pfx_o;                  // [casc_max_items][page_kv_heads][kQTile][head_dim] fp32: prefix partials, per Q-tile row
+    float2* pfx_ml;                // [casc_max_items][page_kv_heads][kQTile]
 };
 static_assert(L32_KV_PAGE == kKvTile, "a KV-cache page is one key tile");
 
@@ -96,8 +108,38 @@ L32_DEVICE uint64_t add_f32x2(uint64_t a, uint64_t b) {
 
 // kLse: training forward, also stores the per-row log-sum-exp (a separate instantiation: the inference kernel is unchanged)
 // kPaged: K / V from a paged cache, lengths per sequence from device memory (AttnParams, "paged cache")
-template <int kD, typename T, bool kLse, bool kPaged>
+// kCascade (with kPaged): a cascade decode CTA, prefix work item or own-key split (AttnParams, "cascade decode")
+template <int kD, typename T, bool kLse, bool kPaged, bool kCascade = false>
 __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ AttnParams p) {
+    static_assert(!kCascade || (kPaged && !kLse), "the cascade is a paged decode");
+    // cascade: the CTA's work, read after the PDL wait (the plan may be written by earlier work of the stream).  A prefix CTA
+    // past the plan's item count leaves before it allocates anything.  c_item < 0: an own-key CTA of sequence c_seq.
+    int c_item = -1, c_seq = 0, c_split = 0, c_tile0 = 0, c_tiles = 0, c_kv_len = 0, c_member0 = 0, c_members = 1;
+    if constexpr (kCascade) {
+        pdl_wait_prior_grid();
+        const int x = static_cast<int>(blockIdx.x);
+        if (x < p.casc_max_items) {
+            if (x >= p.casc_items[0]) return;
+            const int* it = p.casc_items + 1 + 5 * x;
+            c_item = x;
+            c_seq = it[0];
+            c_tile0 = it[1];
+            c_tiles = it[2];
+            c_member0 = it[3];
+            c_members = it[4];
+            c_kv_len = (c_tile0 + c_tiles) * kKvTile;         // shared pages are full: every prefix key is visible
+        } else {
+            c_seq = (x - p.casc_max_items) / p.splits;
+            c_split = (x - p.casc_max_items) % p.splits;
+            const int n_new = p.new_lens != nullptr ? p.new_lens[c_seq] : 1;
+            c_kv_len = p.past_lens[c_seq] + n_new;
+            const int shared = p.casc_seq[4 * c_seq];
+            const int own = n_new > 0 ? (c_kv_len + kKvTile - 1) / kKvTile - shared : 0;
+            const int per = (own + p.splits - 1) / p.splits;
+            c_tile0 = shared + c_split * per;
+            c_tiles = max(0, min(per, shared + own - c_tile0));
+        }
+    }
     constexpr int kDAtoms = kD / 64;                       // 64-element (128-byte) column blocks of a head
     constexpr int kQBytes = kQTile * kD * 2;
     constexpr int kKBytes = kKvTile * kD * 2;              // also the V tile
@@ -136,7 +178,7 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
         tma_prefetch_desc(&p.map_q);
         tma_prefetch_desc(&p.map_k);
         tma_prefetch_desc(&p.map_v);
-        mbar_init(bar_q, 1);
+        mbar_init(bar_q, kCascade ? kQTile : 1);           // cascade: one arrival per gathered Q row
         for (int i = 0; i < 2; ++i) {
             mbar_init(&bar_k[i], 1);
             mbar_init(&bar_v[i], 1);
@@ -164,7 +206,11 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
     // [q_rows, q_len) are right padding of a ragged call: they see no key and store zeros.
     int kv_len = p.kv_len, past_len = p.past_len, q_rows = p.q_len, tiles_per_split = p.tiles_per_split;
     int seq = b, kvh_pool = kvh;
-    if constexpr (kPaged) {
+    if constexpr (kCascade) {
+        seq = c_seq;                                        // a prefix item reads the pages of its group's first member
+        kvh_pool = static_cast<int>(blockIdx.y);
+        kv_len = c_kv_len;
+    } else if constexpr (kPaged) {
         if (p.packed) {
             seq = b / p.page_kv_heads;
             kvh_pool = b % p.page_kv_heads;
@@ -183,8 +229,12 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
     }
     const int total_tiles = (hi + kKvTile - 1) / kKvTile;
     if constexpr (kPaged) tiles_per_split = (total_tiles + p.splits - 1) / p.splits;   // the host plan, per sequence
-    const int tile0 = split * tiles_per_split;                            // first key tile of this CTA (0 without split-KV)
-    const int ntiles = p.splits > 1 ? max(0, min(tiles_per_split, total_tiles - tile0)) : total_tiles;
+    int tile0 = split * tiles_per_split;                                  // first key tile of this CTA (0 without split-KV)
+    int ntiles = p.splits > 1 ? max(0, min(tiles_per_split, total_tiles - tile0)) : total_tiles;
+    if constexpr (kCascade) {
+        tile0 = c_tile0;
+        ntiles = c_tiles;
+    }
     const int kv_plane = b * p.kv_heads + kvh;
     const int key0 = tile0 * kKvTile;
 
@@ -248,10 +298,12 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
                 }
                 umma_commit<1>(&bar_s[s]);
             };
-            mbar_arrive_expect_tx(bar_q, kQBytes);
+            if constexpr (!kCascade) {                    // (cascade: the softmax warps gather Q)
+                mbar_arrive_expect_tx(bar_q, kQBytes);
 #pragma unroll
-            for (int a = 0; a < kDAtoms; ++a)
-                tma_load_2d(sq + a * (kQTile * 128), &p.map_q, bar_q, head * kD + a * 64, b * p.q_len + q0, kEvictNormal);
+                for (int a = 0; a < kDAtoms; ++a)
+                    tma_load_2d(sq + a * (kQTile * 128), &p.map_q, bar_q, head * kD + a * 64, b * p.q_len + q0, kEvictNormal);
+            }
             load_k(0, pg0);
             if (ntiles > 1) load_k(1, pg1);
             load_v(0, pg0);
@@ -300,6 +352,27 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
         }
     } else {
         // ------------------------------------------------------------------ softmax warps: one query row per thread = one TMEM lane
+        if constexpr (kCascade) {
+            // Q tile row tid = query head tid % group of member tid / group, gathered with plain loads (members are arbitrary
+            // sequences, so no TMA box fits them) and stored where the 128-byte swizzle puts its 16-byte chunks (tile base
+            // 1024-byte aligned: chunk j of row r at r * 128 + (j ^ (r % 8)) * 16 in each 64-column block); rows past the last
+            // member are zeros.  Then a proxy fence: the tcgen05.mma reads the tile through the async proxy.
+            if (ntiles > 0) {
+                const int group = p.q_len, m = tid / group;
+                const bool live = m < c_members;
+                const int qseq = c_item >= 0 ? p.casc_members[c_member0 + (live ? m : 0)] : c_seq;
+                const uint4* src = reinterpret_cast<const uint4*>(static_cast<const T*>(p.q) +
+                                                                  ((static_cast<size_t>(qseq) * p.page_kv_heads + kvh_pool) * group +
+                                                                   tid % group) * kD);
+#pragma unroll
+                for (int c = 0; c < kD / 8; ++c) {
+                    const uint4 v = live ? __ldg(src + c) : make_uint4(0u, 0u, 0u, 0u);
+                    *reinterpret_cast<uint4*>(sq + (c / 8) * (kQTile * 128) + tid * 128 + (((c % 8) ^ (tid & 7)) * 16)) = v;
+                }
+                fence_proxy_async_smem();
+                mbar_arrive(bar_q);
+            }
+        }
         const int qi = q0 + tid;                       // query index inside the sequence
         const int qpos = past_len + qi;                // its absolute position
         const bool row_ok = qi < p.q_len;
@@ -452,7 +525,41 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
             mbar_wait(bar_o, (ntiles - 1) & 1u);
             tc_fence_after();
         }
-        if (p.splits > 1) {
+        if constexpr (kCascade) {
+            // cascade: every CTA leaves partials.  A prefix item's row tid (member tid / group) goes to its item's slot, an
+            // own-key split's row tid < group to the split-KV slot of (sequence, kv head, split)
+            const int group = p.q_len;
+            const bool mine = tid < c_members * group;
+            size_t slot;
+            float* dstf;
+            float2* dml;
+            if (c_item >= 0) {
+                slot = (static_cast<size_t>(c_item) * p.page_kv_heads + kvh_pool) * kQTile + tid;
+                dstf = p.pfx_o + slot * kD;
+                dml = p.pfx_ml + slot;
+            } else {
+                slot = ((static_cast<size_t>(c_seq) * p.page_kv_heads + kvh_pool) * p.splits + c_split) * group + (mine ? tid : 0);
+                dstf = p.part_o + slot * kD;
+                dml = p.part_ml + slot;
+            }
+            if (mine) *dml = make_float2(ntiles > 0 ? m_ref : -INFINITY, ntiles > 0 ? l : 0.f);
+#pragma unroll
+            for (int c = 0; c < kD / 32; ++c) {
+                uint32_t v[32];
+                if (ntiles > 0) {
+                    tmem_ld_32x32b_x32(tmem_o + lane_off + c * 32, v);
+                    tmem_ld_wait();
+                } else {
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) v[j] = 0u;
+                }
+                if (mine) {
+#pragma unroll
+                    for (int j4 = 0; j4 < 8; ++j4)
+                        *reinterpret_cast<uint4*>(dstf + c * 32 + 4 * j4) = make_uint4(v[4 * j4], v[4 * j4 + 1], v[4 * j4 + 2], v[4 * j4 + 3]);
+                }
+            }
+        } else if (p.splits > 1) {
             // split-KV: the unnormalised accumulator row and its (reference, sum) leave for the combine kernel
             const size_t slot = ((static_cast<size_t>(b) * p.heads + head) * p.splits + split) * p.q_len + (row_ok ? qi : 0);
             if (row_ok) p.part_ml[slot] = make_float2(ntiles > 0 ? m_ref : -INFINITY, ntiles > 0 ? l : 0.f);
@@ -518,10 +625,14 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
 }
 
 // Split-KV combine: out[row] = sum_s O_s 2^(m_s - M) / sum_s l_s 2^(m_s - M), M = max_s m_s.  One warp per (batch, head, row).
-template <typename T>
+// kCascade: a cascade decode (packed shapes: batch = sequences * kv_heads, heads = 1, q_len = group); the row's prefix slots
+// (casc_seq[sequence] = (shared tiles, first item, items, row offset), in pfx_o / pfx_ml) come first, then its split slots.
+// Only the prefix slots the plan names are read: the rest of the workspace may hold anything.
+template <typename T, bool kCascade = false>
 __global__ void __launch_bounds__(128) attention_combine_kernel(const float* __restrict__ part_o, const float2* __restrict__ part_ml,
                                                                T* __restrict__ out, int batch, int heads, int q_len, int splits,
-                                                               int d) {
+                                                               int d, const int* __restrict__ casc_seq, const float* __restrict__ pfx_o,
+                                                               const float2* __restrict__ pfx_ml, int kv_heads) {
     pdl_wait_prior_grid();
     const long long w = blockIdx.x * 4ll + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
@@ -530,9 +641,31 @@ __global__ void __launch_bounds__(128) attention_combine_kernel(const float* __r
     const int qi = static_cast<int>(w % q_len);
     const long long bh = w / q_len;                       // b * heads + head
     float mx = -INFINITY;
+    int pf = 0, pn = 0;
+    size_t prow = 0;                                      // the row's slot in item 0; item k adds k * kv_heads * kQTile
+    if constexpr (kCascade) {
+        const int* cs = casc_seq + 4 * (bh / kv_heads);
+        pf = cs[1];
+        pn = cs[2];
+        prow = static_cast<size_t>(bh % kv_heads) * kQTile + cs[3] + qi;
+        for (int k = pf; k < pf + pn; ++k) mx = fmaxf(mx, pfx_ml[static_cast<size_t>(k) * kv_heads * kQTile + prow].x);
+    }
     for (int s = 0; s < splits; ++s) mx = fmaxf(mx, part_ml[(bh * splits + s) * q_len + qi].x);
     float lsum = 0.f;
     float acc[4] = {0.f, 0.f, 0.f, 0.f};                  // d <= 128: 4 columns per lane
+    if constexpr (kCascade) {
+        for (int k = pf; k < pf + pn; ++k) {
+            const size_t slot = static_cast<size_t>(k) * kv_heads * kQTile + prow;
+            const float2 ml = pfx_ml[slot];
+            if (ml.x == -INFINITY) continue;
+            const float sc = exp2f(ml.x - mx);
+            lsum += ml.y * sc;
+            for (int c = 0; c < 4; ++c) {
+                const int col = lane + 32 * c;
+                if (col < d) acc[c] = fmaf(pfx_o[slot * d + col], sc, acc[c]);
+            }
+        }
+    }
     for (int s = 0; s < splits; ++s) {
         const size_t slot = (bh * splits + s) * q_len + qi;
         const float2 ml = part_ml[slot];
@@ -648,9 +781,9 @@ __global__ void __launch_bounds__(128) rope_kv_append_kernel(T* q, const T* __re
     }
 }
 
-template <int kD, typename T, bool kLse, bool kPaged>
+template <int kD, typename T, bool kLse, bool kPaged, bool kCascade = false>
 int launch_attention(const AttnParams& p, cudaStream_t s) {
-    auto* kernel = gqa_attention_kernel<kD, T, kLse, kPaged>;
+    auto* kernel = gqa_attention_kernel<kD, T, kLse, kPaged, kCascade>;
     size_t smem = kQTile * kD * 2 + 4 * kKvTile * kD * 2 + 128;   // tiles + barriers
     if (const char* v = getenv("L32_ATT_ONE_CTA_PER_SM")) {   // experiments only: pad so that only one CTA fits per SM
         if (*v == '1') smem = 160 * 1024;
@@ -671,7 +804,10 @@ int launch_attention(const AttnParams& p, cudaStream_t s) {
         }
     }
     cudaLaunchConfig_t cfg = {};
-    if (p.splits > 1)
+    if (kCascade)
+        cfg.gridDim = dim3(static_cast<unsigned>(p.casc_max_items + (p.batch / p.page_kv_heads) * p.splits),
+                           static_cast<unsigned>(p.page_kv_heads));
+    else if (p.splits > 1)
         cfg.gridDim = dim3(static_cast<unsigned>(p.splits), static_cast<unsigned>(p.heads), static_cast<unsigned>(p.batch));
     else
         cfg.gridDim = dim3(static_cast<unsigned>(p.heads), static_cast<unsigned>(p.batch),
@@ -714,17 +850,9 @@ void attention_split(AttnParams& p, int splits, int kv_len, int head_dim, void* 
     }
 }
 
-// The inference kernel, then (split-KV) the merge of its partials.
-template <bool kPaged>
-int attention_run(const AttnParams& p, int head_dim, int dtype, cudaStream_t s) {
-    int rc;
-    if (dtype == L32_BF16) {
-        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16, false, kPaged>(p, s) : launch_attention<64, __nv_bfloat16, false, kPaged>(p, s);
-    } else {
-        rc = head_dim == 128 ? launch_attention<128, __half, false, kPaged>(p, s) : launch_attention<64, __half, false, kPaged>(p, s);
-    }
-    if (rc != L32_OK || p.splits == 1) return rc;
-    // merge the split-KV partials
+// The merge of the split-KV (kCascade: and prefix) partials.
+template <bool kCascade>
+int launch_combine(const AttnParams& p, int head_dim, int dtype, cudaStream_t s) {
     const long long rows = static_cast<long long>(p.batch) * p.heads * p.q_len;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(static_cast<unsigned>((rows + 3) / 4));
@@ -737,15 +865,30 @@ int attention_run(const AttnParams& p, int head_dim, int dtype, cudaStream_t s) 
     cfg.numAttrs = 1;
     const float* po = p.part_o;
     const float2* pml = p.part_ml;
+    const float* pfo = p.pfx_o;
+    const float2* pfml = p.pfx_ml;
     cudaError_t e;
     if (dtype == L32_BF16)
-        e = cudaLaunchKernelEx(&cfg, attention_combine_kernel<__nv_bfloat16>, po, pml, static_cast<__nv_bfloat16*>(p.out), p.batch,
-                               p.heads, p.q_len, p.splits, head_dim);
+        e = cudaLaunchKernelEx(&cfg, attention_combine_kernel<__nv_bfloat16, kCascade>, po, pml, static_cast<__nv_bfloat16*>(p.out),
+                               p.batch, p.heads, p.q_len, p.splits, head_dim, p.casc_seq, pfo, pfml, p.page_kv_heads);
     else
-        e = cudaLaunchKernelEx(&cfg, attention_combine_kernel<__half>, po, pml, static_cast<__half*>(p.out), p.batch, p.heads, p.q_len,
-                               p.splits, head_dim);
+        e = cudaLaunchKernelEx(&cfg, attention_combine_kernel<__half, kCascade>, po, pml, static_cast<__half*>(p.out), p.batch,
+                               p.heads, p.q_len, p.splits, head_dim, p.casc_seq, pfo, pfml, p.page_kv_heads);
     if (e == cudaSuccess) count_launch();
     return static_cast<int>(e);
+}
+
+// The inference kernel, then (split-KV) the merge of its partials.
+template <bool kPaged>
+int attention_run(const AttnParams& p, int head_dim, int dtype, cudaStream_t s) {
+    int rc;
+    if (dtype == L32_BF16) {
+        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16, false, kPaged>(p, s) : launch_attention<64, __nv_bfloat16, false, kPaged>(p, s);
+    } else {
+        rc = head_dim == 128 ? launch_attention<128, __half, false, kPaged>(p, s) : launch_attention<64, __half, false, kPaged>(p, s);
+    }
+    if (rc != L32_OK || p.splits == 1) return rc;
+    return launch_combine<false>(p, head_dim, dtype, s);
 }
 
 // Paged-cache arguments of rope_kv_append_kernel (null: the contiguous cache).
@@ -898,6 +1041,70 @@ int gqa_attention_paged(const void* q, const void* pool_k, const void* pool_v, c
     }
     attention_split(p, splits, max_kv_len, head_dim, workspace);
     return attention_run<true>(p, head_dim, dtype, s);
+}
+
+// Cascade decode workspace: the own-key split partials (the split-KV layout for `splits` splits, at least one), then the prefix
+// partials, one row per (item, kv head, Q-tile row).  Offsets of part_ml, pfx_o, pfx_ml and the total, each 256-aligned.
+struct CascadeLayout {
+    int splits;
+    size_t ml, pfx_o, pfx_ml, bytes;
+};
+static CascadeLayout cascade_layout(int batch, int heads, int kv_heads, int head_dim, int max_kv_len, int max_items) {
+    CascadeLayout c;
+    c.splits = max(1, decode_splits(batch, 1, heads, kv_heads, max_kv_len));
+    auto up = [](size_t x) { return (x + 255) & ~static_cast<size_t>(255); };
+    const size_t own_rows = static_cast<size_t>(batch) * heads * c.splits;
+    const size_t pfx_rows = static_cast<size_t>(max_items) * kv_heads * kQTile;
+    c.ml = up(own_rows * head_dim * sizeof(float));
+    c.pfx_o = c.ml + up(own_rows * sizeof(float2));
+    c.pfx_ml = c.pfx_o + up(pfx_rows * head_dim * sizeof(float));
+    c.bytes = c.pfx_ml + up(pfx_rows * sizeof(float2));
+    return c;
+}
+
+size_t gqa_attention_cascade_workspace_bytes(int batch, int heads, int kv_heads, int head_dim, int max_kv_len, int max_items) {
+    return cascade_layout(batch, heads, kv_heads, head_dim, max_kv_len, max_items).bytes;
+}
+
+// Cascade decode over a paged cache: one launch of the kCascade instance (prefix items and own-key splits), then the combine.
+int gqa_attention_paged_cascade(const void* q, const void* pool_k, const void* pool_v, const int* block_table, const int* past_lens,
+                                const int* new_lens, const int* items, const int* members, const int* seq_plan, int max_items,
+                                void* out, void* workspace, int batch, int heads, int kv_heads, int head_dim, int num_pages,
+                                int max_pages_per_seq, int max_kv_len, int dtype, cudaStream_t s) {
+    const int group = heads / kv_heads;
+    AttnParams p;
+    int rc = attention_setup(p, q, out, batch * kv_heads, group, 1, 1, head_dim, 0, dtype);
+    if (rc != L32_OK) return rc;
+    p.block_table = block_table;
+    p.past_lens = past_lens;
+    p.new_lens = new_lens;
+    p.pages_per_seq = max_pages_per_seq;
+    p.page_kv_heads = kv_heads;
+    p.packed = 1;
+    const uint64_t planes = static_cast<uint64_t>(num_pages) * kv_heads, plane_elems = static_cast<uint64_t>(kKvTile) * head_dim;
+    rc = make_tensor_map_3d(&p.map_k, pool_k, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
+    if (rc != L32_OK) return rc;
+    rc = make_tensor_map_3d(&p.map_v, pool_v, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
+    if (rc != L32_OK) return rc;
+    const CascadeLayout c = cascade_layout(batch, heads, kv_heads, head_dim, max_kv_len, max_items);
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    p.splits = c.splits;
+    p.part_o = reinterpret_cast<float*>(ws);
+    p.part_ml = reinterpret_cast<float2*>(ws + c.ml);
+    p.pfx_o = reinterpret_cast<float*>(ws + c.pfx_o);
+    p.pfx_ml = reinterpret_cast<float2*>(ws + c.pfx_ml);
+    p.q = q;
+    p.casc_items = items;
+    p.casc_members = members;
+    p.casc_seq = seq_plan;
+    p.casc_max_items = max_items;
+    if (dtype == L32_BF16)
+        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16, false, true, true>(p, s)
+                             : launch_attention<64, __nv_bfloat16, false, true, true>(p, s);
+    else
+        rc = head_dim == 128 ? launch_attention<128, __half, false, true, true>(p, s) : launch_attention<64, __half, false, true, true>(p, s);
+    if (rc != L32_OK) return rc;
+    return launch_combine<true>(p, head_dim, dtype, s);
 }
 
 // Training forward: keys [0, q_len) of the K / V buffers, no past, no split-KV; also writes the per-row log-sum-exp.

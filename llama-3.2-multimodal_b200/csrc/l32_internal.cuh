@@ -168,6 +168,11 @@ int rope_kv_append_paged(void* q, const void* k_new, const void* v_new, const lo
 int gqa_attention_paged(const void* q, const void* pool_k, const void* pool_v, const int* block_table, const int* past_lens,
                         const int* new_lens, void* out, void* workspace, size_t workspace_bytes, int batch, int q_len, int heads,
                         int kv_heads, int head_dim, int num_pages, int max_pages_per_seq, int max_kv_len, int dtype, cudaStream_t s);
+size_t gqa_attention_cascade_workspace_bytes(int batch, int heads, int kv_heads, int head_dim, int max_kv_len, int max_items);
+int gqa_attention_paged_cascade(const void* q, const void* pool_k, const void* pool_v, const int* block_table, const int* past_lens,
+                                const int* new_lens, const int* items, const int* members, const int* seq_plan, int max_items,
+                                void* out, void* workspace, int batch, int heads, int kv_heads, int head_dim, int num_pages,
+                                int max_pages_per_seq, int max_kv_len, int dtype, cudaStream_t s);
 // RoPE angle of rotation pair i (of d / 2) at position `pos`: pos * base^(-2 i / d), cos / sin in fp32.  The forward rotation
 // (rope_kv_append_kernel) and the inverse rotation of the backward epilogues share it, so both use bit-identical angles.
 L32_DEVICE void rope_cos_sin(float pos, int i, int d, float log2_base, float& cs, float& sn) {

@@ -549,10 +549,72 @@ class KVCache:
         return self.key_cache[layer_idx], self.value_cache[layer_idx]
 
 
+# A decode step takes the cascade form only for a group sharing at least this many full pages (64 tokens each): below it the
+# prefix pass and the combine are expected to cost more than the repeated prefix reads they save.  Provisional: not yet set
+# from scripts/cascade_attn_bench.py, which times both forms on each side of it (DESIGN.md, K8 shared prefixes).
+CASCADE_MIN_SHARED_PAGES = 4
+
+
+def cascade_items_capacity(sms: int, kv_heads: int) -> int:
+    """Prefix work items of one cascade decode step (its launch shape): two waves of prefix CTAs over all kv heads."""
+    return max(1, -(-2 * int(sms) // int(kv_heads)))
+
+
+def cascade_plan(tables, past_lens, new_lens, group, max_items, min_shared_pages=CASCADE_MIN_SHARED_PAGES):
+    """The cascade plan of one step (include/l32_ffn.h, l32_gqa_attention_forward_paged_cascade), or None when the step
+    takes the plain form.  Pure Python over the host bookkeeping: tables[r] = the page list of batch row r.
+
+    Only a decode step (every new length 1) with 2 <= group <= 128 has one.  Rows whose pages start with the same page form a
+    group; its shared prefix is the longest run of identical leading pages of all members, cut below each member's
+    past length (full pages the step does not write).  A group needs >= 2 members and >= min_shared_pages shared pages.
+    Members (in row order) are cut into chunks of 128 // group (one query tile); chunks past max_items are left out (their
+    rows stay unshared).  Each chunk's prefix tiles are divided into items of tau tiles, tau >= 2 the least with at most
+    max_items items in all.  Returns (items [(first_row, tile0, tiles, member0, members)], members [rows],
+    seq [(shared_tiles, first_item, items, row0)] per row)."""
+    if not tables or any(n != 1 for n in new_lens) or not 2 <= group <= 128:
+        return None
+    by_first = {}
+    for r, pages in enumerate(tables):
+        if past_lens[r] >= ops.KV_PAGE:
+            by_first.setdefault(pages[0], []).append(r)
+    per_chunk = 128 // group
+    chunks = []
+    for rows in by_first.values():
+        if len(rows) < 2:
+            continue
+        full = min(past_lens[r] // ops.KV_PAGE for r in rows)
+        first = tables[rows[0]]
+        k = 0
+        while k < full and all(tables[r][k] == first[k] for r in rows):
+            k += 1
+        if k < min_shared_pages:
+            continue
+        for c0 in range(0, len(rows), per_chunk):
+            if len(chunks) < max_items:
+                chunks.append((rows[c0:c0 + per_chunk], k))
+    if not chunks:
+        return None
+    tau = max(2, -(-sum(k for _, k in chunks) // max_items))
+    while sum(-(-k // tau) for _, k in chunks) > max_items:
+        tau += 1
+    items, members, seq = [], [], [(0, 0, 0, 0)] * len(tables)
+    for rows, k in chunks:
+        first_item, m0 = len(items), len(members)
+        members.extend(rows)
+        for t0 in range(0, k, tau):
+            items.append((rows[0], t0, min(tau, k - t0), m0, len(rows)))
+        for i, r in enumerate(rows):
+            seq[r] = (k, first_item, len(items) - first_item, i * group)
+    return items, members, seq
+
+
 class PagedKVCache:
     """KV cache for serving several sequences at once (inference only): keys / values live in pages of 64 tokens
     (ops.KV_PAGE, one key tile of the attention kernel) named by a block table, and every sequence has its own length.
     A finished sequence hands its pages back (`free_sequence`) and a new one can join in the same step (`add_sequence`).
+    `fork` starts a sequence that shares its parent's full pages (a system prompt, parallel samples of one prompt): pages
+    are reference-counted, a shared page is full and never written again, and a decode step whose batch holds such a group
+    reads each shared prefix once per query tile (the cascade form of the attention, planned by set_batch).
 
     Per layer one pool for K and one for V, [num_pages, kv_heads, 64, head_dim], zero-initialised on the layer's first
     forward; page index p names the same slot in every layer, so one allocator serves all layers.  The host keeps the
@@ -572,6 +634,7 @@ class PagedKVCache:
         self.num_pages, self.max_batch, self.max_pages_per_seq = int(num_pages), int(max_batch), int(max_pages_per_seq)
         self.page_size = ops.KV_PAGE
         self._free = list(range(self.num_pages - 1, -1, -1))   # pop() hands out the lowest free page first
+        self._refs = [0] * self.num_pages                        # sequences holding each page; free <=> 0
         self._pages: dict = {}                                   # sequence id -> its pages, in logical order
         self._len: dict = {}                                     # sequence id -> tokens cached
         self._next_id = 0
@@ -591,6 +654,20 @@ class PagedKVCache:
             self.block_table = self._dev[:t].view(self.max_batch, self.max_pages_per_seq)
             self.past_lens = self._dev[t:t + self.max_batch]
             self.new_lens = self._dev[t + self.max_batch:]
+        # cascade plan (cascade_plan), a buffer of its own: items [1 + 5 * cap], members [max_batch], per row [max_batch, 4];
+        # cap covers any kv_heads >= 1.  Planned once the attention's geometry is known (the first paged forward).
+        self.cascade = False                                     # the last set_batch planned a cascade decode step
+        self.cascade_geometry = None                             # (group, kv_heads) of the first paged forward
+        self.cascade_max_items = None
+        self._plan_dev = self.plan_items = self.plan_members = self.plan_seq = None
+        self._plan_uploaded = False                               # the device plan is not an empty one
+        if self.device is not None:
+            self._sms = torch.cuda.get_device_properties(self.device).multi_processor_count
+            cap = cascade_items_capacity(self._sms, 1)
+            self._plan_dev = torch.zeros(1 + 5 * cap + 5 * self.max_batch, dtype=torch.int32, device=self.device)
+            self.plan_items = self._plan_dev[:1 + 5 * cap]
+            self.plan_members = self._plan_dev[1 + 5 * cap:1 + 5 * cap + self.max_batch]
+            self.plan_seq = self._plan_dev[1 + 5 * cap + self.max_batch:].view(self.max_batch, 4)
 
     # -- allocator
     @property
@@ -610,13 +687,46 @@ class PagedKVCache:
         return sid
 
     def free_sequence(self, sid: int) -> None:
-        """Hand the sequence's pages back.  If it is part of the current batch, that batch is dropped: call set_batch again
-        before the next forward."""
+        """Hand the sequence's pages back (a page shared with a forked sequence stays with it).  If it is part of the current
+        batch, that batch is dropped: call set_batch again before the next forward."""
         pages = self._pages.pop(sid)
         del self._len[sid]
-        self._free.extend(reversed(pages))
+        for p in pages:
+            self._refs[p] -= 1
+        self._free.extend(p for p in reversed(pages) if self._refs[p] == 0)
         if sid in self.batch_ids:
             self.batch_ids, self.batch_new_lens = [], []
+
+    def fork(self, sid: int) -> int:
+        """A new sequence that starts as a copy of `sid` (between steps): it shares the parent's full pages by reference and
+        gets a copy of the parent's partial last page, if any (a stream-ordered device copy in every layer pool on the current
+        stream).  Raises before anything changes when no page is free for that copy."""
+        if sid not in self._pages:
+            raise ValueError(f"fork: {sid} is not a live sequence")
+        n = self._len[sid]
+        full, tail = n // self.page_size, n % self.page_size
+        if tail and not self._free:
+            raise RuntimeError(f"PagedKVCache out of pages: fork of sequence {sid} needs 1 more, 0 free of {self.num_pages}")
+        pages = self._pages[sid][:full]
+        for p in pages:
+            self._refs[p] += 1
+        if tail:
+            old, new = self._pages[sid][full], self._take()
+            for pool in self._pool_k + self._pool_v:
+                if pool is not None:
+                    pool[new].copy_(pool[old])
+            pages = pages + [new]
+        child = self.add_sequence()
+        self._pages[child], self._len[child] = pages, n
+        return child
+
+    def refcount(self, page: int) -> int:
+        return self._refs[page]
+
+    def _take(self) -> int:
+        p = self._free.pop()
+        self._refs[p] = 1
+        return p
 
     def length(self, sid: int) -> int:
         return self._len[sid]
@@ -647,7 +757,7 @@ class PagedKVCache:
             raise RuntimeError(f"PagedKVCache out of pages: this step needs {sum(want)} more, {len(self._free)} free of "
                                f"{self.num_pages}")
         for sid, w in zip(ids, want):
-            self._pages[sid].extend(self._free.pop() for _ in range(w))
+            self._pages[sid].extend(self._take() for _ in range(w))
         self.batch_ids, self.batch_new_lens = ids, new_lens
         host = torch.zeros(self.max_batch * (self.max_pages_per_seq + 2), dtype=torch.int32,
                            pin_memory=self._dev is not None)
@@ -665,6 +775,31 @@ class PagedKVCache:
         if self._dev is not None:
             # torch's pinned-memory allocator keeps `host` from being reused until this copy has run, so no host-side wait
             self._dev.copy_(host, non_blocking=True)
+        self._plan_step(ids, new_lens)
+
+    def _plan_step(self, ids, new_lens) -> None:
+        """Plan the step's cascade (cascade_plan) and upload the plan of a decode step.  Once a plan has been uploaded, an
+        empty one replaces it when nothing is shared: a CUDA graph captured over a cascade-form step stays correct when the
+        groups change or vanish.  A cache that never shares uploads nothing."""
+        self.cascade = False
+        if self.cascade_geometry is None or any(n != 1 for n in new_lens):
+            return
+        group, kv_heads = self.cascade_geometry
+        self.cascade_max_items = cascade_items_capacity(self._sms, kv_heads)
+        plan = cascade_plan([self._pages[s] for s in ids], [self._len[s] for s in ids], new_lens, group, self.cascade_max_items)
+        self.cascade = plan is not None
+        if plan is None and not self._plan_uploaded:
+            return
+        self._plan_uploaded = plan is not None
+        host = torch.zeros(self._plan_dev.numel(), dtype=torch.int32, pin_memory=True)
+        if plan is not None:
+            items, members, seq = plan
+            cap = self.plan_items.numel()
+            host[0] = len(items)
+            host[1:1 + 5 * len(items)] = torch.tensor(items, dtype=torch.int32).flatten()
+            host[cap:cap + len(members)] = torch.tensor(members, dtype=torch.int32)
+            host[cap + self.max_batch:cap + self.max_batch + 4 * len(seq)] = torch.tensor(seq, dtype=torch.int32).flatten()
+        self._plan_dev.copy_(host, non_blocking=True)
 
     def advance(self) -> None:
         """After the step's last layer: every sequence of the batch now holds its new tokens."""
@@ -849,8 +984,16 @@ class GroupQueryAttention(nn.Module):
         q, k, v = self._qkv(hidden_states)
         pk, pv = cache.pools(self.layer_idx or 0, self.num_kv_groups, self.head_dim, q.dtype, q.device)
         ops.rope_kv_append_paged(q, k, v, pos, pk, pv, cache.block_table, cache.past_lens, cache.new_lens, self.rope_base)
-        ctx = ops.gqa_attention_forward_paged(q, pk, pv, cache.block_table, cache.past_lens, cache.new_lens,
-                                              max_kv_len=cache.max_kv_len)
+        geometry = (self.group_size, self.num_kv_groups)
+        if cache.cascade_geometry is None:
+            cache.cascade_geometry = geometry                 # the steps planned from now on fit this attention
+        if t == 1 and cache.cascade and cache.cascade_geometry == geometry:
+            ctx = ops.gqa_attention_forward_paged_cascade(q, pk, pv, cache.block_table, cache.past_lens, cache.new_lens,
+                                                          cache.plan_items, cache.plan_members, cache.plan_seq,
+                                                          cache.cascade_max_items, max_kv_len=cache.max_kv_len)
+        else:
+            ctx = ops.gqa_attention_forward_paged(q, pk, pv, cache.block_table, cache.past_lens, cache.new_lens,
+                                                  max_kv_len=cache.max_kv_len)
         return self._project(self.out_proj, ctx)
 
     def forward(self, hidden_states, attention_mask=None, position_ids=None, kv_cache=None):

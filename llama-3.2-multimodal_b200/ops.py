@@ -542,6 +542,36 @@ def gqa_attention_forward_paged(q, pool_k, pool_v, block_table, past_lens, new_l
     return ctx
 
 
+def gqa_attention_forward_paged_cascade(q, pool_k, pool_v, block_table, past_lens, new_lens, plan_items, plan_members, plan_seq,
+                                        max_items, *, max_kv_len=None):
+    """ctx [b, 1, heads*d] of a decode step whose sequences share prefix pages: the same result as gqa_attention_forward_paged
+    (up to the order of the softmax sums), computed as a prefix pass that reads each shared prefix once per query tile of up
+    to 128 // group member sequences, an own-key pass over each sequence's remaining keys, and the combine.  The plan
+    (int32 device buffers: plan_items [>= 1 + 5 * max_items], plan_members [>= b], plan_seq [>= b, 4]; layout in
+    include/l32_ffn.h) is trusted like the table: PagedKVCache builds it (cascade_plan).  max_items fixes the launch shape."""
+    _check_cuda(q, pool_k, pool_v, block_table, past_lens, new_lens, plan_items, plan_members, plan_seq)
+    b, t, heads, kvh, d, num_pages, max_pages = _paged_args(q, pool_k, pool_v, block_table, past_lens, new_lens,
+                                                            "gqa_attention_forward_paged_cascade")
+    if t != 1:
+        raise L32Error(f"gqa_attention_forward_paged_cascade: a decode step has one query per sequence, got q_len {t}")
+    for name, ten, n in (("plan_items", plan_items, 1 + 5 * int(max_items)), ("plan_members", plan_members, b),
+                         ("plan_seq", plan_seq, 4 * b)):
+        if ten.dtype != torch.int32 or not ten.is_contiguous() or ten.numel() < n:
+            raise L32Error(f"gqa_attention_forward_paged_cascade: {name} must be contiguous int32 with >= {n} elements")
+    max_kv_len = max_pages * KV_PAGE if max_kv_len is None else int(max_kv_len)
+    ctx = torch.empty_like(q)
+    L = lib()
+    ws_bytes = L.l32_gqa_attention_cascade_workspace_bytes(b, heads, kvh, d, max_kv_len, int(max_items))
+    ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=q.device)
+    with torch.cuda.device(q.device):
+        check(L.l32_gqa_attention_forward_paged_cascade(_ptr(q), _ptr(pool_k), _ptr(pool_v), _ptr(block_table), _ptr(past_lens),
+                                                        _ptr(new_lens), _ptr(plan_items), _ptr(plan_members), _ptr(plan_seq),
+                                                        _ptr(ctx), _ptr(ws), ws_bytes, b, heads, kvh, d, num_pages, max_pages,
+                                                        max_kv_len, int(max_items), _dtype_code(q), _stream(q)),
+              "l32_gqa_attention_forward_paged_cascade")
+    return ctx
+
+
 def _attention_train_args(q_rot, cache_k, cache_v, key_keep):
     """Shapes of a training call (keys = queries, no past) and the key_keep bytes, checked as gqa_attention_forward does."""
     b, t = q_rot.shape[0], q_rot.shape[1]
