@@ -58,7 +58,8 @@ extern "C" {
  *    l32_rope_kv_append, l32_gqa_attention_forward; later, additively: l32_gqa_attention_forward_train / _backward, and
  *    the tensor-parallel attention GEMMs l32_tp_linear_group_forward_allgather, l32_tp_linear_forward_allgather and
  *    l32_tp_linear_group_backward_dx_reduce_scatter, the paged KV cache l32_rope_kv_append_paged and
- *    l32_gqa_attention_forward_paged, and its cascade decode l32_gqa_attention_forward_paged_cascade. */
+ *    l32_gqa_attention_forward_paged, its cascade decode l32_gqa_attention_forward_paged_cascade, and next-token
+ *    sampling l32_sample_tokens. */
 L32_API int l32_abi_version(void);
 /* Number of CUDA kernels this library has launched in the calling process so far (monotonic). */
 L32_API unsigned long long l32_kernel_launch_count(void);
@@ -382,6 +383,32 @@ L32_API int l32_gqa_attention_forward_paged_cascade(const void* q, const void* p
                                                     size_t workspace_bytes, int batch, int heads, int kv_heads, int head_dim,
                                                     int num_pages, int max_pages_per_seq, int max_kv_len, int max_items, int dtype,
                                                     void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Next-token sampling: one token per row of 16-bit logits [batch, vocab] (row pitch = vocab), written to tokens_out [batch]
+ * (int64).  Replaces the torch sampler of the reference's decode loop (Inference/Inference.py, select_next_token).
+ * Per-row parameters, device arrays of `batch` entries: temperature (f32), top_k (i32), top_p (f32), seed (u64),
+ * position (i64, the position of the token being sampled).  For row r:
+ *   1. Greedy: temperature <= 0 or NaN -> the smallest index among the maximal logits (torch.argmax's choice).
+ *   2. Otherwise z_i = logit_i / temperature in fp32.
+ *   3. Top-k, if 0 < top_k < vocab: keep every token with logit_i >= v_k, the top_k-th largest logit counted with
+ *      multiplicity; all ties at v_k survive.
+ *   4. Top-p, if top_p < 1: over the survivors' softmax of z, keep every token with logit_i >= v_p, the largest logit value
+ *      whose survivors at or above it carry at least top_p of the survivors' mass (top_p <= 0: only the maximal value).
+ *   5. -inf is never kept.
+ *   6. Return the argmax over kept i of z_i + g_i (smallest index on ties), g_i = -log(-log(u_i)): an exact sample of the
+ *      kept set's softmax.  u_i = ((out[i & 3] >> 8) + 0.5) * 2^-24 with out = Philox4x32-10 of counter
+ *      (i >> 2, 0, position_lo, position_hi) under key (seed_lo, seed_hi).
+ * A draw is a function of (logits row, parameters, seed, position) only: not of the batch, the row index or graph capture.
+ * Values outside the contract are clamped: top_k <= 0 or >= vocab means no top-k, top_p >= 1 or NaN means no top-p.
+ * A row without a finite logit returns 0.  The parameter values are TRUSTED (the Python TokenSampler validates them).
+ * kept_min_logit: optional [batch] f32, the smallest kept logit of each row (greedy: the maximum; no finite logit: -inf);
+ * with it NULL nothing extra is computed.  8 <= vocab <= L32_SAMPLE_MAX_VOCAB, vocab % 8 == 0, logits 16-byte aligned;
+ * batch == 0 is a no-op.  One launch (a cluster of up to 8 CTAs per row), deterministic, graph-capturable. */
+#define L32_SAMPLE_MAX_VOCAB 262144
+L32_API int l32_sample_tokens(const void* logits, const float* temperature, const int32_t* top_k, const float* top_p,
+                              const uint64_t* seed, const int64_t* position, int64_t* tokens_out, float* kept_min_logit, int batch,
+                              int vocab, int dtype, void* stream);
 
 /* General tiled GEMM used by the entry points above (exposed for tests, tuning and the tensor-parallel
  * host code):  D[m,n] = A[m,k] B[n,k]^T  (+ A1 B1^T when a1 != NULL).

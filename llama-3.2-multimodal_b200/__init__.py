@@ -20,10 +20,12 @@ from .modules import (  # noqa: F401
     LinearLoRAFunction,
     RMSNormFunction,
     SwiGLUFunction,
+    TokenSampler,
     block_tail,
     chain_block_norms,
     convert_feedforward_to_fused,
     convert_instances,
+    last_token_logits,
     lm_head_loss,
     patch_reference,
     shift_labels,
@@ -33,5 +35,5 @@ __all__ = [
     "FFNFunction", "FFNLoRAFunction", "FusedFeedForward", "FusedFeedforward", "FusedSwiGLU", "LLAMARMSNorm", "Linear_LORA",
     "LinearFunction", "RMSNormFunction", "SwiGLUFunction", "block_tail", "convert_feedforward_to_fused", "convert_instances",
     "patch_reference", "BlockTailFunction", "LinearLoRAFunction", "chain_block_norms", "LMHeadCEFunction", "lm_head_loss", "shift_labels", "GroupQueryAttention", "KVCache",
-    "GQAAttentionFunction", "PagedKVCache",
+    "GQAAttentionFunction", "PagedKVCache", "TokenSampler", "last_token_logits",
 ]

@@ -883,6 +883,23 @@ int l32_gqa_attention_forward_paged_cascade(const void* q, const void* pool_k, c
                                        max_kv_len, dtype, as_stream(stream));
 }
 
+// Next-token sampling (no reference kernel: the reference's decode loop samples with torch, Inference/Inference.py
+// select_next_token).  The per-row parameters live in device memory and are trusted, like the paged cache's tables.
+int l32_sample_tokens(const void* logits, const float* temperature, const int32_t* top_k, const float* top_p, const uint64_t* seed,
+                      const int64_t* position, int64_t* tokens_out, float* kept_min_logit, int batch, int vocab, int dtype,
+                      void* stream) {
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (batch < 0 || vocab < 8 || vocab > L32_SAMPLE_MAX_VOCAB || (vocab % 8) != 0) return L32_ERR_BAD_SHAPE;
+    if (batch == 0) return L32_OK;
+    if (logits == nullptr || temperature == nullptr || top_k == nullptr || top_p == nullptr || seed == nullptr ||
+        position == nullptr || tokens_out == nullptr)
+        return L32_ERR_NULL;
+    if (!is_aligned16(logits)) return L32_ERR_BAD_ALIGN;
+    return sample_tokens(logits, temperature, top_k, top_p, reinterpret_cast<const unsigned long long*>(seed),
+                         reinterpret_cast<const long long*>(position), reinterpret_cast<long long*>(tokens_out), kept_min_logit,
+                         batch, vocab, dtype, as_stream(stream));
+}
+
 int l32_gemm(const void* a, int64_t lda, int a_mn_major, const void* b, int64_t ldb, int b_mn_major, const void* a1,
              int64_t lda1, const void* b1, int64_t ldb1, void* d, int64_t ldd, int m, int n, int k, int k1, int dtype,
              int cta_group, int max_ctas, void* stream) {

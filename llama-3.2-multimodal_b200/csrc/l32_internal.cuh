@@ -187,6 +187,11 @@ int gqa_attention_backward(const void* d_ctx, const void* q, const void* cache_k
                            int q_len, int heads, int kv_heads, int head_dim, int max_len, int causal, float rope_base, int dtype,
                            cudaStream_t s);
 
+// ---- sampling.cu : next-token sampling (contract: l32_sample_tokens); one thread-block cluster per row
+int sample_tokens(const void* logits, const float* temperature, const int* top_k, const float* top_p,
+                  const unsigned long long* seed, const long long* position, long long* tokens_out, float* kept_min_logit,
+                  int batch, int vocab, int dtype, cudaStream_t s);
+
 // ---- tp.cu : tensor-parallel glue (cross-GPU flags, reduction of the partial slots)
 cudaError_t tp_signal(void* const* peer_flags, int world, int index, uint32_t value, uint32_t* zero8, cudaStream_t s);
 cudaError_t tp_peer_copy(void* dst, const void* src, size_t bytes, int ctas, int warps, int unroll, int seg_bytes,

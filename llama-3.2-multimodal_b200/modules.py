@@ -15,6 +15,8 @@ never return a gradient for a None input and never mutate caller tensors.
 """
 from __future__ import annotations
 
+import math
+
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -25,7 +27,7 @@ __all__ = [
     "RMSNormFunction", "LLAMARMSNorm", "SwiGLUFunction", "FusedSwiGLU", "LinearFunction", "Linear_LORA", "FFNFunction", "FFNLoRAFunction",
     "FusedFeedforward", "FusedFeedForward", "convert_feedforward_to_fused", "patch_reference", "convert_instances", "block_tail",
     "BlockTailFunction", "LinearLoRAFunction", "chain_block_norms", "LMHeadCEFunction", "lm_head_loss", "shift_labels", "GroupQueryAttention", "KVCache",
-    "GQAAttentionFunction", "PagedKVCache",
+    "GQAAttentionFunction", "PagedKVCache", "TokenSampler", "last_token_logits",
 ]
 
 
@@ -1081,6 +1083,115 @@ def lm_head_loss(lm_head, hidden_states, labels=None, ignore_index=-100):
         return logits, loss
     loss, logits = LMHeadCEFunction.apply(hidden_states, w, shift_labels(labels, ignore_index), ignore_index)
     return logits, loss
+
+
+# ------------------------------------------------------------------------------------------------ next token
+def last_token_logits(lm_head, hidden_states, new_lens=None):
+    """Logits [b, V] of each sequence's last valid position only: row new_lens[r] - 1 of hidden_states [b, t, H] (a paged
+    step's PagedKVCache.new_lens, int32 in device memory), or t - 1 when new_lens is None.  The gather runs on the device (no
+    host synchronisation, so a CUDA graph can capture it); a row with new_lens 0 reads position 0 and its logits mean
+    nothing.  A bias-free 16-bit head runs ops.linear_forward (the weight-streaming small-M kernel up to 128 rows, the tiled
+    GEMM above); any other head is called on the gathered rows."""
+    b, t, hidden = hidden_states.shape
+    if new_lens is None:
+        rows = hidden_states[:, t - 1]
+    else:
+        idx = (new_lens[:b].to(torch.int64) - 1).clamp_(0, t - 1)
+        rows = torch.gather(hidden_states, 1, idx.view(b, 1, 1).expand(b, 1, hidden)).view(b, hidden)
+    w = lm_head.weight
+    if (ops.supported(rows) and w.is_cuda and w.dtype == rows.dtype and getattr(lm_head, "bias", None) is None and
+            w.shape[0] % 8 == 0 and hidden % 8 == 0 and b > 0):
+        return ops.linear_forward(rows.contiguous(), w)
+    return lm_head(rows)
+
+
+class TokenSampler:
+    """Next-token sampling for a decode loop (ops.sample_tokens): per-row temperature / top-k / top-p / seed in static device
+    buffers and a static [max_batch] int64 output, so a CUDA graph that captures `sampler(logits, position)` stays valid while
+    set_params changes the parameters between replays, and the token address it returns never moves.
+
+    A draw depends only on (logits row, parameters, seed, position): siblings forked from one prompt diverge by their seeds,
+    and a request replays exactly with the same seed.  The position of the token being sampled in a PagedKVCache step is
+    cache.past_lens[:b] + cache.new_lens[:b].  With device=None (and no CUDA) only the host staging is kept."""
+
+    def __init__(self, max_batch: int, device=None):
+        if max_batch <= 0:
+            raise ValueError("TokenSampler: max_batch must be positive")
+        self.max_batch = int(max_batch)
+        if device is None and torch.cuda.is_available():
+            device = torch.device("cuda", torch.cuda.current_device())
+        self.device = None if device is None else torch.device(device)
+        m = self.max_batch
+        # one byte buffer: seed int64 [m], temperature float32 [m], top_k int32 [m], top_p float32 [m]
+        self._nbytes = 20 * m
+        self._host = self._stage([0.0] * m, [0] * m, [1.0] * m, [0] * m)
+        self._dev = self.tokens = None
+        self.seed = self.temperature = self.top_k = self.top_p = None
+        if self.device is not None:
+            self._dev = torch.zeros(self._nbytes, dtype=torch.uint8, device=self.device)
+            self.seed, self.temperature, self.top_k, self.top_p = self._views(self._dev)
+            self.tokens = torch.zeros(m, dtype=torch.int64, device=self.device)
+            self._dev.copy_(self._host)
+
+    def _views(self, buf):
+        m = self.max_batch
+        return (buf[:8 * m].view(torch.int64), buf[8 * m:12 * m].view(torch.float32), buf[12 * m:16 * m].view(torch.int32),
+                buf[16 * m:].view(torch.float32))
+
+    def _stage(self, temperature, top_k, top_p, seed):
+        host = torch.zeros(self._nbytes, dtype=torch.uint8, pin_memory=self.device is not None)
+        sd, tt, tk, tp = self._views(host)
+        n = len(temperature)
+        tt[:n] = torch.tensor(temperature, dtype=torch.float32)
+        tk[:n] = torch.tensor(top_k, dtype=torch.int32)
+        tp[:n] = torch.tensor(top_p, dtype=torch.float32)
+        sd[:n] = torch.tensor([v - (1 << 64) if v >= 1 << 63 else v for v in seed], dtype=torch.int64)   # u64 bits
+        tp[n:] = 1.0                      # rows past the batch: greedy
+        return host
+
+    def set_params(self, temperature, top_k=0, top_p=1.0, seed=0) -> None:
+        """Per-row sampling parameters for the next calls: scalars (every row) or lists (one entry per row; lists must agree
+        in length, at most max_batch).  temperature: finite, >= 0 (0 = greedy); top_k: int >= 0 (0 = off); top_p: in (0, 1]
+        (1 = off); seed: int in [0, 2^64).  Validated on the host: raises before anything is uploaded.  The upload is a
+        stream-ordered copy from pinned memory on the current stream."""
+        cols = {"temperature": temperature, "top_k": top_k, "top_p": top_p, "seed": seed}
+        lens = {len(v) for v in cols.values() if isinstance(v, (list, tuple))}
+        if len(lens) > 1:
+            raise ValueError(f"TokenSampler.set_params: per-row lists of different lengths {sorted(lens)}")
+        n = lens.pop() if lens else self.max_batch
+        if not 0 < n <= self.max_batch:
+            raise ValueError(f"TokenSampler.set_params: {n} rows for a sampler of max_batch {self.max_batch}")
+        rows = {k: (list(v) if isinstance(v, (list, tuple)) else [v] * n) for k, v in cols.items()}
+        for t in rows["temperature"]:
+            if not (isinstance(t, (int, float)) and math.isfinite(t) and t >= 0):
+                raise ValueError(f"TokenSampler.set_params: temperature must be finite and >= 0, got {t!r}")
+        for k in rows["top_k"]:
+            if isinstance(k, bool) or not isinstance(k, int) or not 0 <= k <= 0x7fffffff:
+                raise ValueError(f"TokenSampler.set_params: top_k must be an int >= 0, got {k!r}")
+        for p in rows["top_p"]:
+            if not (isinstance(p, (int, float)) and 0 < p <= 1):
+                raise ValueError(f"TokenSampler.set_params: top_p must lie in (0, 1], got {p!r}")
+        for sd in rows["seed"]:
+            if isinstance(sd, bool) or not isinstance(sd, int) or not 0 <= sd < 1 << 64:
+                raise ValueError(f"TokenSampler.set_params: seed must be an int in [0, 2^64), got {sd!r}")
+        host = self._stage(rows["temperature"], rows["top_k"], rows["top_p"], rows["seed"])
+        self._host = host                   # (the last upload's contents, for inspection)
+        if self._dev is not None:
+            # torch's pinned-memory allocator keeps `host` from being reused until this copy has run, so no host-side wait
+            self._dev.copy_(host, non_blocking=True)
+
+    def __call__(self, logits, position, want_kept_min=False):
+        """Tokens int64 [b] for logits [b, V] (b <= max_batch): a view of the static output buffer.  position: int64 (or
+        int32) device tensor with >= b entries, the position of each row's token being sampled."""
+        if self.device is None:
+            raise RuntimeError("TokenSampler: built without a device")
+        b = logits.shape[0]
+        if b > self.max_batch:
+            raise ValueError(f"TokenSampler: {b} rows for a sampler of max_batch {self.max_batch}")
+        if position.dtype != torch.int64:
+            position = position.to(torch.int64)
+        return ops.sample_tokens(logits, self.temperature, self.top_k, self.top_p, self.seed, position.contiguous(),
+                                 out=self.tokens, want_kept_min=want_kept_min)
 
 
 def _mllama_forward(self, input_ids=None, pixel_values=None, attention_mask=None, position_ids=None, image_mask=None,

@@ -572,6 +572,38 @@ def gqa_attention_forward_paged_cascade(q, pool_k, pool_v, block_table, past_len
     return ctx
 
 
+# --------------------------------------------------------------------------------------------- next-token sampling
+SAMPLE_MAX_VOCAB = 262144   # L32_SAMPLE_MAX_VOCAB
+
+
+def sample_tokens(logits, temperature, top_k, top_p, seed, position, *, out=None, want_kept_min=False):
+    """One token per row of logits [b, V] (16-bit): greedy where temperature <= 0, otherwise temperature / top-k / top-p and a
+    Gumbel-max draw from a Philox stream keyed by seed and counted by position (contract: include/l32_ffn.h,
+    l32_sample_tokens).  Per-row device parameters with >= b entries: temperature float32, top_k int32, top_p float32, seed
+    int64 (the bits of a u64), position int64.  Returns tokens int64 [b] (written into `out[:b]` when given), and with
+    want_kept_min also the smallest kept logit of each row (float32 [b]).  Nothing synchronises; graph-capturable."""
+    _check_cuda(logits, temperature, top_k, top_p, seed, position, out)
+    if logits.dim() != 2 or not logits.is_contiguous():
+        raise L32Error(f"sample_tokens: logits must be contiguous [batch, vocab], got {tuple(logits.shape)}")
+    b, vocab = logits.shape
+    if not (8 <= vocab <= SAMPLE_MAX_VOCAB and vocab % 8 == 0):
+        raise L32Error(f"sample_tokens: vocab {vocab} outside 8..{SAMPLE_MAX_VOCAB} or not a multiple of 8")
+    for name, ten, dt in (("temperature", temperature, torch.float32), ("top_k", top_k, torch.int32),
+                          ("top_p", top_p, torch.float32), ("seed", seed, torch.int64), ("position", position, torch.int64)):
+        if ten.dtype != dt or not ten.is_contiguous() or ten.numel() < b:
+            raise L32Error(f"sample_tokens: {name} must be contiguous {dt} with >= {b} entries")
+    if out is None:
+        out = torch.empty(b, dtype=torch.int64, device=logits.device)
+    elif out.dtype != torch.int64 or not out.is_contiguous() or out.numel() < b:
+        raise L32Error(f"sample_tokens: out must be contiguous int64 with >= {b} entries")
+    kept = torch.empty(b, dtype=torch.float32, device=logits.device) if want_kept_min else None
+    with torch.cuda.device(logits.device):
+        check(lib().l32_sample_tokens(_ptr(logits), _ptr(temperature), _ptr(top_k), _ptr(top_p), _ptr(seed), _ptr(position),
+                                      _ptr(out), _ptr(kept), b, vocab, _dtype_code(logits), _stream(logits)),
+              "l32_sample_tokens")
+    return (out[:b], kept) if want_kept_min else out[:b]
+
+
 def _attention_train_args(q_rot, cache_k, cache_v, key_keep):
     """Shapes of a training call (keys = queries, no past) and the key_keep bytes, checked as gqa_attention_forward does."""
     b, t = q_rot.shape[0], q_rot.shape[1]
