@@ -58,8 +58,9 @@ extern "C" {
  *    l32_rope_kv_append, l32_gqa_attention_forward; later, additively: l32_gqa_attention_forward_train / _backward, and
  *    the tensor-parallel attention GEMMs l32_tp_linear_group_forward_allgather, l32_tp_linear_forward_allgather and
  *    l32_tp_linear_group_backward_dx_reduce_scatter, the paged KV cache l32_rope_kv_append_paged and
- *    l32_gqa_attention_forward_paged, its cascade decode l32_gqa_attention_forward_paged_cascade, and next-token
- *    sampling l32_sample_tokens. */
+ *    l32_gqa_attention_forward_paged, its cascade decode l32_gqa_attention_forward_paged_cascade, next-token
+ *    sampling l32_sample_tokens, and speculative decoding l32_gqa_attention_forward_paged_verify,
+ *    l32_gqa_attention_verify_workspace_bytes, l32_ngram_draft_paged and l32_speculative_accept. */
 L32_API int l32_abi_version(void);
 /* Number of CUDA kernels this library has launched in the calling process so far (monotonic). */
 L32_API unsigned long long l32_kernel_launch_count(void);
@@ -383,6 +384,45 @@ L32_API int l32_gqa_attention_forward_paged_cascade(const void* q, const void* p
                                                     size_t workspace_bytes, int batch, int heads, int kv_heads, int head_dim,
                                                     int num_pages, int max_pages_per_seq, int max_kv_len, int max_items, int dtype,
                                                     void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Speculative decoding on the paged KV cache (inference only; the paged layout, stale-row and trusted-table rules above hold).
+ *
+ * Verify attention: l32_gqa_attention_forward_paged for a step in which each sequence has up to q_len = t new tokens (its
+ * drafts), computed with one query tile per (sequence, kv head) that holds the group = heads / kv_heads query heads of each of
+ * the t tokens, so every key is read once per kv head.  Same arguments, layout and result (up to the order of the softmax
+ * sums) as l32_gqa_attention_forward_paged; query rows i >= new_lens[b] and rows with new_lens[b] == 0 yield exact zeros.
+ * Requires 2 <= group and group * q_len <= L32_VERIFY_TILE_ROWS (L32_ERR_BAD_SHAPE otherwise).  The split-KV plan is the
+ * packed decode's for max_kv_len; workspace: l32_gqa_attention_verify_workspace_bytes(...) bytes (optional: without it the
+ * call runs in one pass).  Enqueues one kernel, or two with the split.  Deterministic. */
+#define L32_VERIFY_TILE_ROWS 128
+L32_API size_t l32_gqa_attention_verify_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int max_kv_len);
+L32_API int l32_gqa_attention_forward_paged_verify(const void* q, const void* pool_k, const void* pool_v, const int32_t* block_table,
+                                                   const int32_t* past_lens, const int32_t* new_lens, void* ctx, void* workspace,
+                                                   size_t workspace_bytes, int batch, int q_len, int heads, int kv_heads, int head_dim,
+                                                   int num_pages, int max_pages_per_seq, int max_kv_len, int dtype, void* stream);
+/* Token history: token_pool int32 [num_pages, L32_KV_PAGE], named by the same block table as K / V: token i of sequence b is
+ * token_pool[block_table[b][i / 64]][i % 64].  A sequence's history holds exactly past_lens[b] tokens (its KV length); the
+ * sampled token whose K / V is not computed yet (the pending token) is kept by the caller.
+ *
+ * N-gram drafts, one row per sequence b < batch: S = history [0, past_lens[b]) followed by pending[b].  For n = n_max down to
+ * n_min (n <= |S| - 1), j is the largest index with S[j, j + n) == S[|S| - n, |S|) and j + n < |S|; the first n with such a j
+ * proposes S[j + n, j + n + k) cut at |S|.  Writes ids[b][0] = pending[b], ids[b][1 .. k] = the proposal, padded with its last
+ * token (with pending[b] when there is none), and draft_len[b] = the proposal's length (optional).  ids: int64 [batch, k + 1].
+ * 1 <= k, 1 <= n_min <= n_max <= L32_NGRAM_MAX.  Deterministic; one launch. */
+#define L32_NGRAM_MAX 16
+L32_API int l32_ngram_draft_paged(const int32_t* token_pool, const int32_t* block_table, const int32_t* past_lens,
+                                  const int64_t* pending, int64_t* ids, int32_t* draft_len, int batch, int k, int n_min, int n_max,
+                                  int num_pages, int max_pages_per_seq, void* stream);
+/* Acceptance.  ids int64 [batch, width] (the pending token, then the drafts), sampled int64 [batch * width], where row i of
+ * sequence b was sampled at position past_lens[b] + i + 1.  For each b with n = min(new_lens[b], width) > 0: a = the number
+ * of leading i < n - 1 with ids[b][i + 1] == sampled[b][i]; ids[b][0 .. a] are written to the history at positions
+ * past_lens[b] .. past_lens[b] + a, and out[b] (int64 [batch, width + 1]) = (a + 1, sampled[b][0 .. a], then -1).  Rows with
+ * new_lens[b] == 0 are not touched.  sampled == NULL keeps all n tokens of the row (a prompt written into the history) and
+ * writes only out[b][0] = n when out is given.  The pages written must be in the table and not shared.  One launch. */
+L32_API int l32_speculative_accept(const int64_t* ids, const int64_t* sampled, int32_t* token_pool, const int32_t* block_table,
+                                   const int32_t* past_lens, const int32_t* new_lens, int64_t* out, int batch, int width,
+                                   int num_pages, int max_pages_per_seq, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Next-token sampling: one token per row of 16-bit logits [batch, vocab] (row pitch = vocab), written to tokens_out [batch]

@@ -19,6 +19,7 @@ from .modules import (  # noqa: F401
     LinearFunction,
     LinearLoRAFunction,
     RMSNormFunction,
+    SpeculativeDecoder,
     SwiGLUFunction,
     TokenSampler,
     block_tail,
@@ -36,4 +37,5 @@ __all__ = [
     "LinearFunction", "RMSNormFunction", "SwiGLUFunction", "block_tail", "convert_feedforward_to_fused", "convert_instances",
     "patch_reference", "BlockTailFunction", "LinearLoRAFunction", "chain_block_norms", "LMHeadCEFunction", "lm_head_loss", "shift_labels", "GroupQueryAttention", "KVCache",
     "GQAAttentionFunction", "PagedKVCache", "TokenSampler", "last_token_logits",
+    "SpeculativeDecoder",
 ]

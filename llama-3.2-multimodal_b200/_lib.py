@@ -58,6 +58,10 @@ SIGNATURES = {
     "l32_gqa_attention_cascade_workspace_bytes": (c_size_t, [c_int] * 6),
     "l32_gqa_attention_forward_paged_cascade": (c_int, [c_void_p] * 11 + [c_size_t] + [c_int] * 9 + [c_void_p]),
     "l32_sample_tokens": (c_int, [c_void_p] * 8 + [c_int, c_int, c_int, c_void_p]),
+    "l32_gqa_attention_verify_workspace_bytes": (c_size_t, [c_int] * 6),
+    "l32_gqa_attention_forward_paged_verify": (c_int, [c_void_p] * 8 + [c_size_t] + [c_int] * 9 + [c_void_p]),
+    "l32_ngram_draft_paged": (c_int, [c_void_p] * 6 + [c_int] * 6 + [c_void_p]),
+    "l32_speculative_accept": (c_int, [c_void_p] * 7 + [c_int] * 4 + [c_void_p]),
     "l32_ffn_backward_workspace_bytes": (c_size_t, [c_int64, c_int]),
     "l32_ffn_backward": (c_int, [c_void_p] * 12 + [c_size_t, c_int64, c_int, c_int, c_int, c_void_p]),
     "l32_ffn_lora_forward": (c_int, [c_void_p] * 11 + [c_int64, c_int, c_int, c_int, c_int, c_void_p]),

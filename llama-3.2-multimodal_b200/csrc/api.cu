@@ -883,6 +883,64 @@ int l32_gqa_attention_forward_paged_cascade(const void* q, const void* pool_k, c
                                        max_kv_len, dtype, as_stream(stream));
 }
 
+// Speculative decoding: the verify step's attention, n-gram drafts and acceptance (include/l32_ffn.h).  The tables, lengths and
+// token values in device memory are trusted, as for the paged cache.
+static bool verify_shape_ok(int batch, int q_len, int heads, int kv_heads, int head_dim) {
+    return batch >= 0 && q_len >= 0 && heads > 0 && kv_heads > 0 && (heads % kv_heads) == 0 && heads / kv_heads >= 2 &&
+           static_cast<long long>(heads / kv_heads) * q_len <= L32_VERIFY_TILE_ROWS && (head_dim == 64 || head_dim == 128);
+}
+
+size_t l32_gqa_attention_verify_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int max_kv_len) {
+    if (!verify_shape_ok(batch, q_len, heads, kv_heads, head_dim) || max_kv_len < 0 || batch == 0 || q_len == 0) return 0;
+    return gqa_attention_verify_workspace_bytes(batch, q_len, heads, kv_heads, head_dim, max_kv_len);
+}
+
+int l32_gqa_attention_forward_paged_verify(const void* q, const void* pool_k, const void* pool_v, const int32_t* block_table,
+                                           const int32_t* past_lens, const int32_t* new_lens, void* ctx, void* workspace,
+                                           size_t workspace_bytes, int batch, int q_len, int heads, int kv_heads, int head_dim,
+                                           int num_pages, int max_pages_per_seq, int max_kv_len, int dtype, void* stream) {
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (!paged_shape_ok(batch, q_len, heads, kv_heads, head_dim, num_pages, max_pages_per_seq) ||
+        !verify_shape_ok(batch, q_len, heads, kv_heads, head_dim) || max_kv_len < 0 ||
+        static_cast<long long>(max_kv_len) > static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE)
+        return L32_ERR_BAD_SHAPE;
+    if (batch == 0 || q_len == 0) return L32_OK;
+    if (q == nullptr || pool_k == nullptr || pool_v == nullptr || block_table == nullptr || past_lens == nullptr || ctx == nullptr)
+        return L32_ERR_NULL;
+    if (!is_aligned16(q) || !is_aligned16(pool_k) || !is_aligned16(pool_v) || !is_aligned16(ctx)) return L32_ERR_BAD_ALIGN;
+    if (workspace != nullptr && !is_aligned16(workspace)) return L32_ERR_WORKSPACE;
+    return gqa_attention_paged_verify(q, pool_k, pool_v, block_table, past_lens, new_lens, ctx, workspace, workspace_bytes, batch,
+                                      q_len, heads, kv_heads, head_dim, num_pages, max_pages_per_seq, max_kv_len, dtype,
+                                      as_stream(stream));
+}
+
+int l32_ngram_draft_paged(const int32_t* token_pool, const int32_t* block_table, const int32_t* past_lens, const int64_t* pending,
+                          int64_t* ids, int32_t* draft_len, int batch, int k, int n_min, int n_max, int num_pages,
+                          int max_pages_per_seq, void* stream) {
+    if (batch < 0 || k < 1 || n_min < 1 || n_max < n_min || n_max > L32_NGRAM_MAX || num_pages <= 0 || max_pages_per_seq <= 0 ||
+        static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE > 0x7fffffffll)
+        return L32_ERR_BAD_SHAPE;
+    if (batch == 0) return L32_OK;
+    if (token_pool == nullptr || block_table == nullptr || past_lens == nullptr || pending == nullptr || ids == nullptr)
+        return L32_ERR_NULL;
+    return ngram_draft_paged(token_pool, block_table, past_lens, reinterpret_cast<const long long*>(pending),
+                             reinterpret_cast<long long*>(ids), draft_len, batch, k, n_min, n_max, max_pages_per_seq, as_stream(stream));
+}
+
+int l32_speculative_accept(const int64_t* ids, const int64_t* sampled, int32_t* token_pool, const int32_t* block_table,
+                           const int32_t* past_lens, const int32_t* new_lens, int64_t* out, int batch, int width, int num_pages,
+                           int max_pages_per_seq, void* stream) {
+    if (batch < 0 || width < 1 || num_pages <= 0 || max_pages_per_seq <= 0 ||
+        static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE > 0x7fffffffll)
+        return L32_ERR_BAD_SHAPE;
+    if (batch == 0) return L32_OK;
+    if (ids == nullptr || token_pool == nullptr || block_table == nullptr || past_lens == nullptr || new_lens == nullptr)
+        return L32_ERR_NULL;
+    return speculative_accept(reinterpret_cast<const long long*>(ids), reinterpret_cast<const long long*>(sampled), token_pool,
+                              block_table, past_lens, new_lens, reinterpret_cast<long long*>(out), batch, width, max_pages_per_seq,
+                              as_stream(stream));
+}
+
 // Next-token sampling (no reference kernel: the reference's decode loop samples with torch, Inference/Inference.py
 // select_next_token).  The per-row parameters live in device memory and are trusted, like the paged cache's tables.
 int l32_sample_tokens(const void* logits, const float* temperature, const int32_t* top_k, const float* top_p, const uint64_t* seed,

@@ -68,6 +68,12 @@ struct AttnParams {
     int casc_max_items;
     float* pfx_o;                  // [casc_max_items][page_kv_heads][kQTile][head_dim] fp32: prefix partials, per Q-tile row
     float2* pfx_ml;                // [casc_max_items][page_kv_heads][kQTile]
+    // Verify step (kVerify instances): packed shapes (batch = sequences * page_kv_heads, heads = 1, q_len = verify_group *
+    // verify_t rows); Q-tile row r is query head r % verify_group of new token r / verify_group, which sees the keys
+    // [0, past + r / verify_group].  map_q is {d, heads, sequences * verify_t} with box {64, verify_group, verify_t}.
+    // Split partials of row r go to slot (((seq * verify_t + token) * verify_group + g) * splits + split) * page_kv_heads + kv
+    // head: the plain combine with batch = sequences * verify_t, heads = verify_group, q_len = page_kv_heads then writes ctx.
+    int verify_t, verify_group;
 };
 static_assert(L32_KV_PAGE == kKvTile, "a KV-cache page is one key tile");
 
@@ -109,9 +115,11 @@ L32_DEVICE uint64_t add_f32x2(uint64_t a, uint64_t b) {
 // kLse: training forward, also stores the per-row log-sum-exp (a separate instantiation: the inference kernel is unchanged)
 // kPaged: K / V from a paged cache, lengths per sequence from device memory (AttnParams, "paged cache")
 // kCascade (with kPaged): a cascade decode CTA, prefix work item or own-key split (AttnParams, "cascade decode")
-template <int kD, typename T, bool kLse, bool kPaged, bool kCascade = false>
+// kVerify (with kPaged): one (sequence, kv head) of a speculative verify step (AttnParams, "verify step")
+template <int kD, typename T, bool kLse, bool kPaged, bool kCascade = false, bool kVerify = false>
 __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ AttnParams p) {
     static_assert(!kCascade || (kPaged && !kLse), "the cascade is a paged decode");
+    static_assert(!kVerify || (kPaged && !kLse && !kCascade), "the verify step is a paged packed step");
     // cascade: the CTA's work, read after the PDL wait (the plan may be written by earlier work of the stream).  A prefix CTA
     // past the plan's item count leaves before it allocates anything.  c_item < 0: an own-key CTA of sequence c_seq.
     int c_item = -1, c_seq = 0, c_split = 0, c_tile0 = 0, c_tiles = 0, c_kv_len = 0, c_member0 = 0, c_members = 1;
@@ -216,14 +224,17 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
             kvh_pool = b % p.page_kv_heads;
         }
         past_len = p.past_lens[seq];
-        const int n_new = p.new_lens != nullptr ? p.new_lens[seq] : (p.packed ? 1 : p.q_len);
+        const int n_new = p.new_lens != nullptr ? p.new_lens[seq] : (kVerify ? p.verify_t : (p.packed ? 1 : p.q_len));
         kv_len = past_len + n_new;
-        q_rows = p.packed ? (n_new > 0 ? p.q_len : 0) : min(n_new, p.q_len);
+        if constexpr (kVerify)
+            q_rows = min(n_new, p.verify_t) * p.verify_group;
+        else
+            q_rows = p.packed ? (n_new > 0 ? p.q_len : 0) : min(n_new, p.q_len);
     }
     // keys this query tile can see: [0, hi)
     const int q_last = min(q0 + kQTile, q_rows) - 1;
     int hi = kv_len;
-    if (p.causal) hi = min(hi, past_len + q_last + 1);
+    if (p.causal) hi = min(hi, past_len + (kVerify ? q_last / p.verify_group : q_last) + 1);
     if constexpr (kPaged) {
         if (q_last < q0) hi = 0;                                          // the whole query tile is padding
     }
@@ -298,7 +309,13 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
                 }
                 umma_commit<1>(&bar_s[s]);
             };
-            if constexpr (!kCascade) {                    // (cascade: the softmax warps gather Q)
+            if constexpr (kVerify) {                      // the verify rows: verify_t tokens x verify_group heads, one box
+                mbar_arrive_expect_tx(bar_q, p.q_len * kD * 2);
+#pragma unroll
+                for (int a = 0; a < kDAtoms; ++a)
+                    tma_load_3d(sq + a * (kQTile * 128), &p.map_q, bar_q, a * 64, kvh_pool * p.verify_group, seq * p.verify_t,
+                                kEvictNormal);
+            } else if constexpr (!kCascade) {             // (cascade: the softmax warps gather Q)
                 mbar_arrive_expect_tx(bar_q, kQBytes);
 #pragma unroll
                 for (int a = 0; a < kDAtoms; ++a)
@@ -374,7 +391,7 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
             }
         }
         const int qi = q0 + tid;                       // query index inside the sequence
-        const int qpos = past_len + qi;                // its absolute position
+        const int qpos = past_len + (kVerify ? qi / p.verify_group : qi);   // its absolute position
         const bool row_ok = qi < p.q_len;
         // Online softmax with a LAZY reference: the output accumulator stays in TMEM across the key tiles (P V accumulates
         // there) and is rescaled -- a TMEM read-modify-write of this thread's row -- only when the row maximum outgrows the
@@ -561,8 +578,15 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
             }
         } else if (p.splits > 1) {
             // split-KV: the unnormalised accumulator row and its (reference, sum) leave for the combine kernel
-            const size_t slot = ((static_cast<size_t>(b) * p.heads + head) * p.splits + split) * p.q_len + (row_ok ? qi : 0);
-            if (row_ok) p.part_ml[slot] = make_float2(ntiles > 0 ? m_ref : -INFINITY, ntiles > 0 ? l : 0.f);
+            size_t slot = ((static_cast<size_t>(b) * p.heads + head) * p.splits + split) * p.q_len + (row_ok ? qi : 0);
+            bool live = ntiles > 0;
+            if constexpr (kVerify) {                   // a padded token row (>= new_lens) leaves an empty partial: zeros
+                const int r = row_ok ? qi : 0;
+                slot = ((static_cast<size_t>(seq) * p.verify_t + r / p.verify_group) * p.verify_group + r % p.verify_group) * p.splits + split;
+                slot = slot * p.page_kv_heads + kvh_pool;
+                live = live && qi < q_rows;
+            }
+            if (row_ok) p.part_ml[slot] = make_float2(live ? m_ref : -INFINITY, live ? l : 0.f);
             float* dstf = p.part_o + slot * kD;
 #pragma unroll
             for (int c = 0; c < kD / 32; ++c) {
@@ -586,6 +610,11 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
             p.lse[(static_cast<size_t>(b) * p.heads + head) * p.q_len + qi] = inv > 0.f ? m_ref + log2f(l) : INFINITY;
         T* dst = static_cast<T*>(p.out) + (static_cast<size_t>(b) * p.q_len + (row_ok ? qi : 0)) * (static_cast<size_t>(p.heads) * kD) +
                  head * kD;
+        if constexpr (kVerify) {                       // ctx [sequences, verify_t, page_kv_heads * verify_group, d]
+            const int r = row_ok ? qi : 0;
+            dst = static_cast<T*>(p.out) + ((static_cast<size_t>(seq) * p.verify_t + r / p.verify_group) * p.page_kv_heads + kvh_pool) *
+                                               (static_cast<size_t>(p.verify_group) * kD) + (r % p.verify_group) * kD;
+        }
 #pragma unroll
         for (int c = 0; c < kD / 32; ++c) {
             uint32_t v[32];
@@ -781,9 +810,9 @@ __global__ void __launch_bounds__(128) rope_kv_append_kernel(T* q, const T* __re
     }
 }
 
-template <int kD, typename T, bool kLse, bool kPaged, bool kCascade = false>
+template <int kD, typename T, bool kLse, bool kPaged, bool kCascade = false, bool kVerify = false>
 int launch_attention(const AttnParams& p, cudaStream_t s) {
-    auto* kernel = gqa_attention_kernel<kD, T, kLse, kPaged, kCascade>;
+    auto* kernel = gqa_attention_kernel<kD, T, kLse, kPaged, kCascade, kVerify>;
     size_t smem = kQTile * kD * 2 + 4 * kKvTile * kD * 2 + 128;   // tiles + barriers
     if (const char* v = getenv("L32_ATT_ONE_CTA_PER_SM")) {   // experiments only: pad so that only one CTA fits per SM
         if (*v == '1') smem = 160 * 1024;
@@ -1105,6 +1134,61 @@ int gqa_attention_paged_cascade(const void* q, const void* pool_k, const void* p
         rc = head_dim == 128 ? launch_attention<128, __half, false, true, true>(p, s) : launch_attention<64, __half, false, true, true>(p, s);
     if (rc != L32_OK) return rc;
     return launch_combine<true>(p, head_dim, dtype, s);
+}
+
+// Verify step: one query tile per (sequence, kv head) holding the group query heads of each of the sequence's q_len new tokens,
+// split over the keys with the packed decode's plan for max_kv_len.  The partials' layout (AttnParams, "verify step") lets the
+// plain combine write ctx in its [batch, q_len, heads, d] layout.
+static int verify_splits(int batch, int heads, int kv_heads, int max_kv_len) {
+    return decode_splits(batch, 1, heads, kv_heads, max_kv_len);
+}
+
+size_t gqa_attention_verify_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int max_kv_len) {
+    const int splits = verify_splits(batch, heads, kv_heads, max_kv_len);
+    if (splits < 2) return 0;
+    return static_cast<size_t>(batch) * heads * q_len * splits * (static_cast<size_t>(head_dim) + 2) * sizeof(float) + 256;
+}
+
+int gqa_attention_paged_verify(const void* q, const void* pool_k, const void* pool_v, const int* block_table, const int* past_lens,
+                               const int* new_lens, void* out, void* workspace, size_t workspace_bytes, int batch, int q_len, int heads,
+                               int kv_heads, int head_dim, int num_pages, int max_pages_per_seq, int max_kv_len, int dtype,
+                               cudaStream_t s) {
+    const int group = heads / kv_heads;
+    AttnParams p;
+    int rc = attention_setup(p, q, out, batch * kv_heads, group * q_len, 1, 1, head_dim, 1, dtype);
+    if (rc != L32_OK) return rc;
+    rc = make_tensor_map_3d_box(&p.map_q, q, static_cast<uint64_t>(batch) * q_len, heads, head_dim, head_dim,
+                                static_cast<uint64_t>(heads) * head_dim, group, q_len, dtype);
+    if (rc != L32_OK) return rc;
+    p.block_table = block_table;
+    p.past_lens = past_lens;
+    p.new_lens = new_lens;
+    p.pages_per_seq = max_pages_per_seq;
+    p.page_kv_heads = kv_heads;
+    p.packed = 1;
+    p.verify_t = q_len;
+    p.verify_group = group;
+    const uint64_t planes = static_cast<uint64_t>(num_pages) * kv_heads, plane_elems = static_cast<uint64_t>(kKvTile) * head_dim;
+    rc = make_tensor_map_3d(&p.map_k, pool_k, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
+    if (rc != L32_OK) return rc;
+    rc = make_tensor_map_3d(&p.map_v, pool_v, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
+    if (rc != L32_OK) return rc;
+    const size_t need = gqa_attention_verify_workspace_bytes(batch, q_len, heads, kv_heads, head_dim, max_kv_len);
+    const int splits = (need > 0 && workspace != nullptr && workspace_bytes >= need) ? verify_splits(batch, heads, kv_heads, max_kv_len)
+                                                                                     : 1;
+    attention_split(p, splits, max_kv_len, head_dim, workspace);
+    if (dtype == L32_BF16)
+        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16, false, true, false, true>(p, s)
+                             : launch_attention<64, __nv_bfloat16, false, true, false, true>(p, s);
+    else
+        rc = head_dim == 128 ? launch_attention<128, __half, false, true, false, true>(p, s)
+                             : launch_attention<64, __half, false, true, false, true>(p, s);
+    if (rc != L32_OK || p.splits == 1) return rc;
+    AttnParams c = p;                                      // the combine's view of the partials: rows (token, group head)
+    c.batch = batch * q_len;
+    c.heads = group;
+    c.q_len = kv_heads;
+    return launch_combine<false>(c, head_dim, dtype, s);
 }
 
 // Training forward: keys [0, q_len) of the K / V buffers, no past, no split-KV; also writes the per-row log-sum-exp.

@@ -958,13 +958,18 @@ int make_tensor_map_2d_sw(CUtensorMap* map, const void* ptr, uint64_t rows, uint
 
 int make_tensor_map_3d(CUtensorMap* map, const void* ptr, uint64_t planes, uint64_t rows, uint64_t cols, uint64_t ld_elems,
                        uint64_t plane_elems, uint32_t box_rows, int dtype) {
+    return make_tensor_map_3d_box(map, ptr, planes, rows, cols, ld_elems, plane_elems, box_rows, 1, dtype);
+}
+
+int make_tensor_map_3d_box(CUtensorMap* map, const void* ptr, uint64_t planes, uint64_t rows, uint64_t cols, uint64_t ld_elems,
+                           uint64_t plane_elems, uint32_t box_rows, uint32_t box_planes, int dtype) {
     EncodeTiledFn fn = encode_tiled_fn();
     if (fn == nullptr) return L32_ERR_DRIVER;
     if (!is_aligned16(ptr) || (ld_elems % 8) != 0 || (plane_elems % 8) != 0) return L32_ERR_BAD_ALIGN;
-    if (box_rows == 0 || box_rows > 256 || planes == 0 || rows == 0) return L32_ERR_BAD_SHAPE;
+    if (box_rows == 0 || box_rows > 256 || box_planes == 0 || box_planes > 256 || planes == 0 || rows == 0) return L32_ERR_BAD_SHAPE;
     const cuuint64_t gdim[3] = {cols, rows, planes};
     const cuuint64_t gstride[2] = {ld_elems * 2, plane_elems * 2};
-    const cuuint32_t box[3] = {64, box_rows, 1};
+    const cuuint32_t box[3] = {64, box_rows, box_planes};
     const cuuint32_t estride[3] = {1, 1, 1};
     const CUtensorMapDataType dt = (dtype == L32_BF16) ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
     auto encode = [&] {

@@ -173,6 +173,12 @@ int gqa_attention_paged_cascade(const void* q, const void* pool_k, const void* p
                                 const int* new_lens, const int* items, const int* members, const int* seq_plan, int max_items,
                                 void* out, void* workspace, int batch, int heads, int kv_heads, int head_dim, int num_pages,
                                 int max_pages_per_seq, int max_kv_len, int dtype, cudaStream_t s);
+// speculative verify step: each sequence has up to q_len new tokens, group * q_len <= 128 rows in one query tile per kv head
+size_t gqa_attention_verify_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int max_kv_len);
+int gqa_attention_paged_verify(const void* q, const void* pool_k, const void* pool_v, const int* block_table, const int* past_lens,
+                               const int* new_lens, void* out, void* workspace, size_t workspace_bytes, int batch, int q_len, int heads,
+                               int kv_heads, int head_dim, int num_pages, int max_pages_per_seq, int max_kv_len, int dtype,
+                               cudaStream_t s);
 // RoPE angle of rotation pair i (of d / 2) at position `pos`: pos * base^(-2 i / d), cos / sin in fp32.  The forward rotation
 // (rope_kv_append_kernel) and the inverse rotation of the backward epilogues share it, so both use bit-identical angles.
 L32_DEVICE void rope_cos_sin(float pos, int i, int d, float log2_base, float& cs, float& sn) {
@@ -192,6 +198,12 @@ int sample_tokens(const void* logits, const float* temperature, const int* top_k
                   const unsigned long long* seed, const long long* position, long long* tokens_out, float* kept_min_logit,
                   int batch, int vocab, int dtype, cudaStream_t s);
 
+// ---- speculative.cu : token history of a paged cache, n-gram drafts and exact acceptance (contract: include/l32_ffn.h)
+int ngram_draft_paged(const int* token_pool, const int* block_table, const int* past_lens, const long long* pending, long long* ids,
+                      int* draft_len, int batch, int k, int n_min, int n_max, int max_pages_per_seq, cudaStream_t s);
+int speculative_accept(const long long* ids, const long long* sampled, int* token_pool, const int* block_table, const int* past_lens,
+                       const int* new_lens, long long* out, int batch, int width, int max_pages_per_seq, cudaStream_t s);
+
 // ---- tp.cu : tensor-parallel glue (cross-GPU flags, reduction of the partial slots)
 cudaError_t tp_signal(void* const* peer_flags, int world, int index, uint32_t value, uint32_t* zero8, cudaStream_t s);
 cudaError_t tp_peer_copy(void* dst, const void* src, size_t bytes, int ctas, int warps, int unroll, int seg_bytes,
@@ -209,5 +221,9 @@ int make_tensor_map_2d_sw(CUtensorMap* map, const void* ptr, uint64_t rows, uint
 // 128-byte swizzled.  A box row at or beyond `rows` of its plane is zero-filled, never read from the next plane.
 int make_tensor_map_3d(CUtensorMap* map, const void* ptr, uint64_t planes, uint64_t rows, uint64_t cols, uint64_t ld_elems,
                        uint64_t plane_elems, uint32_t box_rows, int dtype);
+// The same with a box of box_planes planes: {64 cols, box_rows, box_planes}, landing as box_planes * box_rows consecutive
+// 128-byte rows in shared memory.
+int make_tensor_map_3d_box(CUtensorMap* map, const void* ptr, uint64_t planes, uint64_t rows, uint64_t cols, uint64_t ld_elems,
+                           uint64_t plane_elems, uint32_t box_rows, uint32_t box_planes, int dtype);
 
 }  // namespace l32

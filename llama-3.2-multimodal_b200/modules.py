@@ -27,7 +27,7 @@ __all__ = [
     "RMSNormFunction", "LLAMARMSNorm", "SwiGLUFunction", "FusedSwiGLU", "LinearFunction", "Linear_LORA", "FFNFunction", "FFNLoRAFunction",
     "FusedFeedforward", "FusedFeedForward", "convert_feedforward_to_fused", "patch_reference", "convert_instances", "block_tail",
     "BlockTailFunction", "LinearLoRAFunction", "chain_block_norms", "LMHeadCEFunction", "lm_head_loss", "shift_labels", "GroupQueryAttention", "KVCache",
-    "GQAAttentionFunction", "PagedKVCache", "TokenSampler", "last_token_logits",
+    "GQAAttentionFunction", "PagedKVCache", "TokenSampler", "last_token_logits", "SpeculativeDecoder",
 ]
 
 
@@ -625,6 +625,8 @@ class PagedKVCache:
     so a CUDA graph captured over a forward stays valid while `set_batch` changes their contents between replays.
 
     One step:  set_batch(ids, new_lens) -> every layer's forward -> advance().
+    A speculative verify step:  set_batch(ids, new_lens, verify=True) -> every layer's forward -> commit(counts), which keeps
+    only each row's first counts[r] tokens.  `token_pool()` adds the token history next to K / V (SpeculativeDecoder).
     Rows of the device buffers past len(ids) hold zero lengths: a forward over more rows than the batch (a graph captured
     at a larger batch) leaves those rows' output zero and writes no page.
     Pages handed out again keep what the previous sequence wrote: finite values, which is all the kernels require of rows
@@ -642,6 +644,9 @@ class PagedKVCache:
         self._next_id = 0
         self.batch_ids: list = []
         self.batch_new_lens: list = []
+        self.verify = False                                      # the last set_batch marked a verify step
+        self._held: list = []                                    # pages each batch row held before set_batch reserved more
+        self._tokens = None                                      # token history [num_pages, 64] int32 (token_pool)
         self._pool_k: list = []                                  # per layer
         self._pool_v: list = []
         if device is None and torch.cuda.is_available():
@@ -714,7 +719,7 @@ class PagedKVCache:
             self._refs[p] += 1
         if tail:
             old, new = self._pages[sid][full], self._take()
-            for pool in self._pool_k + self._pool_v:
+            for pool in self._pool_k + self._pool_v + ([self._tokens] if self._tokens is not None else []):
                 if pool is not None:
                     pool[new].copy_(pool[old])
             pages = pages + [new]
@@ -736,11 +741,12 @@ class PagedKVCache:
     def pages(self, sid: int) -> list:
         return list(self._pages[sid])
 
-    def set_batch(self, ids, new_lens) -> None:
+    def set_batch(self, ids, new_lens, verify=False) -> None:
         """Choose the sequences (rows, in this order) of the next forward calls and the number of tokens each appends, reserve
         the pages those tokens need and upload the block table and lengths (stream-ordered copies from pinned host memory on
         the current stream).  Raises before anything is reserved or enqueued when the pages run out or a sequence would
-        outgrow max_pages_per_seq."""
+        outgrow max_pages_per_seq.  verify=True marks a speculative verify step: the attention takes the verify kernel where
+        its geometry fits (ops.verify_fits), and the step ends with commit() instead of advance()."""
         ids, new_lens = [int(i) for i in ids], [int(n) for n in new_lens]
         if len(ids) != len(new_lens) or not 0 < len(ids) <= self.max_batch:
             raise ValueError(f"set_batch: {len(ids)} ids / {len(new_lens)} lengths for a cache of max_batch {self.max_batch}")
@@ -758,9 +764,11 @@ class PagedKVCache:
         if sum(want) > len(self._free):
             raise RuntimeError(f"PagedKVCache out of pages: this step needs {sum(want)} more, {len(self._free)} free of "
                                f"{self.num_pages}")
+        self._held = [len(self._pages[sid]) for sid in ids]
         for sid, w in zip(ids, want):
             self._pages[sid].extend(self._take() for _ in range(w))
         self.batch_ids, self.batch_new_lens = ids, new_lens
+        self.verify = bool(verify)
         host = torch.zeros(self.max_batch * (self.max_pages_per_seq + 2), dtype=torch.int32,
                            pin_memory=self._dev is not None)
         t = self.max_batch * self.max_pages_per_seq
@@ -784,7 +792,7 @@ class PagedKVCache:
         empty one replaces it when nothing is shared: a CUDA graph captured over a cascade-form step stays correct when the
         groups change or vanish.  A cache that never shares uploads nothing."""
         self.cascade = False
-        if self.cascade_geometry is None or any(n != 1 for n in new_lens):
+        if self.cascade_geometry is None or any(n != 1 for n in new_lens) or self.verify:
             return
         group, kv_heads = self.cascade_geometry
         self.cascade_max_items = cascade_items_capacity(self._sms, kv_heads)
@@ -807,6 +815,34 @@ class PagedKVCache:
         """After the step's last layer: every sequence of the batch now holds its new tokens."""
         for sid, n in zip(self.batch_ids, self.batch_new_lens):
             self._len[sid] += n
+
+    def commit(self, counts) -> None:
+        """After a verify step's last layer: row r keeps its first counts[r] <= new_lens[r] tokens (K / V written past them
+        stays as stale rows).  Pages this step reserved that now hold no kept token go back to the free list.  The batch is
+        dropped: call set_batch before the next forward."""
+        counts = [int(c) for c in counts]
+        if len(counts) != len(self.batch_ids):
+            raise ValueError(f"commit: {len(counts)} counts for a batch of {len(self.batch_ids)} sequences")
+        if any(not 0 <= c <= n for c, n in zip(counts, self.batch_new_lens)):
+            raise ValueError(f"commit: counts {counts} must lie in [0, new_lens] = {self.batch_new_lens}")
+        for sid, c, held in zip(self.batch_ids, counts, self._held):
+            self._len[sid] += c
+            keep = max(held, -(-self._len[sid] // self.page_size))
+            pages = self._pages[sid]
+            spare, self._pages[sid] = pages[keep:], pages[:keep]
+            for p in spare:
+                self._refs[p] = 0
+            self._free.extend(reversed(spare))
+        self.batch_ids, self.batch_new_lens, self._held = [], [], []
+
+    def token_pool(self):
+        """The token history, int32 [num_pages, 64] named by the same block table as K / V (created zeroed on first use).  A
+        sequence's history holds exactly its length in tokens; fork copies a partial last page of it with K / V."""
+        if self._tokens is None:
+            if self.device is None:
+                raise RuntimeError("PagedKVCache.token_pool: the cache has no device")
+            self._tokens = torch.zeros(self.num_pages, self.page_size, dtype=torch.int32, device=self.device)
+        return self._tokens
 
     # -- per-layer pools
     def pools(self, layer_idx, kv_heads, head_dim, dtype, device):
@@ -989,7 +1025,10 @@ class GroupQueryAttention(nn.Module):
         geometry = (self.group_size, self.num_kv_groups)
         if cache.cascade_geometry is None:
             cache.cascade_geometry = geometry                 # the steps planned from now on fit this attention
-        if t == 1 and cache.cascade and cache.cascade_geometry == geometry:
+        if cache.verify and ops.verify_fits(self.group_size, t):
+            ctx = ops.gqa_attention_forward_paged_verify(q, pk, pv, cache.block_table, cache.past_lens, cache.new_lens,
+                                                         max_kv_len=cache.max_kv_len)
+        elif t == 1 and cache.cascade and cache.cascade_geometry == geometry:
             ctx = ops.gqa_attention_forward_paged_cascade(q, pk, pv, cache.block_table, cache.past_lens, cache.new_lens,
                                                           cache.plan_items, cache.plan_members, cache.plan_seq,
                                                           cache.cascade_max_items, max_kv_len=cache.max_kv_len)
@@ -1192,6 +1231,181 @@ class TokenSampler:
             position = position.to(torch.int64)
         return ops.sample_tokens(logits, self.temperature, self.top_k, self.top_p, self.seed, position.contiguous(),
                                  out=self.tokens, want_kept_min=want_kept_min)
+
+
+class SpeculativeDecoder:
+    """Speculative decoding on a PagedKVCache with n-gram (prompt lookup) drafts and exact acceptance.
+
+    model(ids [b, t] int64, cache) must return the final-normed hidden states [b, t, H] of a paged forward; lm_head maps them
+    to logits.  One step per call of `step(ids)`: (1) k drafts per sequence from its own history (or the caller's `drafts`),
+    (2) one forward over the pending token + drafts as a verify step, (3) the head on all b * (k + 1) rows, (4) the sampler
+    at positions past + 1 + i, (5) the accept kernel, which keeps the leading drafts equal to the token sampled for the row
+    before them, then (6) one device-to-host copy and cache.commit.  A draw depends only on (logits row, parameters, seed,
+    position), so the emitted tokens are the ones plain decoding samples with the same seeds, up to rounding differences
+    between the kernel paths.  With graph=True, stages 1-5 run as a CUDA graph captured once at max_batch.
+
+    Stop tokens are the caller's business: cut the returned list and free the sequence (free_sequence)."""
+
+    def __init__(self, model, lm_head, cache, max_batch, k, ngram=(1, 3)):
+        if not isinstance(cache, PagedKVCache):
+            raise ValueError("SpeculativeDecoder: needs a PagedKVCache")
+        if isinstance(k, bool) or not isinstance(k, int) or k < 1:
+            raise ValueError(f"SpeculativeDecoder: k must be an int >= 1, got {k!r}")
+        groups = {m.group_size for m in model.modules() if isinstance(m, GroupQueryAttention)} if isinstance(model, nn.Module) else set()
+        for g in groups:
+            if g * (k + 1) > ops.VERIFY_TILE_ROWS:
+                raise ValueError(f"SpeculativeDecoder: group {g} * (k + 1) = {g * (k + 1)} rows exceed one verify tile of "
+                                 f"{ops.VERIFY_TILE_ROWS}")
+        n_min, n_max = (int(v) for v in ngram)
+        if not 1 <= n_min <= n_max <= ops.NGRAM_MAX:
+            raise ValueError(f"SpeculativeDecoder: ngram must satisfy 1 <= n_min <= n_max <= {ops.NGRAM_MAX}, got {ngram!r}")
+        if not 0 < int(max_batch) <= cache.max_batch:
+            raise ValueError(f"SpeculativeDecoder: max_batch {max_batch} outside 1..{cache.max_batch} (the cache's max_batch)")
+        if cache.device is None:
+            raise ValueError("SpeculativeDecoder: the PagedKVCache has no CUDA device")
+        self.model, self.lm_head, self.cache = model, lm_head, cache
+        self.max_batch, self.k, self.ngram = int(max_batch), k, (n_min, n_max)
+        w, dev = k + 1, cache.device
+        self.pool = cache.token_pool()
+        self.ids = torch.zeros(self.max_batch, w, dtype=torch.int64, device=dev)       # pending token, then the drafts
+        self.pending = torch.zeros(self.max_batch, dtype=torch.int64, device=dev)
+        self.drafts = torch.zeros(self.max_batch, k, dtype=torch.int64, device=dev)    # the caller's drafts (graph input)
+        self.draft_len = torch.zeros(self.max_batch, dtype=torch.int32, device=dev)    # n-gram proposal lengths (statistics)
+        self.out = torch.zeros(self.max_batch, w + 1, dtype=torch.int64, device=dev)   # (accepted, emitted..., -1...)
+        self._offs = torch.arange(1, w + 1, dtype=torch.int64, device=dev)
+        self.sampler = TokenSampler(self.max_batch * w, dev)                            # row r * w + i: sequence r, token i
+        self._first = TokenSampler(self.max_batch, dev)                                 # prefill: one row per sequence
+        self._pending: dict = {}                                                        # sequence id -> its pending token
+        self._graphs: dict = {}
+        self.logits = None                                                              # the last step's logits [rows * w, V]
+
+    # -- parameters and sequences
+    def set_params(self, temperature, top_k=0, top_p=1.0, seed=0) -> None:
+        """Per-sequence sampling parameters (TokenSampler.set_params), one entry per row of the next prefill / step calls."""
+        self._first.set_params(temperature, top_k, top_p, seed)
+        rep = lambda v: [x for x in v for _ in range(self.k + 1)] if isinstance(v, (list, tuple)) else v
+        self.sampler.set_params(rep(temperature), rep(top_k), rep(top_p), rep(seed))
+
+    def fork(self, sid: int) -> int:
+        """A sibling of `sid` (PagedKVCache.fork) that continues from the same pending token."""
+        if sid not in self._pending:
+            raise ValueError(f"SpeculativeDecoder.fork: {sid} has no pending token (prefill it first)")
+        child = self.cache.fork(sid)
+        self._pending[child] = self._pending[sid]
+        return child
+
+    def free_sequence(self, sid: int) -> None:
+        self._pending.pop(sid, None)
+        self.cache.free_sequence(sid)
+
+    def _logits(self, h):
+        w = self.lm_head.weight
+        if (ops.supported(h) and w.is_cuda and w.dtype == h.dtype and getattr(self.lm_head, "bias", None) is None and
+                w.shape[0] % 8 == 0 and h.shape[-1] % 8 == 0):
+            return ops.linear_forward(h.contiguous(), w)
+        return self.lm_head(h)
+
+    def prefill(self, prompts) -> dict:
+        """New sequences for `prompts` (lists of token ids): one forward over the prompts, the first token sampled from each
+        last row, the prompts written into the token history.  Returns {sid: [first token]}."""
+        prompts = [[int(t) for t in p] for p in prompts]
+        b = len(prompts)
+        if not 0 < b <= self.max_batch or any(len(p) == 0 for p in prompts):
+            raise ValueError(f"SpeculativeDecoder.prefill: 1..{self.max_batch} non-empty prompts expected")
+        cache, n = self.cache, max(len(p) for p in prompts)
+        ids = [cache.add_sequence() for _ in prompts]
+        try:
+            cache.set_batch(ids, [len(p) for p in prompts])
+        except Exception:
+            for sid in ids:
+                cache.free_sequence(sid)
+            raise
+        x = torch.zeros(b, n, dtype=torch.int64)
+        for r, p in enumerate(prompts):
+            x[r, :len(p)] = torch.tensor(p, dtype=torch.int64)
+        x = x.to(cache.device)
+        with torch.no_grad():
+            logits = last_token_logits(self.lm_head, self.model(x, cache), cache.new_lens)
+            tok = self._first(logits, cache.past_lens[:b] + cache.new_lens[:b])
+            ops.speculative_accept(x, None, self.pool, cache.block_table, cache.past_lens, cache.new_lens, batch=b)
+        tok = tok.cpu().tolist()
+        cache.advance()
+        self._pending.update(zip(ids, tok))
+        return {sid: [t] for sid, t in zip(ids, tok)}
+
+    # -- one speculative step
+    def _stages(self, rows, drafts):
+        cache, w = self.cache, self.k + 1
+        if drafts:
+            self.ids[:rows, 0] = self.pending[:rows]
+            self.ids[:rows, 1:] = self.drafts[:rows]
+        else:
+            ops.ngram_draft(self.pool, cache.block_table, cache.past_lens, self.pending, self.ids, self.draft_len,
+                            n_min=self.ngram[0], n_max=self.ngram[1], batch=rows)
+        h = self.model(self.ids[:rows], cache)
+        logits = self.logits = self._logits(h.reshape(rows * w, h.shape[-1]))   # (kept for inspection: row r * w + i)
+        pos = (cache.past_lens[:rows].to(torch.int64)[:, None] + self._offs[None]).reshape(-1)
+        s = self.sampler(logits, pos)
+        ops.speculative_accept(self.ids[:rows], s, self.pool, cache.block_table, cache.past_lens, cache.new_lens, self.out,
+                               batch=rows)
+
+    def _capture(self, drafts):
+        """Stages 1-5 at max_batch, captured over a batch of empty placeholder sequences (zero new tokens: the warm-up run and
+        the capture write nothing)."""
+        cache = self.cache
+        slots = [cache.add_sequence() for _ in range(self.max_batch)]
+        try:
+            cache.set_batch(slots, [0] * self.max_batch, verify=True)
+            with torch.no_grad():
+                self._stages(self.max_batch, drafts)
+                torch.cuda.synchronize(cache.device)
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g):
+                    self._stages(self.max_batch, drafts)
+        finally:
+            for sid in slots:
+                cache.free_sequence(sid)
+        return g
+
+    def step(self, ids, drafts=None, graph=False) -> dict:
+        """One verify step for sequences `ids` (prefilled, live): returns {sid: the 1 .. k + 1 tokens emitted}.  drafts: an
+        int64 tensor [len(ids), k] to verify instead of the n-gram drafts.  Validated before anything is enqueued."""
+        ids = [int(i) for i in ids]
+        b, w, cache = len(ids), self.k + 1, self.cache
+        if not 0 < b <= self.max_batch or len(set(ids)) != b:
+            raise ValueError(f"SpeculativeDecoder.step: 1..{self.max_batch} distinct sequences expected, got {ids}")
+        for sid in ids:
+            if sid not in self._pending:
+                raise ValueError(f"SpeculativeDecoder.step: sequence {sid} is not live here (prefill it first)")
+            if cache.length(sid) + w > cache.max_kv_len:
+                raise ValueError(f"SpeculativeDecoder.step: sequence {sid} holds {cache.length(sid)} tokens, no room for "
+                                 f"{w} more (max {cache.max_kv_len})")
+        if drafts is not None:
+            if not isinstance(drafts, torch.Tensor) or drafts.dtype != torch.int64 or tuple(drafts.shape) != (b, self.k):
+                raise ValueError(f"SpeculativeDecoder.step: drafts must be an int64 tensor [{b}, {self.k}], got "
+                                 f"{getattr(drafts, 'dtype', type(drafts))} {tuple(getattr(drafts, 'shape', ()))}")
+        key = drafts is not None
+        if graph and key not in self._graphs:
+            self._graphs[key] = self._capture(key)
+        host = torch.tensor([self._pending[sid] for sid in ids], dtype=torch.int64).pin_memory()
+        self.pending[:b].copy_(host, non_blocking=True)
+        if drafts is not None:
+            self.drafts[:b].copy_(drafts, non_blocking=True)
+        cache.set_batch(ids, [w] * b, verify=True)
+        if graph:
+            self._graphs[key].replay()
+        else:
+            with torch.no_grad():
+                self._stages(b, key)
+        out = self.out[:b].cpu()                             # the step's one read-back (synchronises)
+        counts = out[:, 0].tolist()
+        cache.commit(counts)
+        emitted = {}
+        for r, sid in enumerate(ids):
+            toks = out[r, 1:1 + counts[r]].tolist()
+            emitted[sid] = toks
+            self._pending[sid] = toks[-1]
+        return emitted
 
 
 def _mllama_forward(self, input_ids=None, pixel_values=None, attention_mask=None, position_ids=None, image_mask=None,

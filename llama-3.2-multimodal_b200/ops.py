@@ -572,6 +572,101 @@ def gqa_attention_forward_paged_cascade(q, pool_k, pool_v, block_table, past_len
     return ctx
 
 
+# --------------------------------------------------------------------------------------------- speculative decoding
+VERIFY_TILE_ROWS = 128   # L32_VERIFY_TILE_ROWS: group * q_len of a verify step fits one query tile
+NGRAM_MAX = 16           # L32_NGRAM_MAX
+
+
+def verify_fits(group: int, t: int) -> bool:
+    """True when a step of t new tokens per sequence with `group` query heads per kv head takes the verify kernel."""
+    return group >= 2 and 1 <= t and group * t <= VERIFY_TILE_ROWS
+
+
+def gqa_attention_forward_paged_verify(q, pool_k, pool_v, block_table, past_lens, new_lens=None, *, max_kv_len=None):
+    """gqa_attention_forward_paged for a speculative verify step (t = q_len new tokens per sequence, group * t <= 128): the
+    same result up to the order of the softmax sums, computed with one query tile per (sequence, kv head) holding the group
+    query heads of all t tokens, so the keys are read once per kv head (contract: include/l32_ffn.h)."""
+    _check_cuda(q, pool_k, pool_v, block_table, past_lens, new_lens)
+    b, t, heads, kvh, d, num_pages, max_pages = _paged_args(q, pool_k, pool_v, block_table, past_lens, new_lens,
+                                                            "gqa_attention_forward_paged_verify")
+    if heads % kvh != 0 or not verify_fits(heads // kvh, t):
+        raise L32Error(f"gqa_attention_forward_paged_verify: needs group >= 2 and group * q_len <= {VERIFY_TILE_ROWS}, got "
+                       f"{heads} heads / {kvh} kv heads, q_len {t}")
+    max_kv_len = max_pages * KV_PAGE if max_kv_len is None else int(max_kv_len)
+    ctx = torch.empty_like(q)
+    L = lib()
+    ws_bytes = L.l32_gqa_attention_verify_workspace_bytes(b, t, heads, kvh, d, max_kv_len)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=q.device) if ws_bytes else None
+    with torch.cuda.device(q.device):
+        check(L.l32_gqa_attention_forward_paged_verify(_ptr(q), _ptr(pool_k), _ptr(pool_v), _ptr(block_table), _ptr(past_lens),
+                                                       _ptr(new_lens), _ptr(ctx), _ptr(ws), ws_bytes, b, t, heads, kvh, d, num_pages,
+                                                       max_pages, max_kv_len, _dtype_code(q), _stream(q)),
+              "l32_gqa_attention_forward_paged_verify")
+    return ctx
+
+
+def _token_args(token_pool, block_table, what):
+    if token_pool.dtype != torch.int32 or token_pool.dim() != 2 or token_pool.shape[1] != KV_PAGE or not token_pool.is_contiguous():
+        raise L32Error(f"{what}: token_pool must be contiguous int32 [num_pages, {KV_PAGE}], got {tuple(token_pool.shape)} "
+                       f"{token_pool.dtype}")
+    if block_table.dtype != torch.int32 or block_table.dim() != 2 or not block_table.is_contiguous():
+        raise L32Error(f"{what}: block_table must be contiguous int32 [batch, max_pages]")
+    return token_pool.shape[0], block_table.shape[1]
+
+
+def _int_vec(ten, dt, n, what, name):
+    if ten is not None and (ten.dtype != dt or not ten.is_contiguous() or ten.numel() < n):
+        raise L32Error(f"{what}: {name} must be contiguous {dt} with >= {n} entries")
+
+
+def ngram_draft(token_pool, block_table, past_lens, pending, ids, draft_len=None, *, n_min=1, n_max=3, batch=None):
+    """Prompt-lookup drafts (l32_ngram_draft_paged) into ids int64 [>= batch, k + 1]: ids[b, 0] = pending[b], ids[b, 1:] =
+    what followed the latest earlier occurrence of the last n tokens of the row's history + pending token, for the largest
+    n in [n_min, n_max] that occurs (padded with the proposal's last token).  draft_len int32 [>= batch]: optional."""
+    _check_cuda(token_pool, block_table, past_lens, pending, ids, draft_len)
+    what = "ngram_draft"
+    num_pages, max_pages = _token_args(token_pool, block_table, what)
+    if ids.dtype != torch.int64 or ids.dim() != 2 or ids.shape[1] < 2 or not ids.is_contiguous():
+        raise L32Error(f"{what}: ids must be contiguous int64 [batch, k + 1] with k >= 1, got {tuple(ids.shape)} {ids.dtype}")
+    b = ids.shape[0] if batch is None else int(batch)
+    if not 0 <= b <= ids.shape[0] or block_table.shape[0] < b:
+        raise L32Error(f"{what}: batch {b} does not fit ids {tuple(ids.shape)} / block_table {tuple(block_table.shape)}")
+    _int_vec(past_lens, torch.int32, b, what, "past_lens")
+    _int_vec(pending, torch.int64, b, what, "pending")
+    _int_vec(draft_len, torch.int32, b, what, "draft_len")
+    if not 1 <= int(n_min) <= int(n_max) <= NGRAM_MAX:
+        raise L32Error(f"{what}: n-gram range must satisfy 1 <= n_min <= n_max <= {NGRAM_MAX}, got ({n_min}, {n_max})")
+    with torch.cuda.device(ids.device):
+        check(lib().l32_ngram_draft_paged(_ptr(token_pool), _ptr(block_table), _ptr(past_lens), _ptr(pending), _ptr(ids),
+                                          _ptr(draft_len), b, ids.shape[1] - 1, int(n_min), int(n_max), num_pages, max_pages,
+                                          _stream(ids)),
+              "l32_ngram_draft_paged")
+
+
+def speculative_accept(ids, sampled, token_pool, block_table, past_lens, new_lens, out=None, *, batch=None):
+    """Exact acceptance (l32_speculative_accept): per row b, a = the leading drafts ids[b, i + 1] equal to sampled[b, i];
+    ids[b, 0 .. a] go to the token history at positions past_lens[b] .. past_lens[b] + a and out[b] = (a + 1, the a + 1
+    emitted tokens sampled[b, 0 .. a], then -1).  sampled None: keeps all new_lens[b] tokens (a prompt).  ids int64 [batch,
+    width]; sampled int64 [>= batch * width]; out int64 [>= batch, width + 1].  Rows with new_lens 0 are not touched."""
+    _check_cuda(ids, sampled, token_pool, block_table, past_lens, new_lens, out)
+    what = "speculative_accept"
+    num_pages, max_pages = _token_args(token_pool, block_table, what)
+    if ids.dtype != torch.int64 or ids.dim() != 2 or ids.shape[1] < 1 or not ids.is_contiguous():
+        raise L32Error(f"{what}: ids must be contiguous int64 [batch, width], got {tuple(ids.shape)} {ids.dtype}")
+    b = ids.shape[0] if batch is None else int(batch)
+    width = ids.shape[1]
+    if not 0 <= b <= ids.shape[0] or block_table.shape[0] < b:
+        raise L32Error(f"{what}: batch {b} does not fit ids {tuple(ids.shape)} / block_table {tuple(block_table.shape)}")
+    _int_vec(past_lens, torch.int32, b, what, "past_lens")
+    _int_vec(new_lens, torch.int32, b, what, "new_lens")
+    _int_vec(sampled, torch.int64, b * width, what, "sampled")
+    _int_vec(out, torch.int64, b * (width + 1), what, "out")
+    with torch.cuda.device(ids.device):
+        check(lib().l32_speculative_accept(_ptr(ids), _ptr(sampled), _ptr(token_pool), _ptr(block_table), _ptr(past_lens),
+                                           _ptr(new_lens), _ptr(out), b, width, num_pages, max_pages, _stream(ids)),
+              "l32_speculative_accept")
+
+
 # --------------------------------------------------------------------------------------------- next-token sampling
 SAMPLE_MAX_VOCAB = 262144   # L32_SAMPLE_MAX_VOCAB
 
