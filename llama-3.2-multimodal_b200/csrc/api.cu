@@ -745,6 +745,11 @@ int l32_rope_kv_append(void* q, const void* k_new, const void* v_new, const int6
                           kv_heads, head_dim, max_len, past_len, rope_base, dtype, as_stream(stream));
 }
 
+// Heads of every attention entry point: whole KV groups of 64- or 128-wide heads.
+static bool attention_heads_ok(int heads, int kv_heads, int head_dim) {
+    return heads > 0 && kv_heads > 0 && (heads % kv_heads) == 0 && (head_dim == 64 || head_dim == 128);
+}
+
 size_t l32_gqa_attention_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int kv_len) {
     if (batch <= 0 || q_len <= 0 || heads <= 0 || kv_heads <= 0 || (heads % kv_heads) != 0 || kv_len <= 0) return 0;
     return gqa_attention_workspace_bytes(batch, q_len, heads, kv_heads, head_dim, kv_len);
@@ -754,8 +759,8 @@ int l32_gqa_attention_forward(const void* q, const void* cache_k, const void* ca
                               void* workspace, size_t workspace_bytes, int batch, int q_len, int heads, int kv_heads, int head_dim,
                               int max_len, int kv_len, int past_len, int causal, int dtype, void* stream) {
     if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
-    if (batch < 0 || q_len < 0 || heads <= 0 || kv_heads <= 0 || (heads % kv_heads) != 0 || (head_dim != 64 && head_dim != 128) ||
-        max_len <= 0 || kv_len < 0 || kv_len > max_len || past_len < 0)
+    if (batch < 0 || q_len < 0 || !attention_heads_ok(heads, kv_heads, head_dim) || max_len <= 0 || kv_len < 0 || kv_len > max_len ||
+        past_len < 0)
         return L32_ERR_BAD_SHAPE;
     if (batch == 0 || q_len == 0) return L32_OK;
     if (q == nullptr || cache_k == nullptr || cache_v == nullptr || ctx == nullptr) return L32_ERR_NULL;
@@ -771,8 +776,7 @@ int l32_gqa_attention_forward_train(const void* q_rot, const void* cache_k, cons
                                     float* lse, int batch, int q_len, int heads, int kv_heads, int head_dim, int max_len, int causal,
                                     int dtype, void* stream) {
     if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
-    if (batch < 0 || q_len < 0 || heads <= 0 || kv_heads <= 0 || (heads % kv_heads) != 0 || (head_dim != 64 && head_dim != 128) ||
-        max_len < q_len || max_len <= 0)
+    if (batch < 0 || q_len < 0 || !attention_heads_ok(heads, kv_heads, head_dim) || max_len < q_len || max_len <= 0)
         return L32_ERR_BAD_SHAPE;
     if (batch == 0 || q_len == 0) return L32_OK;
     if (q_rot == nullptr || cache_k == nullptr || cache_v == nullptr || ctx == nullptr || lse == nullptr) return L32_ERR_NULL;
@@ -791,8 +795,8 @@ int l32_gqa_attention_backward(const void* d_ctx, const void* q_rot, const void*
                                void* workspace, size_t workspace_bytes, int batch, int q_len, int heads, int kv_heads, int head_dim,
                                int max_len, int causal, float rope_base, int dtype, void* stream) {
     if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
-    if (batch < 0 || q_len < 0 || heads <= 0 || kv_heads <= 0 || (heads % kv_heads) != 0 || (head_dim != 64 && head_dim != 128) ||
-        max_len < q_len || max_len <= 0 || !(rope_base > 1.0f))
+    if (batch < 0 || q_len < 0 || !attention_heads_ok(heads, kv_heads, head_dim) || max_len < q_len || max_len <= 0 ||
+        !(rope_base > 1.0f))
         return L32_ERR_BAD_SHAPE;
     if (batch == 0 || q_len == 0) return L32_OK;
     if (d_ctx == nullptr || q_rot == nullptr || cache_k == nullptr || cache_v == nullptr || ctx == nullptr || lse == nullptr ||
@@ -811,9 +815,32 @@ int l32_gqa_attention_backward(const void* d_ctx, const void* q_rot, const void*
 // Paged KV cache (no reference counterpart: the reference's cache is one torch.cat'ed tensor per layer).  Only the host-side
 // arguments can be checked here; the table and length values in device memory are trusted (include/l32_ffn.h).
 static bool paged_shape_ok(int batch, int q_len, int heads, int kv_heads, int head_dim, int num_pages, int max_pages_per_seq) {
-    return batch >= 0 && q_len >= 0 && heads > 0 && kv_heads > 0 && (heads % kv_heads) == 0 && (head_dim == 64 || head_dim == 128) &&
-           num_pages > 0 && max_pages_per_seq > 0 && static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE <= 0x7fffffffll &&
+    return batch >= 0 && q_len >= 0 && attention_heads_ok(heads, kv_heads, head_dim) && num_pages > 0 && max_pages_per_seq > 0 &&
+           static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE <= 0x7fffffffll &&
            static_cast<long long>(num_pages) * kv_heads <= 0x7fffffffll;
+}
+
+// The checks the three paged attention forwards share, in this order: dtype; shape, with the form's own shape rule (form_ok),
+// and the max_kv_len bound; the empty batch; null pointers, with the form's own pointers (ptrs_ok); alignment; then the
+// alignment of a workspace that is given.  Returns the code of the first that fails; *run is set when all pass and the batch
+// is not empty.
+static int paged_forward_check(int dtype, bool form_ok, bool ptrs_ok, const void* q, const void* pool_k, const void* pool_v,
+                               const int32_t* block_table, const int32_t* past_lens, const void* ctx, const void* workspace,
+                               int batch, int q_len, int heads, int kv_heads, int head_dim, int num_pages, int max_pages_per_seq,
+                               int max_kv_len, bool* run) {
+    *run = false;
+    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
+    if (!paged_shape_ok(batch, q_len, heads, kv_heads, head_dim, num_pages, max_pages_per_seq) || !form_ok || max_kv_len < 0 ||
+        static_cast<long long>(max_kv_len) > static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE)
+        return L32_ERR_BAD_SHAPE;
+    if (batch == 0 || q_len == 0) return L32_OK;
+    if (q == nullptr || pool_k == nullptr || pool_v == nullptr || block_table == nullptr || past_lens == nullptr || ctx == nullptr ||
+        !ptrs_ok)
+        return L32_ERR_NULL;
+    if (!is_aligned16(q) || !is_aligned16(pool_k) || !is_aligned16(pool_v) || !is_aligned16(ctx)) return L32_ERR_BAD_ALIGN;
+    if (workspace != nullptr && !is_aligned16(workspace)) return L32_ERR_WORKSPACE;
+    *run = true;
+    return L32_OK;
 }
 
 int l32_rope_kv_append_paged(void* q, const void* k_new, const void* v_new, const int64_t* position_ids, void* pool_k, void* pool_v,
@@ -836,23 +863,17 @@ int l32_gqa_attention_forward_paged(const void* q, const void* pool_k, const voi
                                     const int32_t* past_lens, const int32_t* new_lens, void* ctx, void* workspace, size_t workspace_bytes,
                                     int batch, int q_len, int heads, int kv_heads, int head_dim, int num_pages, int max_pages_per_seq,
                                     int max_kv_len, int dtype, void* stream) {
-    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
-    if (!paged_shape_ok(batch, q_len, heads, kv_heads, head_dim, num_pages, max_pages_per_seq) || max_kv_len < 0 ||
-        static_cast<long long>(max_kv_len) > static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE)
-        return L32_ERR_BAD_SHAPE;
-    if (batch == 0 || q_len == 0) return L32_OK;
-    if (q == nullptr || pool_k == nullptr || pool_v == nullptr || block_table == nullptr || past_lens == nullptr || ctx == nullptr)
-        return L32_ERR_NULL;
-    if (!is_aligned16(q) || !is_aligned16(pool_k) || !is_aligned16(pool_v) || !is_aligned16(ctx)) return L32_ERR_BAD_ALIGN;
-    if (workspace != nullptr && !is_aligned16(workspace)) return L32_ERR_WORKSPACE;
+    bool run;
+    const int rc = paged_forward_check(dtype, true, true, q, pool_k, pool_v, block_table, past_lens, ctx, workspace, batch, q_len,
+                                       heads, kv_heads, head_dim, num_pages, max_pages_per_seq, max_kv_len, &run);
+    if (!run) return rc;
     return gqa_attention_paged(q, pool_k, pool_v, block_table, past_lens, new_lens, ctx, workspace, workspace_bytes, batch, q_len, heads,
                                kv_heads, head_dim, num_pages, max_pages_per_seq, max_kv_len, dtype, as_stream(stream));
 }
 
 static bool cascade_shape_ok(int batch, int heads, int kv_heads, int head_dim, int max_kv_len, int max_items) {
-    return batch >= 0 && heads > 0 && kv_heads > 0 && (heads % kv_heads) == 0 && heads / kv_heads >= 2 &&
-           heads / kv_heads <= L32_CASCADE_TILE_ROWS && (head_dim == 64 || head_dim == 128) && max_kv_len >= 0 && max_items > 0 &&
-           max_items <= L32_CASCADE_MAX_ITEMS;
+    return batch >= 0 && attention_heads_ok(heads, kv_heads, head_dim) && heads / kv_heads >= 2 &&
+           heads / kv_heads <= L32_CASCADE_TILE_ROWS && max_kv_len >= 0 && max_items > 0 && max_items <= L32_CASCADE_MAX_ITEMS;
 }
 
 size_t l32_gqa_attention_cascade_workspace_bytes(int batch, int heads, int kv_heads, int head_dim, int max_kv_len, int max_items) {
@@ -865,18 +886,13 @@ int l32_gqa_attention_forward_paged_cascade(const void* q, const void* pool_k, c
                                             const int32_t* plan_members, const int32_t* plan_seq, void* ctx, void* workspace,
                                             size_t workspace_bytes, int batch, int heads, int kv_heads, int head_dim, int num_pages,
                                             int max_pages_per_seq, int max_kv_len, int max_items, int dtype, void* stream) {
-    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
-    if (!paged_shape_ok(batch, 1, heads, kv_heads, head_dim, num_pages, max_pages_per_seq) ||
-        !cascade_shape_ok(batch, heads, kv_heads, head_dim, max_kv_len, max_items) ||
-        static_cast<long long>(max_kv_len) > static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE)
-        return L32_ERR_BAD_SHAPE;
-    if (batch == 0) return L32_OK;
-    if (q == nullptr || pool_k == nullptr || pool_v == nullptr || block_table == nullptr || past_lens == nullptr || ctx == nullptr ||
-        plan_items == nullptr || plan_members == nullptr || plan_seq == nullptr || workspace == nullptr)
-        return L32_ERR_NULL;
-    if (!is_aligned16(q) || !is_aligned16(pool_k) || !is_aligned16(pool_v) || !is_aligned16(ctx)) return L32_ERR_BAD_ALIGN;
-    if (!is_aligned16(workspace) ||
-        workspace_bytes < gqa_attention_cascade_workspace_bytes(batch, heads, kv_heads, head_dim, max_kv_len, max_items))
+    const bool plan_ok = plan_items != nullptr && plan_members != nullptr && plan_seq != nullptr && workspace != nullptr;
+    bool run;
+    const int rc = paged_forward_check(dtype, cascade_shape_ok(batch, heads, kv_heads, head_dim, max_kv_len, max_items), plan_ok, q,
+                                       pool_k, pool_v, block_table, past_lens, ctx, workspace, batch, 1, heads, kv_heads, head_dim,
+                                       num_pages, max_pages_per_seq, max_kv_len, &run);
+    if (!run) return rc;
+    if (workspace_bytes < gqa_attention_cascade_workspace_bytes(batch, heads, kv_heads, head_dim, max_kv_len, max_items))
         return L32_ERR_WORKSPACE;
     return gqa_attention_paged_cascade(q, pool_k, pool_v, block_table, past_lens, new_lens, plan_items, plan_members, plan_seq,
                                        max_items, ctx, workspace, batch, heads, kv_heads, head_dim, num_pages, max_pages_per_seq,
@@ -886,8 +902,8 @@ int l32_gqa_attention_forward_paged_cascade(const void* q, const void* pool_k, c
 // Speculative decoding: the verify step's attention, n-gram drafts and acceptance (include/l32_ffn.h).  The tables, lengths and
 // token values in device memory are trusted, as for the paged cache.
 static bool verify_shape_ok(int batch, int q_len, int heads, int kv_heads, int head_dim) {
-    return batch >= 0 && q_len >= 0 && heads > 0 && kv_heads > 0 && (heads % kv_heads) == 0 && heads / kv_heads >= 2 &&
-           static_cast<long long>(heads / kv_heads) * q_len <= L32_VERIFY_TILE_ROWS && (head_dim == 64 || head_dim == 128);
+    return batch >= 0 && q_len >= 0 && attention_heads_ok(heads, kv_heads, head_dim) && heads / kv_heads >= 2 &&
+           static_cast<long long>(heads / kv_heads) * q_len <= L32_VERIFY_TILE_ROWS;
 }
 
 size_t l32_gqa_attention_verify_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int max_kv_len) {
@@ -899,16 +915,11 @@ int l32_gqa_attention_forward_paged_verify(const void* q, const void* pool_k, co
                                            const int32_t* past_lens, const int32_t* new_lens, void* ctx, void* workspace,
                                            size_t workspace_bytes, int batch, int q_len, int heads, int kv_heads, int head_dim,
                                            int num_pages, int max_pages_per_seq, int max_kv_len, int dtype, void* stream) {
-    if (!dtype_ok(dtype)) return L32_ERR_BAD_DTYPE;
-    if (!paged_shape_ok(batch, q_len, heads, kv_heads, head_dim, num_pages, max_pages_per_seq) ||
-        !verify_shape_ok(batch, q_len, heads, kv_heads, head_dim) || max_kv_len < 0 ||
-        static_cast<long long>(max_kv_len) > static_cast<long long>(max_pages_per_seq) * L32_KV_PAGE)
-        return L32_ERR_BAD_SHAPE;
-    if (batch == 0 || q_len == 0) return L32_OK;
-    if (q == nullptr || pool_k == nullptr || pool_v == nullptr || block_table == nullptr || past_lens == nullptr || ctx == nullptr)
-        return L32_ERR_NULL;
-    if (!is_aligned16(q) || !is_aligned16(pool_k) || !is_aligned16(pool_v) || !is_aligned16(ctx)) return L32_ERR_BAD_ALIGN;
-    if (workspace != nullptr && !is_aligned16(workspace)) return L32_ERR_WORKSPACE;
+    bool run;
+    const int rc = paged_forward_check(dtype, verify_shape_ok(batch, q_len, heads, kv_heads, head_dim), true, q, pool_k, pool_v,
+                                       block_table, past_lens, ctx, workspace, batch, q_len, heads, kv_heads, head_dim, num_pages,
+                                       max_pages_per_seq, max_kv_len, &run);
+    if (!run) return rc;
     return gqa_attention_paged_verify(q, pool_k, pool_v, block_table, past_lens, new_lens, ctx, workspace, workspace_bytes, batch,
                                       q_len, heads, kv_heads, head_dim, num_pages, max_pages_per_seq, max_kv_len, dtype,
                                       as_stream(stream));

@@ -18,9 +18,8 @@
 // triu(-inf, 1), model.py:314-317), key padding (model.py:318, as a per-key keep byte) and the cache length.
 #include "l32_internal.cuh"
 
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
+#include <type_traits>
 
 namespace l32 {
 namespace {
@@ -77,16 +76,10 @@ struct AttnParams {
 };
 static_assert(L32_KV_PAGE == kKvTile, "a KV-cache page is one key tile");
 
-// L32_ATT_NOEXP / L32_ATT_NOPV / L32_ATT_NOLD: experiment builds only (wrong results) -- what the kernel costs without the
-// exponentials, without the P V MMAs, without the S reads from TMEM.
 L32_DEVICE float fast_exp2(float x) {
-#ifdef L32_ATT_NOEXP
-    return x * 0.001f;
-#else
     float y;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));   // not volatile: a pure function the scheduler may interleave freely
     return y;
-#endif
 }
 
 // Packed fp32 pairs (Blackwell FFMA2 / FADD2): half the FMA-pipe instructions of the exponent arguments and the row sums.
@@ -112,14 +105,20 @@ L32_DEVICE uint64_t add_f32x2(uint64_t a, uint64_t b) {
     return d;
 }
 
-// kLse: training forward, also stores the per-row log-sum-exp (a separate instantiation: the inference kernel is unchanged)
-// kPaged: K / V from a paged cache, lengths per sequence from device memory (AttnParams, "paged cache")
-// kCascade (with kPaged): a cascade decode CTA, prefix work item or own-key split (AttnParams, "cascade decode")
-// kVerify (with kPaged): one (sequence, kv head) of a speculative verify step (AttnParams, "verify step")
-template <int kD, typename T, bool kLse, bool kPaged, bool kCascade = false, bool kVerify = false>
+// The forms of the attention forward, one kernel instance each:
+//   Contig   K / V from the contiguous cache [batch, kv_heads, max_len, d] (prefill, decode and its split-KV form)
+//   Train    Contig that also stores the per-row log-sum-exp (a separate instance: the inference kernel is unchanged)
+//   Paged    K / V from a paged cache, lengths per sequence from device memory (AttnParams, "paged cache")
+//   Cascade  a paged cascade decode CTA, prefix work item or own-key split (AttnParams, "cascade decode")
+//   Verify   one (sequence, kv head) of a paged speculative verify step (AttnParams, "verify step")
+enum class AttnForm { Contig, Train, Paged, Cascade, Verify };
+
+template <int kD, typename T, AttnForm kForm>
 __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ AttnParams p) {
-    static_assert(!kCascade || (kPaged && !kLse), "the cascade is a paged decode");
-    static_assert(!kVerify || (kPaged && !kLse && !kCascade), "the verify step is a paged packed step");
+    constexpr bool kLse = kForm == AttnForm::Train;
+    constexpr bool kCascade = kForm == AttnForm::Cascade;
+    constexpr bool kVerify = kForm == AttnForm::Verify;
+    constexpr bool kPaged = kForm == AttnForm::Paged || kCascade || kVerify;
     // cascade: the CTA's work, read after the PDL wait (the plan may be written by earlier work of the stream).  A prefix CTA
     // past the plan's item count leaves before it allocates anything.  c_item < 0: an own-key CTA of sequence c_seq.
     int c_item = -1, c_seq = 0, c_split = 0, c_tile0 = 0, c_tiles = 0, c_kv_len = 0, c_member0 = 0, c_members = 1;
@@ -346,13 +345,11 @@ __global__ void __maxnreg__(160) gqa_attention_kernel(const __grid_constant__ At
                 tc_fence_after();
                 const uint32_t v_addr = smem_u32(sv + s * kKBytes);
                 const uint32_t p_tmem = tmem_base + s * kKvTile;
-#ifndef L32_ATT_NOPV
 #pragma unroll
                 for (int kk = 0; kk < kKvTile / kUmmaKAtt; ++kk)
                     umma_f16_ts(tmem_o, p_tmem + kk * (kUmmaKAtt / 2),
                                 make_smem_desc_sw128(v_addr + kk * (kUmmaKAtt * 128), kKvTile * 128, 1024), p.idesc_o,
                                 (t > 0 || kk > 0) ? 1u : 0u);
-#endif
                 umma_commit<1>(bar_o);
                 if (t + 2 < ntiles) issue_s(t + 2);       // (K of tile t + 2 was requested a tile ago)
                 if (t + 3 < ntiles) {                     // K stage (t + 1) & 1 is free once S of tile t + 1 is complete
@@ -810,30 +807,19 @@ __global__ void __launch_bounds__(128) rope_kv_append_kernel(T* q, const T* __re
     }
 }
 
-template <int kD, typename T, bool kLse, bool kPaged, bool kCascade = false, bool kVerify = false>
+template <int kD, typename T, AttnForm kForm>
 int launch_attention(const AttnParams& p, cudaStream_t s) {
-    auto* kernel = gqa_attention_kernel<kD, T, kLse, kPaged, kCascade, kVerify>;
-    size_t smem = kQTile * kD * 2 + 4 * kKvTile * kD * 2 + 128;   // tiles + barriers
-    if (const char* v = getenv("L32_ATT_ONE_CTA_PER_SM")) {   // experiments only: pad so that only one CTA fits per SM
-        if (*v == '1') smem = 160 * 1024;
-    }
+    auto* kernel = gqa_attention_kernel<kD, T, kForm>;
+    const size_t smem = kQTile * kD * 2 + 4 * kKvTile * kD * 2 + 128;   // tiles + barriers
     static bool configured_dev[kMaxDevices] = {};
     bool& configured = configured_dev[current_device_slot()];
     if (!configured) {
         cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         if (e != cudaSuccess) return static_cast<int>(e);
         configured = true;
-        if (getenv("L32_ATT_DEBUG") != nullptr) {
-            int nb = 0;
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, kAttThreads, smem);
-            cudaFuncAttributes fa;
-            cudaFuncGetAttributes(&fa, kernel);
-            fprintf(stderr, "[l32] gqa_attention_kernel<%d>: %d CTAs / SM, %d registers, %zu B local, %zu B dynamic smem\n", kD, nb,
-                    fa.numRegs, fa.localSizeBytes, smem);
-        }
     }
     cudaLaunchConfig_t cfg = {};
-    if (kCascade)
+    if (kForm == AttnForm::Cascade)
         cfg.gridDim = dim3(static_cast<unsigned>(p.casc_max_items + (p.batch / p.page_kv_heads) * p.splits),
                            static_cast<unsigned>(p.page_kv_heads));
     else if (p.splits > 1)
@@ -854,6 +840,21 @@ int launch_attention(const AttnParams& p, cudaStream_t s) {
     return static_cast<int>(e);
 }
 
+// f(T*) with a null pointer of the element type of `dtype`, bf16 or fp16: the kernel instance of each type.
+template <typename F>
+auto with_dtype(int dtype, F&& f) {
+    return dtype == L32_BF16 ? f(static_cast<__nv_bfloat16*>(nullptr)) : f(static_cast<__half*>(nullptr));
+}
+
+// The instance of form kForm for the call's dtype and head_dim (64 or 128).
+template <AttnForm kForm>
+int launch_form(const AttnParams& p, int head_dim, int dtype, cudaStream_t s) {
+    return with_dtype(dtype, [&](auto* tag) {
+        using T = std::remove_pointer_t<decltype(tag)>;
+        return head_dim == 128 ? launch_attention<128, T, kForm>(p, s) : launch_attention<64, T, kForm>(p, s);
+    });
+}
+
 // Fields every attention launch shares: shapes, scale, instruction descriptors and the Q map.
 int attention_setup(AttnParams& p, const void* q, void* out, int batch, int q_len, int heads, int kv_heads, int head_dim,
                     int causal, int dtype) {
@@ -867,16 +868,89 @@ int attention_setup(AttnParams& p, const void* q, void* out, int batch, int q_le
                               static_cast<uint64_t>(heads) * head_dim, kQTile, 64, dtype);
 }
 
+// Fields the paged forms share: the block table, the lengths and the page-pool maps.  K / V: one plane per (page, kv head) of
+// kKvTile rows.  Rows of a page past its sequence's length are read as they are and get P = 0: the pool's contract keeps
+// them finite (include/l32_ffn.h).
+int paged_setup(AttnParams& p, const void* pool_k, const void* pool_v, const int* block_table, const int* past_lens,
+                const int* new_lens, int num_pages, int max_pages_per_seq, int kv_heads, int head_dim, int dtype, bool packed) {
+    p.block_table = block_table;
+    p.past_lens = past_lens;
+    p.new_lens = new_lens;
+    p.pages_per_seq = max_pages_per_seq;
+    p.page_kv_heads = kv_heads;
+    p.packed = packed ? 1 : 0;
+    const uint64_t planes = static_cast<uint64_t>(num_pages) * kv_heads, plane_elems = static_cast<uint64_t>(kKvTile) * head_dim;
+    const int rc = make_tensor_map_3d(&p.map_k, pool_k, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
+    if (rc != L32_OK) return rc;
+    return make_tensor_map_3d(&p.map_v, pool_v, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
+}
+
+// Split-KV plan of a packed step without key padding (a decode, or a verify step of several tokens): the number of key splits
+// (1 = none).  The `group` query heads of a KV group are the rows of ONE query tile (a split CTA covers rows [0, kQTile)
+// only, so a larger group is not split).
+int decode_splits(int batch, int heads, int kv_heads, int kv_len) {
+    const int group = heads / kv_heads;
+    if (batch <= 0 || group < 2 || group > kQTile) return 1;
+    const int tiles = (kv_len + kKvTile - 1) / kKvTile;
+    const int ctas = batch * kv_heads;                    // one CTA per (sequence, KV group)
+    int splits = (2 * num_sms() + ctas - 1) / ctas;       // aim at two CTAs per SM
+    if (splits > tiles / 2) splits = tiles / 2;           // at least two key tiles (128 keys) per split
+    return splits < 2 ? 1 : splits;
+}
+
+// Split-KV partials of `rows` query rows over `splits` splits in a workspace: part_o, rows * splits rows of head_dim fp32, at
+// offset 0; part_ml, rows * splits float2, from `ml` (256-aligned) to `ml_end`.  `bytes` holds both.
+struct SplitLayout {
+    size_t ml, ml_end, bytes;
+};
+SplitLayout split_layout(size_t rows, int splits, int head_dim) {
+    const size_t n = rows * splits;
+    const size_t ml = (n * head_dim * sizeof(float) + 255) & ~static_cast<size_t>(255);
+    return {ml, ml + n * sizeof(float2), n * (static_cast<size_t>(head_dim) + 2) * sizeof(float) + 256};
+}
+
+// Workspace of a packed step with t query tokens per sequence (0: the step does not split).
+size_t packed_workspace_bytes(int batch, int t, int heads, int kv_heads, int head_dim, int kv_len) {
+    const int splits = decode_splits(batch, heads, kv_heads, kv_len);
+    return splits < 2 ? 0 : split_layout(static_cast<size_t>(batch) * heads * t, splits, head_dim).bytes;
+}
+
+// The splits a packed step takes: its plan, or one pass when the caller's workspace cannot hold the partials.
+int packed_splits(int batch, int t, int heads, int kv_heads, int head_dim, int kv_len, const void* workspace,
+                  size_t workspace_bytes) {
+    const size_t need = packed_workspace_bytes(batch, t, heads, kv_heads, head_dim, kv_len);
+    return need > 0 && workspace != nullptr && workspace_bytes >= need ? decode_splits(batch, heads, kv_heads, kv_len) : 1;
+}
+
 // Split-KV: `splits` CTAs per (batch, head) over the key tiles of kv_len keys; the partials go to the workspace.
 void attention_split(AttnParams& p, int splits, int kv_len, int head_dim, void* workspace) {
     p.splits = splits > 1 ? splits : 1;
     if (p.splits > 1) {
         const int tiles = (kv_len + kKvTile - 1) / kKvTile;
         p.tiles_per_split = (tiles + p.splits - 1) / p.splits;
-        const size_t rows = static_cast<size_t>(p.batch) * p.heads * p.splits * p.q_len;
+        const size_t rows = static_cast<size_t>(p.batch) * p.heads * p.q_len;
         p.part_o = static_cast<float*>(workspace);
-        p.part_ml = reinterpret_cast<float2*>(static_cast<uint8_t*>(workspace) + ((rows * head_dim * sizeof(float) + 255) & ~static_cast<size_t>(255)));
+        p.part_ml = reinterpret_cast<float2*>(static_cast<uint8_t*>(workspace) + split_layout(rows, p.splits, head_dim).ml);
     }
+}
+
+// Cascade decode workspace: the own-key split partials (the split-KV layout for `splits` splits, at least one), then the prefix
+// partials, one row per (item, kv head, Q-tile row).  Offsets of part_ml, pfx_o, pfx_ml and the total, each 256-aligned.
+struct CascadeLayout {
+    int splits;
+    size_t ml, pfx_o, pfx_ml, bytes;
+};
+CascadeLayout cascade_layout(int batch, int heads, int kv_heads, int head_dim, int max_kv_len, int max_items) {
+    auto up = [](size_t x) { return (x + 255) & ~static_cast<size_t>(255); };
+    CascadeLayout c;
+    c.splits = decode_splits(batch, heads, kv_heads, max_kv_len);
+    const SplitLayout own = split_layout(static_cast<size_t>(batch) * heads, c.splits, head_dim);
+    const size_t pfx_rows = static_cast<size_t>(max_items) * kv_heads * kQTile;
+    c.ml = own.ml;
+    c.pfx_o = up(own.ml_end);
+    c.pfx_ml = c.pfx_o + up(pfx_rows * head_dim * sizeof(float));
+    c.bytes = c.pfx_ml + up(pfx_rows * sizeof(float2));
+    return c;
 }
 
 // The merge of the split-KV (kCascade: and prefix) partials.
@@ -896,28 +970,45 @@ int launch_combine(const AttnParams& p, int head_dim, int dtype, cudaStream_t s)
     const float2* pml = p.part_ml;
     const float* pfo = p.pfx_o;
     const float2* pfml = p.pfx_ml;
-    cudaError_t e;
-    if (dtype == L32_BF16)
-        e = cudaLaunchKernelEx(&cfg, attention_combine_kernel<__nv_bfloat16, kCascade>, po, pml, static_cast<__nv_bfloat16*>(p.out),
-                               p.batch, p.heads, p.q_len, p.splits, head_dim, p.casc_seq, pfo, pfml, p.page_kv_heads);
-    else
-        e = cudaLaunchKernelEx(&cfg, attention_combine_kernel<__half, kCascade>, po, pml, static_cast<__half*>(p.out), p.batch,
-                               p.heads, p.q_len, p.splits, head_dim, p.casc_seq, pfo, pfml, p.page_kv_heads);
+    const cudaError_t e = with_dtype(dtype, [&](auto* tag) {
+        using T = std::remove_pointer_t<decltype(tag)>;
+        return cudaLaunchKernelEx(&cfg, attention_combine_kernel<T, kCascade>, po, pml, static_cast<T*>(p.out), p.batch, p.heads,
+                                  p.q_len, p.splits, head_dim, p.casc_seq, pfo, pfml, p.page_kv_heads);
+    });
     if (e == cudaSuccess) count_launch();
     return static_cast<int>(e);
 }
 
-// The inference kernel, then (split-KV) the merge of its partials.
-template <bool kPaged>
+// The kernel, then (split-KV) the merge of its partials.
+template <AttnForm kForm>
 int attention_run(const AttnParams& p, int head_dim, int dtype, cudaStream_t s) {
-    int rc;
-    if (dtype == L32_BF16) {
-        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16, false, kPaged>(p, s) : launch_attention<64, __nv_bfloat16, false, kPaged>(p, s);
-    } else {
-        rc = head_dim == 128 ? launch_attention<128, __half, false, kPaged>(p, s) : launch_attention<64, __half, false, kPaged>(p, s);
-    }
+    const int rc = launch_form<kForm>(p, head_dim, dtype, s);
     if (rc != L32_OK || p.splits == 1) return rc;
     return launch_combine<false>(p, head_dim, dtype, s);
+}
+
+// Contiguous cache, form Contig or Train (lse: the per-row log-sum-exp).  K / V: one plane per (batch, kv head), cut at
+// kv_len.  Masked keys get P = 0, but 0 * NaN and 0 * Inf are NaN in the P V product: the rows of the last tile beyond kv_len
+// (stale cache capacity, or the next head's keys) must not reach shared memory with whatever they hold, so TMA fills them
+// with zeros.
+template <AttnForm kForm>
+int contiguous_forward(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, float* lse, void* out,
+                       int batch, int q_len, int heads, int kv_heads, int head_dim, int max_len, int kv_len, int past_len,
+                       int causal, int splits, void* workspace, int dtype, cudaStream_t s) {
+    AttnParams p;
+    int rc = attention_setup(p, q, out, batch, q_len, heads, kv_heads, head_dim, causal, dtype);
+    if (rc != L32_OK) return rc;
+    p.lse = lse;
+    p.keep = keep;
+    p.max_len = max_len; p.kv_len = kv_len; p.past_len = past_len;
+    const uint64_t planes = static_cast<uint64_t>(batch) * kv_heads, plane_elems = static_cast<uint64_t>(max_len) * head_dim;
+    const uint64_t kv_rows = static_cast<uint64_t>(kv_len > 0 ? kv_len : 1);   // kv_len 0: no tile is loaded
+    rc = make_tensor_map_3d(&p.map_k, cache_k, planes, kv_rows, head_dim, head_dim, plane_elems, kKvTile, dtype);
+    if (rc != L32_OK) return rc;
+    rc = make_tensor_map_3d(&p.map_v, cache_v, planes, kv_rows, head_dim, head_dim, plane_elems, kKvTile, dtype);
+    if (rc != L32_OK) return rc;
+    attention_split(p, splits, kv_len, head_dim, workspace);
+    return attention_run<kForm>(p, head_dim, dtype, s);
 }
 
 // Paged-cache arguments of rope_kv_append_kernel (null: the contiguous cache).
@@ -959,28 +1050,18 @@ int rope_append(void* q, const void* k_new, const void* v_new, const long long* 
     const float log2_base = log2f(rope_base);
     const RopePages none = {nullptr, nullptr, nullptr, 0};
     const RopePages& pg = pages != nullptr ? *pages : none;
-    cudaError_t e;
-    if (dtype == L32_BF16)
-        e = pages != nullptr ? launch_rope<__nv_bfloat16, true>(cfg, q, k_new, v_new, position_ids, cache_k, cache_v, q_len, heads,
-                                                                kv_heads, head_dim, max_len, past_len, log2_base, pg)
-                             : launch_rope<__nv_bfloat16, false>(cfg, q, k_new, v_new, position_ids, cache_k, cache_v, q_len, heads,
-                                                                 kv_heads, head_dim, max_len, past_len, log2_base, pg);
-    else
-        e = pages != nullptr ? launch_rope<__half, true>(cfg, q, k_new, v_new, position_ids, cache_k, cache_v, q_len, heads, kv_heads,
-                                                         head_dim, max_len, past_len, log2_base, pg)
-                             : launch_rope<__half, false>(cfg, q, k_new, v_new, position_ids, cache_k, cache_v, q_len, heads, kv_heads,
-                                                          head_dim, max_len, past_len, log2_base, pg);
+    const cudaError_t e = with_dtype(dtype, [&](auto* tag) {
+        using T = std::remove_pointer_t<decltype(tag)>;
+        return pages != nullptr ? launch_rope<T, true>(cfg, q, k_new, v_new, position_ids, cache_k, cache_v, q_len, heads, kv_heads,
+                                                       head_dim, max_len, past_len, log2_base, pg)
+                                : launch_rope<T, false>(cfg, q, k_new, v_new, position_ids, cache_k, cache_v, q_len, heads,
+                                                        kv_heads, head_dim, max_len, past_len, log2_base, pg);
+    });
     if (e == cudaSuccess) count_launch();
     return static_cast<int>(e);
 }
 
 }  // namespace
-
-int gqa_attention_packed(const void* q, const void* cache_k, const void* cache_v, void* out, int batch2, int group, int head_dim,
-                         int max_len, int kv_len, int splits, void* workspace, int dtype, cudaStream_t s);
-int gqa_attention_launch(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, int batch, int q_len,
-                         int heads, int kv_heads, int head_dim, int max_len, int kv_len, int past_len, int causal, int splits,
-                         void* workspace, int dtype, cudaStream_t s, float* lse = nullptr);
 
 int rope_kv_append(void* q, const void* k_new, const void* v_new, const long long* position_ids, void* cache_k, void* cache_v,
                    int batch, int q_len, int heads, int kv_heads, int head_dim, int max_len, int past_len, float rope_base,
@@ -997,23 +1078,9 @@ int rope_kv_append_paged(void* q, const void* k_new, const void* v_new, const lo
                        dtype, s, &pages);
 }
 
-// Split-KV plan of a decode call without key padding: the number of key splits (1 = none).  Only the packed decode path
-// splits: one query per sequence, the `group` query heads of a KV group as the rows of ONE query tile (a split CTA covers
-// rows [0, kQTile) only, so a larger group is not split).
-static int decode_splits(int batch, int q_len, int heads, int kv_heads, int kv_len) {
-    const int group = heads / kv_heads;
-    if (q_len != 1 || batch <= 0 || group < 2 || group > kQTile) return 1;
-    const int tiles = (kv_len + kKvTile - 1) / kKvTile;
-    const int ctas = batch * kv_heads;                    // decode packs the heads of a KV group into one CTA
-    int splits = (2 * num_sms() + ctas - 1) / ctas;       // aim at two CTAs per SM
-    if (splits > tiles / 2) splits = tiles / 2;           // at least two key tiles (128 keys) per split
-    return splits < 2 ? 1 : splits;
-}
-
+// Only a decode without key padding splits (the packed decode).
 size_t gqa_attention_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int kv_len) {
-    const int splits = decode_splits(batch, q_len, heads, kv_heads, kv_len);
-    if (splits < 2) return 0;
-    return static_cast<size_t>(batch) * heads * splits * (static_cast<size_t>(head_dim) + 2) * sizeof(float) + 256;
+    return q_len == 1 ? packed_workspace_bytes(batch, 1, heads, kv_heads, head_dim, kv_len) : 0;
 }
 
 int gqa_attention(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, int batch, int q_len,
@@ -1025,15 +1092,21 @@ int gqa_attention(const void* q, const void* cache_k, const void* cache_v, const
         // Decode: the query heads of one KV group become the ROWS of one tile (q is [batch, kv_heads, group, head_dim] in
         // memory), so every K / V tile is read once per group instead of once per query head.  One query per sequence sees
         // the whole cache: no causal predicate needed.
-        const int group = heads / kv_heads;
-        const size_t need = gqa_attention_workspace_bytes(batch, 1, heads, kv_heads, head_dim, kv_len);
-        const int splits = (need > 0 && workspace != nullptr && workspace_bytes >= need) ? decode_splits(batch, 1, heads, kv_heads, kv_len)
-                                                                                         : 1;   // too short: one pass
-        return gqa_attention_packed(q, cache_k, cache_v, out, batch * kv_heads, group, head_dim, max_len, kv_len, splits, workspace,
-                                    dtype, s);
+        const int splits = packed_splits(batch, 1, heads, kv_heads, head_dim, kv_len, workspace, workspace_bytes);
+        return contiguous_forward<AttnForm::Contig>(q, cache_k, cache_v, nullptr, nullptr, out, batch * kv_heads, heads / kv_heads, 1,
+                                                    1, head_dim, max_len, kv_len, 0, 0, splits, workspace, dtype, s);
     }
-    return gqa_attention_launch(q, cache_k, cache_v, keep, out, batch, q_len, heads, kv_heads, head_dim, max_len, kv_len, past_len,
-                                causal, 1, nullptr, dtype, s);
+    return contiguous_forward<AttnForm::Contig>(q, cache_k, cache_v, keep, nullptr, out, batch, q_len, heads, kv_heads, head_dim,
+                                                max_len, kv_len, past_len, causal, 1, nullptr, dtype, s);
+}
+
+// Training forward: keys [0, q_len) of the K / V buffers, no past, no split-KV; also writes the per-row log-sum-exp.
+int gqa_attention_train(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, float* lse, int batch,
+                        int q_len, int heads, int kv_heads, int head_dim, int max_len, int causal, int dtype, cudaStream_t s) {
+    if (head_dim != 64 && head_dim != 128) return L32_ERR_BAD_SHAPE;
+    if (batch <= 0 || q_len <= 0) return L32_OK;
+    return contiguous_forward<AttnForm::Train>(q, cache_k, cache_v, keep, lse, out, batch, q_len, heads, kv_heads, head_dim, max_len,
+                                               q_len, 0, causal, 1, nullptr, dtype, s);
 }
 
 // Paged cache: the same three launch shapes (packed decode, its split-KV form, the general causal kernel) with K / V tiles
@@ -1049,71 +1122,29 @@ int gqa_attention_paged(const void* q, const void* pool_k, const void* pool_v, c
     AttnParams p;
     int rc = packed ? attention_setup(p, q, out, batch * kv_heads, heads / kv_heads, 1, 1, head_dim, 0, dtype)
                     : attention_setup(p, q, out, batch, q_len, heads, kv_heads, head_dim, 1, dtype);
+    if (rc == L32_OK)
+        rc = paged_setup(p, pool_k, pool_v, block_table, past_lens, new_lens, num_pages, max_pages_per_seq, kv_heads, head_dim, dtype,
+                         packed);
     if (rc != L32_OK) return rc;
-    p.block_table = block_table;
-    p.past_lens = past_lens;
-    p.new_lens = new_lens;
-    p.pages_per_seq = max_pages_per_seq;
-    p.page_kv_heads = kv_heads;
-    p.packed = packed ? 1 : 0;
-    // K / V: one plane per (page, kv head) of kKvTile rows.  Rows of a page past its sequence's length are read as they are
-    // and get P = 0: the pool's contract keeps them finite (include/l32_ffn.h).
-    const uint64_t planes = static_cast<uint64_t>(num_pages) * kv_heads, plane_elems = static_cast<uint64_t>(kKvTile) * head_dim;
-    rc = make_tensor_map_3d(&p.map_k, pool_k, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
-    if (rc != L32_OK) return rc;
-    rc = make_tensor_map_3d(&p.map_v, pool_v, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
-    if (rc != L32_OK) return rc;
-    int splits = 1;
-    if (packed) {
-        const size_t need = gqa_attention_workspace_bytes(batch, 1, heads, kv_heads, head_dim, max_kv_len);
-        if (need > 0 && workspace != nullptr && workspace_bytes >= need) splits = decode_splits(batch, 1, heads, kv_heads, max_kv_len);
-    }
+    const int splits = packed ? packed_splits(batch, 1, heads, kv_heads, head_dim, max_kv_len, workspace, workspace_bytes) : 1;
     attention_split(p, splits, max_kv_len, head_dim, workspace);
-    return attention_run<true>(p, head_dim, dtype, s);
-}
-
-// Cascade decode workspace: the own-key split partials (the split-KV layout for `splits` splits, at least one), then the prefix
-// partials, one row per (item, kv head, Q-tile row).  Offsets of part_ml, pfx_o, pfx_ml and the total, each 256-aligned.
-struct CascadeLayout {
-    int splits;
-    size_t ml, pfx_o, pfx_ml, bytes;
-};
-static CascadeLayout cascade_layout(int batch, int heads, int kv_heads, int head_dim, int max_kv_len, int max_items) {
-    CascadeLayout c;
-    c.splits = max(1, decode_splits(batch, 1, heads, kv_heads, max_kv_len));
-    auto up = [](size_t x) { return (x + 255) & ~static_cast<size_t>(255); };
-    const size_t own_rows = static_cast<size_t>(batch) * heads * c.splits;
-    const size_t pfx_rows = static_cast<size_t>(max_items) * kv_heads * kQTile;
-    c.ml = up(own_rows * head_dim * sizeof(float));
-    c.pfx_o = c.ml + up(own_rows * sizeof(float2));
-    c.pfx_ml = c.pfx_o + up(pfx_rows * head_dim * sizeof(float));
-    c.bytes = c.pfx_ml + up(pfx_rows * sizeof(float2));
-    return c;
+    return attention_run<AttnForm::Paged>(p, head_dim, dtype, s);
 }
 
 size_t gqa_attention_cascade_workspace_bytes(int batch, int heads, int kv_heads, int head_dim, int max_kv_len, int max_items) {
     return cascade_layout(batch, heads, kv_heads, head_dim, max_kv_len, max_items).bytes;
 }
 
-// Cascade decode over a paged cache: one launch of the kCascade instance (prefix items and own-key splits), then the combine.
+// Cascade decode over a paged cache: one launch of the Cascade instance (prefix items and own-key splits), then the combine.
 int gqa_attention_paged_cascade(const void* q, const void* pool_k, const void* pool_v, const int* block_table, const int* past_lens,
                                 const int* new_lens, const int* items, const int* members, const int* seq_plan, int max_items,
                                 void* out, void* workspace, int batch, int heads, int kv_heads, int head_dim, int num_pages,
                                 int max_pages_per_seq, int max_kv_len, int dtype, cudaStream_t s) {
-    const int group = heads / kv_heads;
     AttnParams p;
-    int rc = attention_setup(p, q, out, batch * kv_heads, group, 1, 1, head_dim, 0, dtype);
-    if (rc != L32_OK) return rc;
-    p.block_table = block_table;
-    p.past_lens = past_lens;
-    p.new_lens = new_lens;
-    p.pages_per_seq = max_pages_per_seq;
-    p.page_kv_heads = kv_heads;
-    p.packed = 1;
-    const uint64_t planes = static_cast<uint64_t>(num_pages) * kv_heads, plane_elems = static_cast<uint64_t>(kKvTile) * head_dim;
-    rc = make_tensor_map_3d(&p.map_k, pool_k, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
-    if (rc != L32_OK) return rc;
-    rc = make_tensor_map_3d(&p.map_v, pool_v, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
+    int rc = attention_setup(p, q, out, batch * kv_heads, heads / kv_heads, 1, 1, head_dim, 0, dtype);
+    if (rc == L32_OK)
+        rc = paged_setup(p, pool_k, pool_v, block_table, past_lens, new_lens, num_pages, max_pages_per_seq, kv_heads, head_dim, dtype,
+                         true);
     if (rc != L32_OK) return rc;
     const CascadeLayout c = cascade_layout(batch, heads, kv_heads, head_dim, max_kv_len, max_items);
     uint8_t* ws = static_cast<uint8_t*>(workspace);
@@ -1127,11 +1158,7 @@ int gqa_attention_paged_cascade(const void* q, const void* pool_k, const void* p
     p.casc_members = members;
     p.casc_seq = seq_plan;
     p.casc_max_items = max_items;
-    if (dtype == L32_BF16)
-        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16, false, true, true>(p, s)
-                             : launch_attention<64, __nv_bfloat16, false, true, true>(p, s);
-    else
-        rc = head_dim == 128 ? launch_attention<128, __half, false, true, true>(p, s) : launch_attention<64, __half, false, true, true>(p, s);
+    rc = launch_form<AttnForm::Cascade>(p, head_dim, dtype, s);
     if (rc != L32_OK) return rc;
     return launch_combine<true>(p, head_dim, dtype, s);
 }
@@ -1139,14 +1166,8 @@ int gqa_attention_paged_cascade(const void* q, const void* pool_k, const void* p
 // Verify step: one query tile per (sequence, kv head) holding the group query heads of each of the sequence's q_len new tokens,
 // split over the keys with the packed decode's plan for max_kv_len.  The partials' layout (AttnParams, "verify step") lets the
 // plain combine write ctx in its [batch, q_len, heads, d] layout.
-static int verify_splits(int batch, int heads, int kv_heads, int max_kv_len) {
-    return decode_splits(batch, 1, heads, kv_heads, max_kv_len);
-}
-
 size_t gqa_attention_verify_workspace_bytes(int batch, int q_len, int heads, int kv_heads, int head_dim, int max_kv_len) {
-    const int splits = verify_splits(batch, heads, kv_heads, max_kv_len);
-    if (splits < 2) return 0;
-    return static_cast<size_t>(batch) * heads * q_len * splits * (static_cast<size_t>(head_dim) + 2) * sizeof(float) + 256;
+    return packed_workspace_bytes(batch, q_len, heads, kv_heads, head_dim, max_kv_len);
 }
 
 int gqa_attention_paged_verify(const void* q, const void* pool_k, const void* pool_v, const int* block_table, const int* past_lens,
@@ -1156,82 +1177,24 @@ int gqa_attention_paged_verify(const void* q, const void* pool_k, const void* po
     const int group = heads / kv_heads;
     AttnParams p;
     int rc = attention_setup(p, q, out, batch * kv_heads, group * q_len, 1, 1, head_dim, 1, dtype);
+    if (rc == L32_OK)
+        rc = make_tensor_map_3d_box(&p.map_q, q, static_cast<uint64_t>(batch) * q_len, heads, head_dim, head_dim,
+                                    static_cast<uint64_t>(heads) * head_dim, group, q_len, dtype);
+    if (rc == L32_OK)
+        rc = paged_setup(p, pool_k, pool_v, block_table, past_lens, new_lens, num_pages, max_pages_per_seq, kv_heads, head_dim, dtype,
+                         true);
     if (rc != L32_OK) return rc;
-    rc = make_tensor_map_3d_box(&p.map_q, q, static_cast<uint64_t>(batch) * q_len, heads, head_dim, head_dim,
-                                static_cast<uint64_t>(heads) * head_dim, group, q_len, dtype);
-    if (rc != L32_OK) return rc;
-    p.block_table = block_table;
-    p.past_lens = past_lens;
-    p.new_lens = new_lens;
-    p.pages_per_seq = max_pages_per_seq;
-    p.page_kv_heads = kv_heads;
-    p.packed = 1;
     p.verify_t = q_len;
     p.verify_group = group;
-    const uint64_t planes = static_cast<uint64_t>(num_pages) * kv_heads, plane_elems = static_cast<uint64_t>(kKvTile) * head_dim;
-    rc = make_tensor_map_3d(&p.map_k, pool_k, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
-    if (rc != L32_OK) return rc;
-    rc = make_tensor_map_3d(&p.map_v, pool_v, planes, kKvTile, head_dim, head_dim, plane_elems, kKvTile, dtype);
-    if (rc != L32_OK) return rc;
-    const size_t need = gqa_attention_verify_workspace_bytes(batch, q_len, heads, kv_heads, head_dim, max_kv_len);
-    const int splits = (need > 0 && workspace != nullptr && workspace_bytes >= need) ? verify_splits(batch, heads, kv_heads, max_kv_len)
-                                                                                     : 1;
-    attention_split(p, splits, max_kv_len, head_dim, workspace);
-    if (dtype == L32_BF16)
-        rc = head_dim == 128 ? launch_attention<128, __nv_bfloat16, false, true, false, true>(p, s)
-                             : launch_attention<64, __nv_bfloat16, false, true, false, true>(p, s);
-    else
-        rc = head_dim == 128 ? launch_attention<128, __half, false, true, false, true>(p, s)
-                             : launch_attention<64, __half, false, true, false, true>(p, s);
+    attention_split(p, packed_splits(batch, q_len, heads, kv_heads, head_dim, max_kv_len, workspace, workspace_bytes), max_kv_len,
+                    head_dim, workspace);
+    rc = launch_form<AttnForm::Verify>(p, head_dim, dtype, s);
     if (rc != L32_OK || p.splits == 1) return rc;
     AttnParams c = p;                                      // the combine's view of the partials: rows (token, group head)
     c.batch = batch * q_len;
     c.heads = group;
     c.q_len = kv_heads;
     return launch_combine<false>(c, head_dim, dtype, s);
-}
-
-// Training forward: keys [0, q_len) of the K / V buffers, no past, no split-KV; also writes the per-row log-sum-exp.
-int gqa_attention_train(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, float* lse, int batch,
-                        int q_len, int heads, int kv_heads, int head_dim, int max_len, int causal, int dtype, cudaStream_t s) {
-    if (head_dim != 64 && head_dim != 128) return L32_ERR_BAD_SHAPE;
-    if (batch <= 0 || q_len <= 0) return L32_OK;
-    return gqa_attention_launch(q, cache_k, cache_v, keep, out, batch, q_len, heads, kv_heads, head_dim, max_len, q_len, 0, causal, 1,
-                                nullptr, dtype, s, lse);
-}
-
-// Decode layout: batch' = batch * kv_heads sequences of `group` query rows, one head.
-int gqa_attention_packed(const void* q, const void* cache_k, const void* cache_v, void* out, int batch2, int group, int head_dim,
-                         int max_len, int kv_len, int splits, void* workspace, int dtype, cudaStream_t s) {
-    return gqa_attention_launch(q, cache_k, cache_v, nullptr, out, batch2, group, 1, 1, head_dim, max_len, kv_len, 0, 0, splits,
-                                workspace, dtype, s);
-}
-
-int gqa_attention_launch(const void* q, const void* cache_k, const void* cache_v, const uint8_t* keep, void* out, int batch, int q_len,
-                         int heads, int kv_heads, int head_dim, int max_len, int kv_len, int past_len, int causal, int splits,
-                         void* workspace, int dtype, cudaStream_t s, float* lse) {
-    AttnParams p;
-    int rc = attention_setup(p, q, out, batch, q_len, heads, kv_heads, head_dim, causal, dtype);
-    if (rc != L32_OK) return rc;
-    p.lse = lse;
-    p.keep = keep;
-    p.max_len = max_len; p.kv_len = kv_len; p.past_len = past_len;
-    // K / V: one plane per (batch, kv head), cut at kv_len.  Masked keys get P = 0, but 0 * NaN and 0 * Inf are NaN in the
-    // P V product: the rows of the last tile beyond kv_len (stale cache capacity, or the next head's keys) must not reach
-    // shared memory with whatever they hold, so TMA fills them with zeros.
-    const uint64_t planes = static_cast<uint64_t>(batch) * kv_heads, plane_elems = static_cast<uint64_t>(max_len) * head_dim;
-    const uint64_t kv_rows = static_cast<uint64_t>(kv_len > 0 ? kv_len : 1);   // kv_len 0: no tile is loaded
-    rc = make_tensor_map_3d(&p.map_k, cache_k, planes, kv_rows, head_dim, head_dim, plane_elems, kKvTile, dtype);
-    if (rc != L32_OK) return rc;
-    rc = make_tensor_map_3d(&p.map_v, cache_v, planes, kv_rows, head_dim, head_dim, plane_elems, kKvTile, dtype);
-    if (rc != L32_OK) return rc;
-    attention_split(p, splits, kv_len, head_dim, workspace);
-    if (lse != nullptr) {
-        if (dtype == L32_BF16)
-            return head_dim == 128 ? launch_attention<128, __nv_bfloat16, true, false>(p, s) : launch_attention<64, __nv_bfloat16, true, false>(p, s);
-        return head_dim == 128 ? launch_attention<128, __half, true, false>(p, s) : launch_attention<64, __half, true, false>(p, s);
-    }
-    return attention_run<false>(p, head_dim, dtype, s);
 }
 
 }  // namespace l32

@@ -811,6 +811,26 @@ class PagedKVCache:
             host[cap + self.max_batch:cap + self.max_batch + 4 * len(seq)] = torch.tensor(seq, dtype=torch.int32).flatten()
         self._plan_dev.copy_(host, non_blocking=True)
 
+    def attention(self, q, pool_k, pool_v):
+        """ctx [b, t, heads * d] of the current step over one layer's pools (q RoPE'd, the step's K / V appended), in the form
+        the step was planned for: the verify kernel for a verify step it fits (ops.verify_fits), the cascade for a decode step
+        with a cascade plan for this attention's geometry, else the plain paged attention.  The first call records the
+        geometry the steps planned from then on are sized for."""
+        _, t, width = q.shape
+        _, kv_heads, _, d = pool_k.shape
+        group = width // d // kv_heads
+        if self.cascade_geometry is None:
+            self.cascade_geometry = (group, kv_heads)
+        if self.verify and ops.verify_fits(group, t):
+            return ops.gqa_attention_forward_paged_verify(q, pool_k, pool_v, self.block_table, self.past_lens, self.new_lens,
+                                                          max_kv_len=self.max_kv_len)
+        if t == 1 and self.cascade and self.cascade_geometry == (group, kv_heads):
+            return ops.gqa_attention_forward_paged_cascade(q, pool_k, pool_v, self.block_table, self.past_lens, self.new_lens,
+                                                           self.plan_items, self.plan_members, self.plan_seq,
+                                                           self.cascade_max_items, max_kv_len=self.max_kv_len)
+        return ops.gqa_attention_forward_paged(q, pool_k, pool_v, self.block_table, self.past_lens, self.new_lens,
+                                               max_kv_len=self.max_kv_len)
+
     def advance(self) -> None:
         """After the step's last layer: every sequence of the batch now holds its new tokens."""
         for sid, n in zip(self.batch_ids, self.batch_new_lens):
@@ -1022,20 +1042,7 @@ class GroupQueryAttention(nn.Module):
         q, k, v = self._qkv(hidden_states)
         pk, pv = cache.pools(self.layer_idx or 0, self.num_kv_groups, self.head_dim, q.dtype, q.device)
         ops.rope_kv_append_paged(q, k, v, pos, pk, pv, cache.block_table, cache.past_lens, cache.new_lens, self.rope_base)
-        geometry = (self.group_size, self.num_kv_groups)
-        if cache.cascade_geometry is None:
-            cache.cascade_geometry = geometry                 # the steps planned from now on fit this attention
-        if cache.verify and ops.verify_fits(self.group_size, t):
-            ctx = ops.gqa_attention_forward_paged_verify(q, pk, pv, cache.block_table, cache.past_lens, cache.new_lens,
-                                                         max_kv_len=cache.max_kv_len)
-        elif t == 1 and cache.cascade and cache.cascade_geometry == geometry:
-            ctx = ops.gqa_attention_forward_paged_cascade(q, pk, pv, cache.block_table, cache.past_lens, cache.new_lens,
-                                                          cache.plan_items, cache.plan_members, cache.plan_seq,
-                                                          cache.cascade_max_items, max_kv_len=cache.max_kv_len)
-        else:
-            ctx = ops.gqa_attention_forward_paged(q, pk, pv, cache.block_table, cache.past_lens, cache.new_lens,
-                                                  max_kv_len=cache.max_kv_len)
-        return self._project(self.out_proj, ctx)
+        return self._project(self.out_proj, cache.attention(q, pk, pv))
 
     def forward(self, hidden_states, attention_mask=None, position_ids=None, kv_cache=None):
         if isinstance(kv_cache, PagedKVCache):

@@ -151,3 +151,13 @@ def test_paged_argument_validation_without_device(lib):
     assert att(ctypes.c_void_p(8), one, one, one, one, one, one, null, 0, 2, 1, 32, 8, 128, 16, 4, 256, 0, null) == -3
     assert att(*p8[:7], ctypes.c_void_p(8), 1 << 20, 2, 1, 32, 8, 128, 16, 4, 256, 0, null) == -6
     assert att(null, null, null, null, null, null, null, null, 0, 0, 1, 32, 8, 128, 16, 4, 256, 0, null) == 0
+    assert att(*p8, 0, -1, 1, 32, 8, 128, 16, 4, 256, 0, null) == -2
+    assert att(*p8, 0, 2, 1, 32, 8, 128, 0, 4, 256, 0, null) == -2                      # no pages
+    assert att(one, one, null, one, one, one, one, null, 0, 2, 1, 32, 8, 128, 16, 4, 256, 0, null) == -4   # pool_v
+    assert att(one, one, one, one, null, one, one, null, 0, 2, 1, 32, 8, 128, 16, 4, 256, 0, null) == -4   # past_lens
+    assert att(*p8[:6], ctypes.c_void_p(8), null, 0, 2, 1, 32, 8, 128, 16, 4, 256, 0, null) == -3          # ctx
+    # a call with several faults gets the code of the first check: dtype, shape, empty batch, nulls, alignment, workspace
+    assert att(*[null] * 8, 0, 0, 1, 32, 8, 128, 16, 4, 256, 9, null) == -1
+    assert att(*[null] * 8, 0, 2, 1, 32, 8, 128, 16, 4, 257, 0, null) == -2
+    assert att(ctypes.c_void_p(8), one, one, null, one, one, one, null, 0, 2, 1, 32, 8, 128, 16, 4, 256, 0, null) == -4
+    assert att(ctypes.c_void_p(8), *p8[1:7], ctypes.c_void_p(8), 1 << 20, 2, 1, 32, 8, 128, 16, 4, 256, 0, null) == -3

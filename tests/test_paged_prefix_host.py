@@ -211,3 +211,12 @@ def test_cascade_argument_validation_without_device(lib):
     assert att(*p11, need - 1, 2, 32, 8, 128, 16, 4, 256, 37, 0, null) == -6           # workspace short
     assert att(*p11[:10], ctypes.c_void_p(8), need, 2, 32, 8, 128, 16, 4, 256, 37, 0, null) == -6
     assert att(*([null] * 11), 0, 0, 32, 8, 128, 16, 4, 256, 37, 0, null) == 0          # empty batch
+    assert att(*p11, need, 2, 32, 8, 128, 16, 4, -1, 37, 0, null) == -2
+    assert att(*p11, need, 2, 32, 8, 128, 0, 4, 256, 37, 0, null) == -2                 # no pages
+    assert att(*p11[:9], ctypes.c_void_p(8), one, need, 2, 32, 8, 128, 16, 4, 256, 37, 0, null) == -3   # ctx
+    assert att(one, one, ctypes.c_void_p(8), *p11[3:], need, 2, 32, 8, 128, 16, 4, 256, 37, 0, null) == -3   # pool_v
+    # a call with several faults gets the code of the first check: dtype, shape, empty batch, nulls, alignment, workspace
+    assert att(*([null] * 11), 0, 0, 32, 8, 128, 16, 4, 256, 37, 7, null) == -1
+    assert att(*([null] * 11), 0, 2, 32, 8, 128, 16, 4, 257, 37, 0, null) == -2
+    assert att(ctypes.c_void_p(8), *p11[1:6], null, *p11[7:], need, 2, 32, 8, 128, 16, 4, 256, 37, 0, null) == -4
+    assert att(ctypes.c_void_p(8), *p11[1:10], ctypes.c_void_p(8), need - 1, 2, 32, 8, 128, 16, 4, 256, 37, 0, null) == -3

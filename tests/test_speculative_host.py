@@ -194,6 +194,17 @@ def test_verify_argument_validation_without_device(lib):
     args[7] = ctypes.c_void_p(8)
     assert f(args, 2, 4, 32, 8, 128) == -6                # workspace not 16-byte aligned
     assert f([null] * 8, 0, 4, 32, 8, 128) == 0           # empty batch
+    assert f(p8, 2, 4, 32, 8, 128, mkv=-1) == -2
+    assert f(p8, 2, 4, 32, 8, 128, mp=0) == -2            # no table columns
+    args = list(p8)
+    args[6] = ctypes.c_void_p(8)
+    assert f(args, 2, 4, 32, 8, 128) == -3                # ctx not 16-byte aligned
+    # a call with several faults gets the code of the first check: dtype, shape, empty batch, nulls, alignment, workspace
+    assert f([null] * 8, 0, 4, 32, 8, 128, dt=2) == -1
+    assert f([null] * 8, 2, 4, 32, 8, 128, mkv=257) == -2
+    assert f([null] * 8, 2, 33, 32, 8, 128) == -2
+    assert f([ctypes.c_void_p(8), one, one, null, one, one, one, one], 2, 4, 32, 8, 128) == -4
+    assert f([ctypes.c_void_p(8)] + p8[1:7] + [ctypes.c_void_p(8)], 2, 4, 32, 8, 128) == -3
     assert lib.l32_gqa_attention_verify_workspace_bytes(2, 33, 32, 8, 128, 4096) == 0
 
 
