@@ -187,7 +187,8 @@ __global__ void __launch_bounds__(256) add_rmsnorm_fwd_generic_kernel(
 // registers over all rows of the CTA and leaves as ONE fp32 partial row per CTA (deterministic, no atomics).
 // ------------------------------------------------------------------------------------------------
 constexpr int kBwdConsumersMax = 512;
-constexpr int kBwdMaxStages = 12;
+constexpr int kBwdStagesWanted = 12;   // ring depth, rounded up to a multiple of the row groups (see launch_bwd_fast)
+constexpr int kBwdMaxStages = 16;
 constexpr int kBwdBarrierBytes = 2 * kBwdMaxStages * 8;
 constexpr int kBwdRedBytes = 2 * 16 * 16 * 4 * 2;   // [parity][group][row of the iteration (<= 2)][warp of the group]
 
@@ -332,6 +333,9 @@ __global__ void __launch_bounds__(kBwdConsumers + 32, 1) rmsnorm_bwd_kernel(
                         hraw[r][k] = lds_v4(src + row_bytes + static_cast<size_t>(v) * 16);
                     }
                 }
+                // The refill is a bulk copy (async proxy). Without this fence the arrive does not wait for the loads
+                // above, and a late ld.shared could read part of the next row of the stage.
+                fence_proxy_async_smem();
                 __syncwarp();
                 if ((t & 31) == 0) mbar_arrive(&empty_bar[s]);   // stage may be refilled
             }
@@ -577,7 +581,13 @@ static cudaError_t launch_bwd_fast(const T* dy, const T* h, const T* weight, con
     const size_t row_bytes = static_cast<size_t>(C) * sizeof(T);
     const size_t stage_bytes = 2 * row_bytes;
     int stages = static_cast<int>((200 * 1024 - row_bytes) / stage_bytes);
-    if (stages > kBwdMaxStages) stages = kBwdMaxStages;
+    // Row i goes to stage i % stages and to row group i % G. With stages a multiple of G every stage has one consumer
+    // group, which waits for its uses in order, so the parity wait on full_bar[s] cannot pass on use u - 2's phase while
+    // use u - 1 (a bulk copy of another group's row, which need not complete in issue order) is still in flight.
+    constexpr int kStagesCap = (kBwdStagesWanted + G - 1) / G * G;   // at least kBwdStagesWanted where the ring fits them
+    static_assert(kStagesCap <= kBwdMaxStages, "barrier slots");
+    if (stages > kStagesCap) stages = kStagesCap;
+    stages -= stages % G;
     // the d_weight fold reuses the ring: (G - 1) fp32 rows must fit into it
     if (stages < 2 || static_cast<size_t>(stages) * stage_bytes < static_cast<size_t>(G - 1) * C * sizeof(float))
         return cudaErrorInvalidConfiguration;

@@ -1,7 +1,8 @@
 """GPU: attention backward for training calls (GQAAttentionFunction, l32_gqa_attention_forward_train / _backward).
 
 Gradients are compared with the project's gradient tolerances (rel-L2 <= 1e-2, max-abs <= 2^-5 * max|ref|) against fp32
-autograd on the CPU: of the softmax written out at kernel level, and of the reference's own expressions at module level.
+autograd on the CPU: of the softmax written out at kernel level, and of the reference's own expressions at module level.  At
+4096 and 8192 tokens the softmax written out runs on the GPU in fp32 with TF32 off, in query chunks.
 """
 import copy
 import math
@@ -31,7 +32,7 @@ def close(got, ref, tol, what=""):
 
 def _rope(x, pos, d):
     """RoPE of x [b, h, t, d] at positions pos [b, t] in fp32 (angles as the kernels compute them)."""
-    i = torch.arange(d // 2, dtype=torch.float32)
+    i = torch.arange(d // 2, dtype=torch.float32, device=x.device)
     inv = torch.exp2(-math.log2(BASE) * (2.0 * i / d))
     ang = pos.float()[:, None, :, None] * inv
     cs, sn = ang.cos(), ang.sin()
@@ -39,23 +40,31 @@ def _rope(x, pos, d):
     return torch.cat((x1 * cs - x2 * sn, x2 * cs + x1 * sn), -1)
 
 
-def _attention_ref(q, k, v, pos, causal, keep, heads, kv, d):
-    """fp32 softmax attention over pre-RoPE q [b, t, heads*d], k / v [b, t, kv*d]; rows without a visible key give zeros."""
-    b, t, _ = q.shape
-    q4 = _rope(q.view(b, t, heads, d).transpose(1, 2), pos, d)
+def _attention_ref(q, k, v, pos, causal, keep, heads, kv, d, q0=0):
+    """fp32 softmax attention of pre-RoPE queries q [b, n, heads*d] at rows [q0, q0 + n) over keys k / v [b, t, kv*d], on
+    the inputs' device; pos [b, t] and keep [b, t] are the keys' (and the queries' at their rows).  Rows without a visible
+    key give zeros.  Returns (out [b, n, heads*d], alive [b, n])."""
+    b, n, _ = q.shape
+    t = k.shape[1]
+    dev = q.device
+    q4 = _rope(q.view(b, n, heads, d).transpose(1, 2), pos[:, q0:q0 + n], d)
     k4 = _rope(k.view(b, t, kv, d).transpose(1, 2), pos, d).repeat_interleave(heads // kv, 1)
     v4 = v.view(b, t, kv, d).transpose(1, 2).repeat_interleave(heads // kv, 1)
     sc = q4 @ k4.transpose(-1, -2) / d ** 0.5
-    m = torch.ones(t, t, dtype=torch.bool)
+    m = torch.ones(n, t, dtype=torch.bool, device=dev)
     if causal:
-        m &= torch.arange(t)[None] <= torch.arange(t)[:, None]
+        m &= torch.arange(t, device=dev)[None] <= torch.arange(q0, q0 + n, device=dev)[:, None]
     m = m[None, None] & keep[:, None, None, :].bool()
     alive = m.any(-1, keepdim=True)
     pr = torch.softmax(sc.masked_fill(~m, -1e30), -1) * alive
-    return (pr @ v4).transpose(1, 2).reshape(b, t, heads * d), alive[:, 0, :, 0]
+    return (pr @ v4).transpose(1, 2).reshape(b, n, heads * d), alive[:, 0, :, 0]
 
 
 def _inputs(b, t, heads, kv, d, pad, seed):
+    """bf16-representable q, k, v, d_ctx with key_keep [b, t] and positions [b, t].  `pad` is an int n (keys [0, n) of
+    sequence 0 padded) or a pattern: "holes" (about 15 % of the keys of every sequence), "right" (a trailing run of the last
+    sequence), "all" (the last sequence entirely), "resets" (no padding; positions restart at 0 partway through each
+    sequence, as in packed documents).  Otherwise positions are offset + index with an offset per sequence."""
     gen = torch.Generator().manual_seed(seed)
     rep = lambda x: x.to(torch.bfloat16).float()
     q = rep(torch.randn(b, t, heads * d, generator=gen))
@@ -63,8 +72,22 @@ def _inputs(b, t, heads, kv, d, pad, seed):
     v = rep(torch.randn(b, t, kv * d, generator=gen))
     g = rep(torch.randn(b, t, heads * d, generator=gen))
     keep = torch.ones(b, t, dtype=torch.uint8)
-    keep[0, :pad] = 0
-    pos = (7 + 3 * torch.arange(b)[:, None] + torch.arange(t)[None]).to(torch.int64)   # positions that do not start at 0
+    idx = torch.arange(t)[None]
+    pos = (7 + 3 * torch.arange(b)[:, None] + idx).to(torch.int64)   # positions that do not start at 0
+    if isinstance(pad, int):
+        keep[0, :pad] = 0
+    elif pad == "holes":
+        keep[torch.rand(b, t, generator=gen) < 0.15] = 0
+    elif pad == "right":
+        keep[-1, t - max(1, t // 3):] = 0
+    elif pad == "all":
+        keep[-1] = 0
+    elif pad == "resets":
+        r1 = torch.randint(1, max(2, t // 2), (b, 1), generator=gen)     # document starts: r1, then r2
+        r2 = r1 + torch.randint(1, max(2, t // 2), (b, 1), generator=gen)
+        pos = torch.where(idx < r1, pos, torch.where(idx < r2, idx - r1, idx - r2))
+    else:
+        raise ValueError(pad)
     return q, k, v, g, keep, pos
 
 
@@ -81,6 +104,7 @@ def _gpu_fwd_bwd(q, k, v, g, keep, pos, causal, heads, kv, d, dtype):
 
 
 GRID = [  # (b, t, heads, kv, d, causal, pad, dtype): the forward key-padding test's grid, then t in {1, 63, 129, 300, 2048}
+    # (pad: see _inputs)
     (1, 128, 1, 1, 128, True, 0, torch.bfloat16), (1, 128, 1, 1, 128, True, 5, torch.bfloat16),
     (1, 128, 1, 1, 128, True, 37, torch.bfloat16), (1, 128, 1, 1, 128, True, 64, torch.bfloat16),
     (1, 128, 1, 1, 128, True, 70, torch.bfloat16), (2, 300, 4, 2, 128, True, 37, torch.bfloat16),
@@ -90,6 +114,13 @@ GRID = [  # (b, t, heads, kv, d, causal, pad, dtype): the forward key-padding te
     (1, 129, 8, 2, 128, False, 0, torch.float16), (2, 129, 4, 1, 64, True, 17, torch.bfloat16),
     (2, 300, 8, 2, 128, True, 0, torch.float16), (1, 2048, 4, 1, 64, True, 0, torch.float16),
     (1, 300, 2, 1, 128, False, 40, torch.float16),
+    # group 8 (the 90B geometry's 64 / 8, on every rank of its 2-, 4- and 8-GPU shardings): dK / dV sum 8 heads in TMEM
+    (1, 1024, 8, 1, 128, True, "holes", torch.bfloat16), (2, 300, 16, 2, 64, False, "holes", torch.float16),
+    (1, 1024, 64, 8, 128, True, 100, torch.bfloat16),
+    # padding of sequences b > 0 (the b * q_len offset of key_keep), a fully padded sequence, position resets
+    (3, 200, 8, 2, 128, True, "right", torch.bfloat16), (2, 190, 8, 4, 64, False, "right", torch.float16),
+    (3, 130, 8, 2, 64, True, "all", torch.bfloat16), (2, 257, 4, 2, 128, False, "all", torch.float16),
+    (2, 300, 8, 2, 128, True, "resets", torch.bfloat16), (2, 300, 4, 2, 64, True, "resets", torch.float16),
 ]
 
 
@@ -97,7 +128,7 @@ GRID = [  # (b, t, heads, kv, d, causal, pad, dtype): the forward key-padding te
 def test_attention_backward_kernels_vs_fp32_autograd(b, t, heads, kv, d, causal, pad, dtype):
     """dq, dk, dv of the pre-RoPE projections (inverse RoPE included) against fp32 autograd of the softmax written out.
     Rows that see no key must give dq == 0 exactly and lse == +inf; padded keys dk == dv == 0 exactly."""
-    q, k, v, g, keep, pos = _inputs(b, t, heads, kv, d, pad, seed=b * 131 + t + pad + d)
+    q, k, v, g, keep, pos = _inputs(b, t, heads, kv, d, pad, seed=b * 131 + t + (pad if isinstance(pad, int) else 0) + d)
     ctx, lse, (dq, dk, dv), _ = _gpu_fwd_bwd(q, k, v, g, keep, pos, causal, heads, kv, d, dtype)
     qs, ks, vs = (x.clone().requires_grad_(True) for x in (q, k, v))
     ref, alive = _attention_ref(qs, ks, vs, pos, causal, keep, heads, kv, d)
@@ -246,6 +277,33 @@ def test_attention_training_memory_is_linear_in_tokens():
     peak = torch.cuda.max_memory_allocated() - base
     assert peak < 512 * 2 ** 20, f"peak {peak / 2 ** 20:.0f} MiB above the inputs"
     assert torch.isfinite(q.grad.float()).all() and torch.isfinite(k.grad.float()).all() and torch.isfinite(v.grad.float()).all()
+
+
+@pytest.mark.parametrize("t,heads,pad", [(8192, 32, 0), (4096, 64, "holes")])
+def test_attention_backward_full_length_vs_fp32(t, heads, pad):
+    """1 x t tokens, 8 kv heads of 128, causal, bf16 (groups 4 and 8 at full length): ctx, dq, dk, dv against the
+    reference's expressions in fp32 on the GPU with TF32 off.  The reference runs in query chunks, each backpropagated on its
+    own with dk / dv accumulating, so no [heads, t, t] tensor exists."""
+    b, kv, d, chunk = 1, 8, 128, 512
+    q, k, v, g, keep, pos = _inputs(b, t, heads, kv, d, pad, seed=t + heads)
+    ctx, _, (dq, dk, dv), _ = _gpu_fwd_bwd(q, k, v, g, keep, pos, True, heads, kv, d, torch.bfloat16)
+    qs, ks, vs = (x.to(DEV).requires_grad_(True) for x in (q, k, v))
+    gd, keep_d, pos_d = g.to(DEV), keep.to(DEV), pos.to(DEV)
+    out = torch.empty(b, t, heads * d, device=DEV)
+    tf32 = torch.backends.cuda.matmul.allow_tf32
+    torch.backends.cuda.matmul.allow_tf32 = False
+    try:
+        assert not torch.backends.cuda.matmul.allow_tf32
+        for q0 in range(0, t, chunk):
+            o, _ = _attention_ref(qs[:, q0:q0 + chunk], ks, vs, pos_d, True, keep_d, heads, kv, d, q0)
+            (o * gd[:, q0:q0 + chunk]).sum().backward()
+            out[:, q0:q0 + chunk] = o.detach()
+    finally:
+        torch.backends.cuda.matmul.allow_tf32 = tf32
+    close(ctx, out, FWD, "ctx")
+    close(dq, qs.grad, BWD, "dq")
+    close(dk, ks.grad, BWD, "dk")
+    close(dv, vs.grad, BWD, "dv")
 
 
 def test_attention_train_forward_backward_graph_replay():
